@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- WBC control-cycle solves/s on N B200s (one process per GPU), see DESIGN.md "Measurement".
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one full control cycle (update -> Fgrf -> estimate -> QP assembly -> DENSE-AUL solve -> tau) over one
 batch of synthetic DogBot instances.  At N=1 the workload is BASELINE.json configs[1] (4096 standing instances);
@@ -14,7 +14,11 @@ all-reduce of a 7-double statistics vector at the end).
             the same process; HBM figures beside it (the path is FP64-pipe/latency bound, not HBM bound)
   cpu_baseline  the CPU oracle (C restatement + the reference's own ALGLIB) on all host cores, same inputs
 
-`--impl reference` times that CPU path alone (rank 0 only).
+`--impl reference` times that CPU path alone (rank 0 only).  Where the reference's ALGLIB is not built, the B200 arm reports
+cpu_baseline as unavailable and `--impl reference` fails.
+
+`--dump-outputs DIR` writes what the timed loop computed in its last step (rank 0's shard), one DIR/<name>.npy per output the
+caller receives, so that two builds can be compared output for output: the inputs are seeded, the same arguments give the same ones.
 """
 import argparse
 import json
@@ -67,6 +71,34 @@ def cpu_reference_run(sc, steps, warmup, sample, cores):
         if it >= warmup:
             times.append(secs)
     return kind, float(np.sum(times)), times
+
+
+def reference_built():
+    from oracle import oracle_py as op
+    op.build(ref=True)
+    return op.have_ref()
+
+
+NO_CPU_BASELINE = {"value": None, "unit": UNIT, "kind": "unavailable",
+                   "note": "the reference's ALGLIB (oracle/_ref/libref_alglib_qp.so) is not built, so the CPU path cannot run"}
+DUMP_LIMIT = 64_000_000            # bytes on disk, all files of one dump together
+NPY_HEADER_MAX = 1024               # room left per .npy file for its header (numpy writes 128 bytes for these shapes)
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: each [k, n] output as path/<name>.npy in float64.  Above DUMP_LIMIT bytes on disk in all, the same fixed, seeded
+    sample of instances (columns) is taken from every output, and the sampled instance indices are written as instances.npy."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    n = next(iter(arrays.values())).shape[-1]
+    per_instance = sum(a.nbytes // n for a in arrays.values())
+    if per_instance * n + NPY_HEADER_MAX * len(arrays) > DUMP_LIMIT:
+        room = DUMP_LIMIT - NPY_HEADER_MAX * (len(arrays) + 1)
+        keep = np.sort(np.random.default_rng(0).choice(n, room // (per_instance + 8), replace=False))
+        arrays = {k: a[..., keep] for k, a in arrays.items()}
+        arrays["instances"] = keep.astype(np.float64)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), np.ascontiguousarray(a))
 
 
 class ClockSampler(threading.Thread):
@@ -141,7 +173,7 @@ def single_robot_replay(args):
         batch.cycle_device(one, dev_out, 1, ncyc, stream=sp, sync=False)
 
     host = [{k: (np.ascontiguousarray(v[..., i:i + 1]) if isinstance(v, np.ndarray) else v) for k, v in sc.items()} for i in range(ncyc)]
-    steps, warm = max(args.steps, ncyc), max(args.warmup, 3)
+    steps, warm = (ncyc if args.steps is None else args.steps), args.warmup
     batch.set_observer_state(np.zeros((6, 1)), np.zeros((6, 1)))
     for i in range(warm):
         dev_cycle(i % ncyc)
@@ -156,6 +188,7 @@ def single_robot_replay(args):
         ev[it][1].record(stream)
         ev[it][1].synchronize()
     step_ms = np.array([a.elapsed_time(b) for a, b in ev])
+    last = {k: v.cpu().numpy() for k, v in dev_out.items()}
     batch.set_observer_state(np.zeros((6, 1)), np.zeros((6, 1)))
     e2e_ms = []
     for it in range(warm + steps):
@@ -168,24 +201,28 @@ def single_robot_replay(args):
     line = {"metric": METRIC, "value": 1e3 / float(step_ms.mean()), "unit": UNIT, "n_gpus": 1, "steps": steps, "warmup": warm,
             "ms_per_step": float(step_ms.mean()), "p50_ms": float(np.median(step_ms)), "p95_ms": float(np.percentile(step_ms, 95)),
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
-            "config": {"workload": "%s: ONE DogBot, 184-cycle synthetic trot replay (46 stance + 46 swing{BR,FL} + 46 stance + 46 swing{BL,FR}), one control cycle per step, observer chained" % REPLAY,
+            "config": {"workload": "%s: ONE DogBot, 184-cycle synthetic trot replay (46 stance + 46 swing{BR,FL} + 46 stance + 46 swing{BL,FR}), one control cycle per step, observer chained; timed: the first %d cycles of the replay (wrapping)" % (REPLAY, steps),
                        "instances_per_gpu": 1, "global_batch": 1, "parallelism": "single robot", "l2": "not flushed (a 400 Hz loop keeps its working set warm)"},
             "clocks": clocks,
             "e2e": {"value": 1e3 / float(e2e_ms.mean()), "unit": UNIT, "p50_ms": float(np.median(e2e_ms)), "p95_ms": float(np.percentile(e2e_ms, 95)),
                     "h2d_bytes_per_step": IN_BYTES, "d2h_bytes_per_step": OUT_BYTES},
             "gpu_launches": 2 * steps}
-    if not args.no_cpu_baseline:
+    if not args.no_cpu_baseline and not reference_built():
+        line["cpu_baseline"] = NO_CPU_BASELINE
+    elif not args.no_cpu_baseline:
         from oracle import oracle_py as op
-        op.build(ref=True)
         t0 = time.perf_counter()
         yd, yw = np.zeros((6, 1)), np.zeros((6, 1))
-        for i in range(ncyc):
-            one = dict(host[i]); one["obs_yd"], one["obs_yw"] = yd, yw
+        for i in range(steps):
+            one = dict(host[i % ncyc]); one["obs_yd"], one["obs_yw"] = yd, yw
             ref, _ = op.run_cycle_batch(one, nthreads=1)
             yd, yw = ref["yd"].T.copy(), ref["yw"].T.copy()
         dt = time.perf_counter() - t0
-        line["cpu_baseline"] = {"value": ncyc / dt, "unit": UNIT, "cores": 1, "kind": "reference" if op.have_ref() else "port",
-                                "sample": "the same 184-cycle replay, one host thread (the reference's control loop is single-threaded), %.3f ms per cycle" % (1e3 * dt / ncyc)}
+        line["cpu_baseline"] = {"value": steps / dt, "unit": UNIT, "cores": 1, "kind": "reference" if op.have_ref() else "port",
+                                "sample": "the same %d timed cycles of the %d-cycle replay, one host thread (the reference's control loop is single-threaded), %.3f ms per cycle"
+                                          % (steps, ncyc, 1e3 * dt / steps)}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
     print(json.dumps(line))
     batch.close()
     return 0
@@ -194,7 +231,8 @@ def single_robot_replay(args):
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=30)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default 30; the whole %s, 184 cycles; for %s 400 closed-loop cycles = 1 s)" % (REPLAY, SWEEP))
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="standing_4096", choices=sorted(S.CONFIGS) + [SWEEP, REPLAY, ROLLOUT])
@@ -207,8 +245,16 @@ def parse_args():
     ap.add_argument("--fifo", action="store_true", help="index-order work queue (WBC_FIFO_DISPATCH) instead of longest-first")
     ap.add_argument("--plant", default="momentum", choices=["momentum", "dynamics"],
                     help="push_sweep: the plant that closes the loop -- the CoM-momentum integrator of SURVEY 8d row 5 (default) or forward dynamics with rigid contacts (SURVEY 8f-2)")
-    ap.add_argument("--sweep-cycles", type=int, default=None, help="push_sweep: closed-loop cycles of the rollout (default 400 = 1 s; --steps is ignored)")
+    ap.add_argument("--sweep-cycles", type=int, default=None, help="push_sweep: closed-loop cycles of the rollout, another name for --steps there")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (rank 0) as DIR/<name>.npy, float64, at most 64 MiB (a seeded sample of instances beyond)")
     args = ap.parse_args()
+    if args.workload == SWEEP and args.impl == "b200":
+        if None not in (args.steps, args.sweep_cycles) and args.steps != args.sweep_cycles:
+            ap.error("--steps and --sweep-cycles both set the push_sweep's timed cycles and disagree")
+        args.steps = args.sweep_cycles = next(v for v in (args.steps, args.sweep_cycles, 400) if v is not None)
+    elif args.steps is None and args.workload != REPLAY:       # the replay's default is its length, set where it is loaded
+        args.steps = 30
     args.warmup = max(args.warmup, 3)
     return args
 
@@ -279,9 +325,10 @@ def timed_device_loop(env, batch, step, steps, flush=True):
     return np.array([a.elapsed_time(b) for a, b in ev]), np.array(front_ms), np.array(solve_ms)
 
 
-def bench_batch(env, args, name, steps, warmup, per_gpu=None, cpu_baseline=False, fifo_steps=0, fifo=False, traj_on_device=False):
+def bench_batch(env, args, name, steps, warmup, per_gpu=None, cpu_baseline=False, fifo_steps=0, fifo=False, traj_on_device=False, dump=None):
     """One workload on this rank's shard: device-resident loop (`value`), end-to-end loop through wbc_cycle with host buffers
-    (`e2e`), roofline of the solve kernel, statistics gathered over the ranks.  Returns the JSON line (rank 0) or None."""
+    (`e2e`), roofline of the solve kernel, statistics gathered over the ranks.  Returns the JSON line (rank 0) or None.
+    dump: directory for the device-resident loop's last outputs (dump_outputs)."""
     import torch
     from wbc_quadruped_dob_b200 import api
     rank, world, dev = env.rank, env.world, env.dev
@@ -340,6 +387,7 @@ def bench_batch(env, args, name, steps, warmup, per_gpu=None, cpu_baseline=False
     step_ms, front_ms, solve_ms = timed_device_loop(env, batch, lambda it: step(dev_out), steps)
     env.barrier()
     t_wall = time.perf_counter() - t_wall0
+    last = {k: v.cpu().numpy() for k, v in dev_out.items()} if dump and rank == 0 else None     # the loops below overwrite dev_out
     tot_ms = float(step_ms.sum())
     launches = (3 if sweep else 2) * steps
     sweep_stats = None
@@ -461,10 +509,14 @@ def bench_batch(env, args, name, steps, warmup, per_gpu=None, cpu_baseline=False
                                       "state, so each solve's previous cost predicts this one exactly -- see --workload %s for a state that moves" % (fifo_steps, ROLLOUT)
         if sweep_stats:
             line["stats"]["sweep"] = sweep_stats
-        if world == 1 and cpu_baseline:
+        if world == 1 and cpu_baseline and not reference_built():
+            line["cpu_baseline"] = NO_CPU_BASELINE
+        elif world == 1 and cpu_baseline:
             kind, tot, _ = cpu_reference_run(sc, 1, 0, min(n, 4096), env.cores)
             line["cpu_baseline"] = {"value": min(n, 4096) / tot, "unit": UNIT, "cores": env.cores, "kind": kind,
                                     "sample": "one pass over the first %d instances of the workload, all %d host threads" % (min(n, 4096), env.cores)}
+        if last is not None:
+            dump_outputs(dump, last)
     batch.close()
     del dev_in, dev_out, stat_out
     torch.cuda.empty_cache()
@@ -495,7 +547,8 @@ def main():
         line = bench_push_sweep(env, args)
     else:
         line = bench_batch(env, args, args.workload, args.steps, args.warmup, per_gpu=args.per_gpu, cpu_baseline=not args.no_cpu_baseline,
-                           fifo_steps=0 if (args.no_also or args.fifo) else min(args.steps, 10), fifo=args.fifo, traj_on_device=args.traj_on_device)
+                           fifo_steps=0 if (args.no_also or args.fifo) else min(args.steps, 10), fifo=args.fifo, traj_on_device=args.traj_on_device,
+                           dump=args.dump_outputs)
         if args.workload == "standing_4096" and not args.no_also and not args.fifo and args.per_gpu is None:
             also = {}
             for name in ALSO:

@@ -67,6 +67,7 @@ def bench_trot_rollout(env, args):
     t_wall0 = time.perf_counter()
     step_ms, front_ms, solve_ms = run(False, stat_out)
     t_wall = time.perf_counter() - t_wall0
+    last = {k: stat_out[k].cpu().numpy() for k in dev_out} if args.dump_outputs and rank == 0 else None     # the fifo run overwrites them
     status = stat_out["status"].cpu().numpy()
     qp_info = stat_out["qp_info"].cpu().numpy()
     qp_flops = stat_out["qp_flops"].cpu().numpy()
@@ -129,10 +130,14 @@ def bench_trot_rollout(env, args):
                              "peak_source": "own DFMA microbenchmark in this process (MEASURED_PEAKS.json has no FP64 figure)"},
                 "stats": {"solver_failures": stats["solver_failures"], "mean_ncholesky": stats["sum_ncholesky"] / total,
                           "mean_outer_its": stats["sum_outer_its"] / total, "max_kkt_dim": stats["max_kkt_dim"], "wall_s_timed_region": t_wall}}
-        if not args.no_cpu_baseline and world == 1:
+        if not args.no_cpu_baseline and world == 1 and not B.reference_built():
+            line["cpu_baseline"] = B.NO_CPU_BASELINE
+        elif not args.no_cpu_baseline and world == 1:
             kind, tot, _ = B.cpu_reference_run(dict(host_sc[-1], obs_yd=zero6, obs_yw=zero6), 1, 0, min(n, 4096), env.cores)
             line["cpu_baseline"] = {"value": min(n, 4096) / tot, "unit": UNIT, "cores": env.cores, "kind": kind,
                                     "sample": "one pass over the first %d robots at the last cycle, all %d host threads" % (min(n, 4096), env.cores)}
+        if last is not None:
+            B.dump_outputs(args.dump_outputs, last)
     batch.close()
     return line
 
@@ -150,7 +155,7 @@ def bench_push_sweep(env, args):
     total = B.SWEEP_TOTAL if args.per_gpu is None else args.per_gpu * world
     lo, hi = sharding.shard_range(total, rank, world)
     n = hi - lo
-    cycles = args.sweep_cycles or 400
+    cycles = args.steps                    # --steps or --sweep-cycles, 400 = 1 s by default
     dyn_plant = getattr(args, "plant", "momentum") == "dynamics"
     tail = max(1, min(40, cycles // 4))
     sc = S.push_sweep(n=n, start=lo)
@@ -208,6 +213,8 @@ def bench_push_sweep(env, args):
     status = sout["status"].cpu().numpy()
     qp_info = sout["qp_info"].cpu().numpy()
     qp_flops = sout["qp_flops"].cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        B.dump_outputs(args.dump_outputs, {k: sout[k].cpu().numpy() for k in dout})
     # ---- per-gain reduction on the device, then ONE all-reduce of the packed vector (sums) and one of the maxima
     G = len(S.SWEEP_GAINS)
     ss = ss_acc / tail

@@ -168,28 +168,36 @@ def to_structs(sc, gravity=(0.0, 0.0, -9.8)):
     return arr
 
 
+def qp_solver(solver):
+    """The oracle's QP solver as a C function pointer: "ref" is the compiled reference ALGLIB; otherwise a ctypes function of the
+    wbc_qp_fn signature (QP_FN), for tests that must run where the reference ALGLIB is not built."""
+    if isinstance(solver, C._CFuncPtr):
+        return C.cast(solver, C.c_void_p)
+    if solver == "ref":
+        return C.cast(ref_lib().ref_qp_solve, C.c_void_p)
+    raise ValueError("the oracle's QP solver is the compiled reference ALGLIB or a wbc_qp_fn C function")
+
+
 def run_cycle_batch(sc, params=None, nthreads=1, solver="ref", gravity=(0.0, 0.0, -9.8)):
-    """Full oracle control cycle on every instance.  Returns (dict of [n][k] arrays, wall seconds)."""
+    """Full oracle control cycle on every instance.  Returns (dict of [n][k] arrays, wall seconds).  solver: see qp_solver."""
     params = params or default_params()
     n = sc["mode"].shape[0]
     arr = to_structs(sc, gravity)
     out = (Out * n)()
-    if solver != "ref":
-        raise ValueError("only the compiled reference ALGLIB may serve as the oracle's QP solver")
-    fn = C.cast(ref_lib().ref_qp_solve, C.c_void_p)
+    fn = qp_solver(solver)
     secs = oracle_lib().wbc_oracle_batch(C.byref(params), arr, n, nthreads, fn, out)
     v = np.frombuffer(out, dtype=np.dtype(Out))
     res = {k: np.array(v[k]) for k in ("tau", "w", "yd", "yw", "yg", "x", "qp_obj", "status", "ncholesky")}
     return res, secs
 
 
-def run_cycle_one(sc, i, params=None, gravity=(0.0, 0.0, -9.8)):
+def run_cycle_one(sc, i, params=None, gravity=(0.0, 0.0, -9.8), solver="ref"):
     """One instance with all intermediates (Out, Dyn, Qp ctypes structs)."""
     params = params or default_params()
     one = {k: (v[..., i:i + 1] if isinstance(v, np.ndarray) else v) for k, v in sc.items()}
     arr = to_structs(one, gravity)
     out, dyn, qp = Out(), Dyn(), Qp()
-    fn = C.cast(ref_lib().ref_qp_solve, C.c_void_p)
+    fn = qp_solver(solver)
     oracle_lib().wbc_oracle_cycle(C.byref(params), C.byref(arr[0]), fn, C.byref(out), C.byref(dyn), C.byref(qp))
     return out, dyn, qp
 
@@ -217,12 +225,12 @@ def assemble_only(sc, i, params=None, w=None, gravity=(0.0, 0.0, -9.8)):
     return dyn, qp
 
 
-def run_cycle_batch_gains(sc, params=None, nthreads=1):
+def run_cycle_batch_gains(sc, params=None, nthreads=1, solver="ref"):
     """run_cycle_batch for a scenario with a per-instance observer gain sc["obs_gain"] (BASELINE config 5):
     the oracle's gain is a scalar parameter like the reference's literal (main.cpp:708), so instances are grouped."""
     gains = sc.get("obs_gain")
     if gains is None:
-        return run_cycle_batch(sc, params, nthreads)
+        return run_cycle_batch(sc, params, nthreads, solver)
     n = sc["mode"].shape[0]
     res, secs = None, 0.0
     for gval in np.unique(gains):
@@ -231,7 +239,7 @@ def run_cycle_batch_gains(sc, params=None, nthreads=1):
         p = default_params() if params is None else params
         p2 = Params.from_buffer_copy(p)
         p2.obs_gain = float(gval)
-        r, s = run_cycle_batch(sub, p2, nthreads)
+        r, s = run_cycle_batch(sub, p2, nthreads, solver)
         secs += s
         if res is None:
             res = {k: np.zeros((n,) + v.shape[1:], dtype=v.dtype) for k, v in r.items()}

@@ -33,3 +33,16 @@ extern "C" int emu_qp_solve(const double* Q, const double* c, const double* L, i
     if (dstats) dstats[0] = st.flops;
     return st.termination == 2 ? 0 : -1;
 }
+
+// The CPU oracle's QP callback (wbc_qp_fn, oracle/wbc_oracle.h): the reference settings (1e-2, 1e4, 5; lopt.cpp:101, 138) and
+// the literal multiplier update (kkt_mode 0), not the reduced form the device code runs by default.  Lets the oracle's control
+// cycle run where the reference ALGLIB is not built; this restatement's parity with it is pinned by tests/golden/qp_*.npz.
+extern "C" int emu_qp_solve_oracle(const double* Q, const double* c, const double* L, int nrows, int neq,
+                                   double* x, int* ncholesky, int* termtype)
+{
+    int ist[8] = {0};
+    int rc = emu_qp_solve(Q, c, L, nrows, neq, 1.0e-2, 1.0e+4, 5, 0, x, ist, nullptr);
+    if (ncholesky) *ncholesky = ist[1];
+    if (termtype) *termtype = ist[0];
+    return rc;
+}

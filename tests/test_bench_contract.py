@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -42,3 +43,36 @@ def test_b200_arm_json_line():
     assert d["stats"]["solver_failures"] == 0
     assert "sm_mhz" in d["clocks"] and "reasons" in d["clocks"]
     assert "4096" in d["config"]["workload"]
+
+
+def test_dump_outputs_takes_one_seeded_sample_of_instances_above_the_limit(tmp_path, monkeypatch):
+    import bench
+    n = 1000
+    tau, w = np.arange(12 * n, dtype=np.float64).reshape(12, n), -np.arange(6 * n, dtype=np.float64).reshape(6, n)
+    bench.dump_outputs(str(tmp_path / "all"), {"tau": tau, "w": w})
+    assert sorted(os.listdir(tmp_path / "all")) == ["tau.npy", "w.npy"]
+    assert np.array_equal(np.load(tmp_path / "all" / "tau.npy"), tau)
+    monkeypatch.setattr(bench, "DUMP_LIMIT", 40000)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"tau": tau, "w": w})
+    keep = np.load(tmp_path / "a" / "instances.npy")
+    assert np.array_equal(keep, np.load(tmp_path / "b" / "instances.npy"))
+    assert 0 < keep.size < n and sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= 40000
+    k = keep.astype(np.int64)
+    assert np.array_equal(np.load(tmp_path / "a" / "tau.npy"), tau[:, k]) and np.array_equal(np.load(tmp_path / "a" / "w.npy"), w[:, k])
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_timed_loops_last_step_and_repeat_run_to_run(tmp_path):
+    args = ["--warmup", "3", "--no-cpu-baseline", "--no-also"]
+    d = _run(args + ["--steps", "2", "--dump-outputs", str(tmp_path / "a")])
+    _run(args + ["--steps", "2", "--dump-outputs", str(tmp_path / "b")])
+    d3 = _run(args + ["--steps", "3", "--dump-outputs", str(tmp_path / "c")])
+    assert d["steps"] == 2 and d3["steps"] == 3
+    # the observer state is chained from cycle to cycle: one more timed step moves the estimate, so the dump is the last step's
+    assert not np.array_equal(np.load(tmp_path / "a" / "w.npy"), np.load(tmp_path / "c" / "w.npy"))
+    assert sorted(os.listdir(tmp_path / "a")) == ["tau.npy", "w.npy"]
+    for f, k in (("tau.npy", 12), ("w.npy", 6)):
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype == np.float64 and a.shape == (k, 4096) and np.isfinite(a).all() and np.abs(a).max() > 0
+        assert np.array_equal(a, b), f

@@ -44,10 +44,10 @@ def test_solver_restatement_matches_reference_alglib_golden(emu, name):
         assert flops > 0
 
 
-def test_device_code_matches_oracle_on_fresh_seed(emu, oracle, have_ref):
+def test_device_code_matches_oracle_on_fresh_seed(emu, oracle, oracle_qp):
     sc = S.make(160, mode_mix=(0.34, 0.33, 0.33), pushes=True, terrain=True, seed=1234)
     got = emu.cycle(sc)
-    ref, _ = oracle.run_cycle_batch(sc, nthreads=8)
+    ref, _ = oracle.run_cycle_batch(sc, nthreads=8, solver=oracle_qp)
     util.check_cycle_parity(got, ref, what="seed 1234")
 
 

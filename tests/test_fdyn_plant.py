@@ -66,7 +66,7 @@ def test_energy_balance_under_hard_contacts(oracle):
     assert np.abs((e1 - e0) - work).max() < 2e-2 * max(1e-3, np.abs(work).max()) + 1e-5, (e1 - e0, work)
 
 
-def test_standing_torques_hold_the_robot_still(oracle, have_ref):
+def test_standing_torques_hold_the_robot_still(oracle, oracle_qp):
     """The controller's own torques through the plant: a robot at rest on four feet, desired CoM = actual CoM, stays at rest."""
     n = 8
     sc = _standing(n)
@@ -78,7 +78,7 @@ def test_standing_torques_hold_the_robot_still(oracle, have_ref):
     P = oracle.default_params(observer_enabled=0)
     cur = {k: (v.copy() if isinstance(v, np.ndarray) else v) for k, v in sc.items()}
     for it in range(40):
-        res, _ = oracle.run_cycle_batch(cur, P, nthreads=8)
+        res, _ = oracle.run_cycle_batch(cur, P, nthreads=8, solver=oracle_qp)
         nxt, diag = oracle.fdyn_step(cur, res["tau"].T, np.zeros((6, n)), params=P, nsub=5, gamma=100.0)
         for k in ("base_pos", "base_rot", "base_rpy", "base_vel", "q", "dq", "foot_force"):
             cur[k] = nxt[k]
@@ -185,7 +185,7 @@ def trot_in_place_targets(anchor, mode, s, period_s, height):
 
 
 @pytest.mark.gpu
-def test_closed_loop_trot_under_pushes_through_the_dynamics_plant(gpu_batch, have_ref):
+def test_closed_loop_trot_under_pushes_through_the_dynamics_plant(gpu_batch, oracle_qp):
     """4096 robots trotting in place (stance, swing{BR,FL}, stance, swing{BL,FR}; 40 cycles per phase, 3 cm foot lift), the
     controller closed through the forward-dynamics plant for 320 cycles with a force_plugin-style horizontal push during the second
     and third phase (fp.cpp:203-310).  Contact modes, active sets and joint states all move.  Every robot stays up and no solve
@@ -224,16 +224,16 @@ def test_closed_loop_trot_under_pushes_through_the_dynamics_plant(gpu_batch, hav
             din["mode"] = torch.full((n,), mode, dtype=torch.int32, device=dev)
         sp, sv, sa = trot_in_place_targets(anchor, mode, (c % P) / P, P * 0.0025, height)
         din["sw_des_pos"].copy_(torch.from_numpy(sp)); din["sw_des_vel"].copy_(torch.from_numpy(sv)); din["sw_des_acc"].copy_(torch.from_numpy(sa))
-        if have_ref and c % 20 == 7:
+        if c % 20 == 7:
             # teacher-forced check: the oracle on the states the loop is in right now (observer state included)
             yd, yw = gpu_batch.get_observer_state(n)
             one = {k: din[k].cpu().numpy()[..., sub] for k in din if k not in ("mode",)}
             one["mode"] = np.full(sub.size, mode, dtype=np.int32)
             one["obs_yd"], one["obs_yw"] = yd[:, sub], yw[:, sub]
-            ref, _ = O.run_cycle_batch(one, nthreads=8)
+            ref, _ = O.run_cycle_batch(one, nthreads=8, solver=oracle_qp)
         gpu_batch.cycle_device(din, dout, n, n)
         fails += int((dout["status"] != 0).sum().item())
-        if have_ref and c % 20 == 7:
+        if c % 20 == 7:
             tau = dout["tau"].cpu().numpy()[:, sub]
             ok = ref["status"] == 0
             worst_tau = max(worst_tau, float((np.abs(tau[:, ok] - ref["tau"].T[:, ok]) / (1.0 + np.abs(ref["tau"].T[:, ok]))).max()))
@@ -253,11 +253,10 @@ def test_closed_loop_trot_under_pushes_through_the_dynamics_plant(gpu_batch, hav
     # commanded to zero force and the plant may answer with a slightly negative one; it must stay a rare event of a fraction of a newton
     assert fzmin > -1.0 and pulls < 1e-2 * n * 8 * P
     assert np.abs(pos - base0).max() < 0.08 and np.abs(rpy - sc["base_rpy"]).max() < 0.15 and np.abs(vel).max() < 1.0
-    if have_ref:
-        assert checked > 900 and worst_tau < 1e-6
+    assert checked > 900 and worst_tau < 1e-6
 
 
-def test_oracle_closed_loop_through_the_dynamics_plant_estimates_the_push(oracle, have_ref):
+def test_oracle_closed_loop_through_the_dynamics_plant_estimates_the_push(oracle, oracle_qp):
     """BASELINE config 5 through the forward-dynamics plant (bench.py --workload push_sweep --plant dynamics), on the oracle: robots
     holding their pose under a constant horizontal push.  The estimate settles on the push in x and y; in z it settles on
     m (g_acc - |gravity|) = +0.21 N, the reference's two gravity constants (9.81 in estimate(), main.cpp:702; 9.8 in the dynamics,
@@ -270,7 +269,7 @@ def test_oracle_closed_loop_through_the_dynamics_plant_estimates_the_push(oracle
     sub["com_des_pos"] = np.vstack([com0.T, sub["base_rpy"]])
     push = sub["push"]
     for c in range(160):
-        res, _ = oracle.run_cycle_batch_gains(sub)
+        res, _ = oracle.run_cycle_batch_gains(sub, solver=oracle_qp)
         assert (res["status"] == 0).all()
         sub["obs_yd"], sub["obs_yw"] = res["yd"].T.copy(), res["yw"].T.copy()
         nxt, diag = oracle.fdyn_step(sub, res["tau"].T, push, nsub=5, gamma=100.0)

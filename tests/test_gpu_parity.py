@@ -41,10 +41,10 @@ def test_trot_replay_single_robot_chained_observer(gpu_batch):
 
 
 @pytest.mark.parametrize("cfg,n", [("standing_4096", 4096), ("trot_65536", 3000), ("mixed_terrain_1m", 3000)])
-def test_cycle_matches_oracle_on_baseline_configs(gpu_batch, oracle, have_ref, cfg, n):
+def test_cycle_matches_oracle_on_baseline_configs(gpu_batch, oracle, oracle_qp, cfg, n):
     sc = S.make_config(cfg, n=n)
     got = _run(gpu_batch, sc)
-    ref, _ = oracle.run_cycle_batch(sc, nthreads=16)
+    ref, _ = oracle.run_cycle_batch(sc, nthreads=16, solver=oracle_qp)
     worst = util.check_cycle_parity(got, ref, what=cfg)
     print(cfg, "worst torque rel err", worst)
 
@@ -125,12 +125,12 @@ def test_solver_failure_is_reported(gpu_batch):
     assert status[0] == 0 and status[1] == -9
 
 
-def test_edge_cases_empty_single_and_ragged(gpu_batch, oracle, have_ref):
+def test_edge_cases_empty_single_and_ragged(gpu_batch, oracle, oracle_qp):
     sc = S.make(0)
     out = gpu_batch.cycle(sc, n=0)
     assert out["tau"].shape == (12, 0)
     sc = S.make(37, mode_mix=(0.3, 0.3, 0.4), pushes=True, seed=5)
-    ref, _ = oracle.run_cycle_batch(sc, nthreads=4)
+    ref, _ = oracle.run_cycle_batch(sc, nthreads=4, solver=oracle_qp)
     # ragged: n smaller than the arrays' leading dimension
     gpu_batch.set_observer_state(sc["obs_yd"], sc["obs_yw"])
     got = gpu_batch.cycle(sc, n=21)
@@ -143,7 +143,7 @@ def test_edge_cases_empty_single_and_ragged(gpu_batch, oracle, have_ref):
         gpu_batch.cycle(S.make(8), n=gpu_batch.max_batch + 1)
 
 
-def test_observer_disabled_reproduces_shipped_reference(gpu_batch, oracle, have_ref):
+def test_observer_disabled_reproduces_shipped_reference(gpu_batch, oracle, oracle_qp):
     """The shipped binary never calls estimate() (main.cpp:1029): w = 0 and the state does not move."""
     sc = S.make(64, mode_mix=(0.5, 0.25, 0.25), seed=8)
     p = api.default_params()
@@ -154,7 +154,7 @@ def test_observer_disabled_reproduces_shipped_reference(gpu_batch, oracle, have_
         yd, yw = gpu_batch.get_observer_state(64)
     finally:
         gpu_batch.set_params(api.default_params())
-    ref, _ = oracle.run_cycle_batch(sc, params=oracle.default_params(observer_enabled=0), nthreads=4)
+    ref, _ = oracle.run_cycle_batch(sc, params=oracle.default_params(observer_enabled=0), nthreads=4, solver=oracle_qp)
     util.check_cycle_parity(got, ref, what="observer off")
     assert np.all(got["w"] == 0.0) and np.array_equal(yd, sc["obs_yd"]) and np.array_equal(yw, sc["obs_yw"])
 

@@ -94,7 +94,7 @@ def test_nan_records_terminate(gpu_batch):
     assert not x[1:].any() and np.isfinite(x).all()
 
 
-def test_update_stage_fgrf_and_wcom_des_match_oracle(gpu_batch, oracle, have_ref):
+def test_update_stage_fgrf_and_wcom_des_match_oracle(gpu_batch, oracle, oracle_qp):
     """The two stage outputs the round-1 stage test left unasserted: Fgrf (main.cpp:1022-1026) and Wcom_des (1012-1032), with
     a non-zero observer state in the ctx (wbc_debug_update works on a copy of it)."""
     n = 48
@@ -104,12 +104,12 @@ def test_update_stage_fgrf_and_wcom_des_match_oracle(gpu_batch, oracle, have_ref
     yd, yw = gpu_batch.get_observer_state(n)
     assert np.array_equal(yd, sc["obs_yd"]) and np.array_equal(yw, sc["obs_yw"])       # untouched
     for i in range(0, n, 5):
-        out, dyn, qp = oracle.run_cycle_one(sc, i)
+        out, dyn, qp = oracle.run_cycle_one(sc, i, solver=oracle_qp)
         assert np.abs(dbg["Fgrf"][:, i] - np.array(qp.Fgrf)).max() <= 1e-11 * max(1.0, np.abs(np.array(qp.Fgrf)).max())
         assert np.abs(dbg["Wcom_des"][:, i] - np.array(qp.Wcom_des)).max() <= 1e-9 * max(1.0, np.abs(np.array(qp.Wcom_des)).max())
 
 
-def test_trot_rollout_matches_oracle_every_cycle(gpu_batch, oracle, have_ref):
+def test_trot_rollout_matches_oracle_every_cycle(gpu_batch, oracle, oracle_qp):
     """1024 robots x 184 cycles of the evolving-state herd (contact modes flip, active sets drift, pushes come and go): the
     GPU runs free with its observer state in the ctx, the oracle runs free with its own; torques 1e-6, w 1e-9 every cycle."""
     n, cycles = 1024, 184
@@ -121,7 +121,7 @@ def test_trot_rollout_matches_oracle_every_cycle(gpu_batch, oracle, have_ref):
         sc = S.trot_rollout(n, t)
         got = gpu_batch.cycle(sc)
         ref_in = dict(sc, obs_yd=yd, obs_yw=yw)
-        ref, _ = oracle.run_cycle_batch(ref_in, nthreads=32)
+        ref, _ = oracle.run_cycle_batch(ref_in, nthreads=32, solver=oracle_qp)
         worst = max(worst, util.check_cycle_parity(got, ref, what="rollout cycle %d" % t))
         yd, yw = np.ascontiguousarray(ref["yd"].T), np.ascontiguousarray(ref["yw"].T)
         nch_equal.append(np.mean(got["qp_info"][0] == ref["ncholesky"]))
@@ -135,7 +135,7 @@ def test_trot_rollout_matches_oracle_every_cycle(gpu_batch, oracle, have_ref):
     print("rollout: worst torque rel err %.2e over %d robot-cycles, %d mode changes, ncholesky equal on %.2f%%" % (worst, n * cycles, flips, 100 * np.mean(nch_equal)))
 
 
-def test_sweep_400_cycles_teacher_forced(gpu_batch, oracle, have_ref):
+def test_sweep_400_cycles_teacher_forced(gpu_batch, oracle, oracle_qp):
     """BASELINE config 5 for the full second: a sub-grid (2 directions x 2 magnitudes x all 8 observer gains x 2 states = 64
     instances) through 400 closed-loop cycles on the GPU (wbc_cycle + wbc_plant_step); the oracle is fed the GPU's inputs every
     cycle.  w within 1e-9 throughout; at the end the estimate has converged for every gain >= 10 (below 1e-2 relative)."""
@@ -147,7 +147,7 @@ def test_sweep_400_cycles_teacher_forced(gpu_batch, oracle, have_ref):
     gpu_batch.set_observer_state(cur["obs_yd"], cur["obs_yw"])
     for it in range(400):
         got = gpu_batch.cycle(cur)
-        ref, _ = oracle.run_cycle_batch_gains(cur, P, nthreads=16)
+        ref, _ = oracle.run_cycle_batch_gains(cur, P, nthreads=16, solver=oracle_qp)
         util.check_cycle_parity(got, ref, what="sweep cycle %d" % it)
         yd, yw = gpu_batch.get_observer_state(n)
         gpu_batch.plant_step(cur["base_pos"], cur["base_vel"], cur["push"], foot_force=cur["foot_force"], x=got["x"])
@@ -160,27 +160,29 @@ def test_sweep_400_cycles_teacher_forced(gpu_batch, oracle, have_ref):
 
 
 @pytest.mark.parametrize("cfg,n", [("trot_65536", 65536), ("mixed_terrain_1m", 131072)])
-def test_big_configs_against_live_oracle_every_instance(oracle, have_ref, cfg, n):
+def test_big_configs_against_live_oracle_every_instance(oracle, oracle_qp, cfg, n):
     """EVERY instance of BASELINE config 3 (65 536) and of one GPU's shard of config 4 (131 072 of the 1 M) against the live oracle
-    (reference ALGLIB; 5 + 10 s on the host threads): tolerances as everywhere, plus the histogram of Cholesky-count differences
-    and the number of torque deviations above 1e-7 (SURVEY.md Appendix F predicted about one flipped decision per 2000 swing
-    solves; observed: none above 1e-7 in 196 608)."""
+    (5 + 10 s on the host threads): tolerances as everywhere, plus the histogram of Cholesky-count differences and the number of
+    torque deviations above 1e-7.  With the reference ALGLIB as the oracle's QP solver (SURVEY.md Appendix F predicted about one
+    flipped decision per 2000 swing solves; observed: none above 1e-7 in 196 608).  Where it is not built the oracle solves with
+    the restatement's literal multiplier update (`oracle_qp`), and the Cholesky counts compare the device's reduced update with it."""
     sc = S.make_config(cfg, n=n)
     batch = api.WbcBatch(max_batch=n)
     batch.set_observer_state(sc["obs_yd"], sc["obs_yw"])
     got = batch.cycle(sc)
     batch.close()
-    ref, _ = oracle.run_cycle_batch(sc, nthreads=32)
+    ref, _ = oracle.run_cycle_batch(sc, nthreads=32, solver=oracle_qp)
     worst = util.check_cycle_parity(got, ref, what=cfg)
     d = got["qp_info"][0].astype(int) - ref["ncholesky"].astype(int)
     vals, cnts = np.unique(d, return_counts=True)
     et = util.rel_rows(got["tau"].T, ref["tau"])
-    print("%s: worst torque rel err %.2e; torque deviations > 1e-7: %d of %d; ncholesky(GPU) - ncholesky(ALGLIB) histogram %s"
-          % (cfg, worst, int((et > 1e-7).sum()), n, dict(zip(vals.tolist(), cnts.tolist()))))
+    print("%s: worst torque rel err %.2e; torque deviations > 1e-7: %d of %d; ncholesky(GPU) - ncholesky(%s) histogram %s"
+          % (cfg, worst, int((et > 1e-7).sum()), n, "reference ALGLIB" if oracle_qp == "ref" else "restatement",
+             dict(zip(vals.tolist(), cnts.tolist()))))
     assert np.mean(d == 0) >= 0.99
 
 
-def test_staged_and_monolithic_solver_kernels_agree_bit_for_bit():
+def test_staged_and_monolithic_solver_kernels_agree_bit_for_bit(tmp_path):
     """wbc_solve_staged_kernel (stage tasks handed from warp to warp) against wbc_solve_kernel (one warp per solve): same
     arithmetic, so every output bit for bit."""
     import os
@@ -194,7 +196,7 @@ def test_staged_and_monolithic_solver_kernels_agree_bit_for_bit():
             "np.savez(sys.argv[1], **{k: o[k] for k in ('tau','w','x','qp_obj','status','qp_info')}, **{'2' + k: o2[k] for k in ('tau','w','x')})")
     outs = []
     for solver in ("staged", "mono"):
-        path = "/tmp/wbc_ab_%s.npz" % solver
+        path = str(tmp_path / ("wbc_ab_%s.npz" % solver))
         env = dict(os.environ, WBC_SOLVER=solver)
         subprocess.check_call([sys.executable, "-c", code, path], env=env, cwd=util.ROOT)
         outs.append(np.load(path))

@@ -3,7 +3,10 @@ explicit gain, second-order recursion through `ygamma`, and the foot-wrench map 
 
 PARITY UNPINNED: the reference never calls ESTIMATOR_SEM (SURVEY.md 2, row 4) and holds no vectors for it; the oracle restates
 estimator_sem.cpp's lines, numpy's pinv is the pseudo-inverse getw3 takes from Eigen, and the recursions are also checked against
-their closed-form responses.  CPU tests run the device headers through the host emulation; GPU tests go through the C ABI."""
+their closed-form responses.  CPU tests run the device headers through the host emulation; GPU tests go through the C ABI.
+
+The chained-cycle tests run the oracle with the `oracle_qp` fixture's QP solver (the restatement where the reference ALGLIB is not
+built): what they check is the observer and how its estimate enters the QP and the torques, not the solve."""
 import numpy as np
 import pytest
 
@@ -55,14 +58,14 @@ def test_second_order_recursion_has_the_closed_form_response():
 
 
 @pytest.mark.parametrize("order,form", FORMS)
-def test_emulated_device_code_matches_the_oracle_over_chained_cycles(order, form):
+def test_emulated_device_code_matches_the_oracle_over_chained_cycles(order, form, oracle_qp):
     emu = util.Emu()
     sc = S.make(24, mode_mix=(0.4, 0.3, 0.3), pushes=True, terrain=False, seed=21)
     sc["obs_yg"] = np.zeros((6, 24))
     pe, po = _params(order, form, emu=True), _oracle_params(order, form)
     rng = np.random.default_rng(5)
     for cyc in range(6):
-        ref, _ = O.run_cycle_batch(sc, params=po)
+        ref, _ = O.run_cycle_batch(sc, params=po, solver=oracle_qp)
         got = emu.cycle(sc, params=pe)
         scale = 1.0 + np.abs(ref["w"]).max()
         assert np.max(np.abs(got["w"] - ref["w"].T)) < 1e-9 * scale, (cyc, order, form)
@@ -93,7 +96,7 @@ def test_emulated_foot_wrench_map_matches_getw3_and_reproduces_the_wrench():
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("order,form", FORMS)
-def test_gpu_observer_forms_match_the_oracle_over_chained_cycles(order, form):
+def test_gpu_observer_forms_match_the_oracle_over_chained_cycles(order, form, oracle_qp):
     from wbc_quadruped_dob_b200 import api
     n = 512
     sc = S.make(n, mode_mix=(0.4, 0.3, 0.3), pushes=True, terrain=False, seed=23)
@@ -104,7 +107,7 @@ def test_gpu_observer_forms_match_the_oracle_over_chained_cycles(order, form):
     rng = np.random.default_rng(6)
     worst_w = worst_tau = 0.0
     for cyc in range(8):
-        ref, _ = O.run_cycle_batch(sc, params=po, nthreads=8)
+        ref, _ = O.run_cycle_batch(sc, params=po, nthreads=8, solver=oracle_qp)
         got = batch.cycle(sc, want=("status", "w3"))
         worst_w = max(worst_w, float(np.max(np.abs(got["w"] - ref["w"].T)) / (1.0 + np.abs(ref["w"]).max())))
         ok = (ref["status"] == 0) & (got["status"] == 0)

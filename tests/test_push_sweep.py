@@ -31,7 +31,7 @@ def test_sweep_grid_layout():
     assert full["mode"].shape[0] == 4 and full["grid"][:, -1].tolist() == [15, 7, 7, 255]
 
 
-def test_oracle_closed_loop_rejects_the_push(oracle, have_ref):
+def test_oracle_closed_loop_rejects_the_push(oracle, oracle_qp):
     """Observer estimate converges to the injected wrench like exp(-k t) (main.cpp:707-719 is a first-order filter with
     gain k), faster for larger k, and the closed loop stays bounded."""
     sc = S.push_sweep(n=None, **SMALL)
@@ -41,7 +41,7 @@ def test_oracle_closed_loop_rejects_the_push(oracle, have_ref):
     scale = np.abs(push).max(axis=1)
     err = []
     for it in range(120):
-        res, _ = oracle.run_cycle_batch_gains(cur, P, nthreads=8)
+        res, _ = oracle.run_cycle_batch_gains(cur, P, nthreads=8, solver=oracle_qp)
         assert (res["status"] == 0).all()
         err.append(np.abs(res["w"] - push).max(axis=1) / scale)
         pos, vel, ff = oracle.plant_step(cur, cur["push"], x=res["x"], params=P)
@@ -60,7 +60,7 @@ def test_oracle_closed_loop_rejects_the_push(oracle, have_ref):
 
 
 @pytest.mark.gpu
-def test_sweep_rollout_matches_oracle_every_cycle(gpu_batch, oracle, have_ref):
+def test_sweep_rollout_matches_oracle_every_cycle(gpu_batch, oracle, oracle_qp):
     """GPU closed loop (wbc_cycle + wbc_plant_step, per-instance observer gains, observer state kept in the ctx); the
     oracle is teacher-forced with the GPU's inputs each cycle.  w within 1e-9, torques 1e-6, plant state 1e-10."""
     sc = S.push_sweep(n=None, **SMALL)
@@ -70,7 +70,7 @@ def test_sweep_rollout_matches_oracle_every_cycle(gpu_batch, oracle, have_ref):
     gpu_batch.set_observer_state(cur["obs_yd"], cur["obs_yw"])
     for it in range(40):
         got = gpu_batch.cycle(cur)
-        ref, _ = oracle.run_cycle_batch_gains(cur, P, nthreads=8)
+        ref, _ = oracle.run_cycle_batch_gains(cur, P, nthreads=8, solver=oracle_qp)
         util.check_cycle_parity(got, ref, what="sweep cycle %d" % it)
         yd, yw = gpu_batch.get_observer_state(n)
         assert np.abs(yd.T - ref["yd"]).max() <= util.TOL_OBS * max(1.0, np.abs(ref["yd"]).max())

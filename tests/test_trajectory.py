@@ -53,7 +53,7 @@ def test_device_sampling_code_matches_oracle(emu, oracle, nseg):
 
 
 @pytest.mark.gpu
-def test_gpu_sampling_matches_oracle_and_feeds_the_cycle(gpu_batch, oracle, have_ref):
+def test_gpu_sampling_matches_oracle_and_feeds_the_cycle(gpu_batch, oracle, oracle_qp):
     n = 3000
     sc = S.make(n, mode_mix=(0.3, 0.35, 0.35), pushes=True, terrain=True, seed=33)
     tr = S.make_trajectory(sc, nseg=4, seed=9)
@@ -77,7 +77,7 @@ def test_gpu_sampling_matches_oracle_and_feeds_the_cycle(gpu_batch, oracle, have
     # ... and agrees with the CPU controller run on the oracle's samples
     sc_o = dict(sc)
     sc_o.update(ref)
-    want, _ = oracle.run_cycle_batch(sc_o, nthreads=8)
+    want, _ = oracle.run_cycle_batch(sc_o, nthreads=8, solver=oracle_qp)
     util.check_cycle_parity(dev, want, what="sampled trajectory")
 
 

@@ -144,6 +144,12 @@ class Emu:
                              epsx, rho, outerits, kkt_mode, x.ctypes.data_as(_dp), ist, ds)
         return x, list(ist), ds[0]
 
+    def oracle_qp_fn(self):
+        """The solver restatement as the oracle's QP solver (emu_qp_solve_oracle: reference settings, literal multiplier update),
+        a C function the oracle calls from all its threads.  Its parity with the reference ALGLIB is pinned by
+        tests/golden/qp_*.npz (test_emulation.py)."""
+        return self.qp.emu_qp_solve_oracle
+
 
 def check_cycle_parity(got, ref, n=None, what=""):
     """got: dict of SoA [k, n] arrays from the CUDA path / emulation; ref: oracle dict of [n, k] arrays."""
