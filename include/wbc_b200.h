@@ -42,6 +42,8 @@ extern "C" {
 /* per-instance status words (wbc_outputs.status) for inputs the cycle refuses to process */
 #define WBC_ST_BAD_MODE (-20)    /* contact mode outside {0, 1, 2} */
 #define WBC_ST_NONFINITE (-21)   /* a NaN or infinity among the inputs, or produced from them before the QP */
+#define WBC_ST_INFEASIBLE (-22)  /* exact mode (WBC_QP_EXACT): the constraints admit no point (row-scaled residuals) */
+#define WBC_ST_NOT_PD (-23)      /* exact mode: H (the lower triangle of Q mirrored) is not positive definite */
 
 /* contact modes: which feet swing */
 #define WBC_MODE_STANCE 0        /* main.cpp:979-1148, 1516-1675 */
@@ -58,6 +60,15 @@ extern "C" {
                                     express lanes, DESIGN.md 4.2); the order never changes a result, only when the batch's tail ends. */
 #define WBC_SAMPLED_TRAJ 16u     /* wbc_cycle: com_des_* and sw_des_* come from the last wbc_sample_trajectory(out = NULL) on this ctx;
                                   * those six wbc_inputs pointers are ignored (may be NULL) and are not copied from the host */
+#define WBC_QP_EXACT 32u         /* wbc_cycle / wbc_qp_solve: solve each QP to its exact optimum with a Goldfarb-Idnani dual active-set
+                                  * solver (one warp per QP, wbc_solve_exact_kernel) instead of the DENSE-AUL restatement at the
+                                  * reference's settings; qp_epsx, qp_rho, qp_outerits and qp_literal_kkt are ignored.  Status 0 means
+                                  * every row is satisfied to 1e-12 row-scaled and every active inequality multiplier is >= 0;
+                                  * WBC_ST_INFEASIBLE, WBC_ST_NOT_PD, or -100 (iteration cap 2 nrows + 30) otherwise, with x = 0.
+                                  * qp_info in this mode: [0] factorisations (1), [1] rows added to the active set (equalities
+                                  * included), [2] rows dropped, [3] active inequality rows, [4] active-set size, [5] flags: 256 always
+                                  * (exact mode), | 512 a dependent consistent equality was skipped, | 1024 a violated row depended on
+                                  * the active set and dual steps were taken; [6], [7] 0.  qp_flops: the exact solver's own count. */
 #define WBC_HOST_SLAB 8u         /* (host pointers) the input arrays are carved, in wbc_inputs field order, from ONE page-locked
                                   * allocation with ld == n: adjacent fields are moved with a single copy */
 
@@ -242,7 +253,8 @@ int wbc_last_launches(wbc_ctx* ctx);
 /* Launch shape of the persistent solver kernel: resident CTAs (= warps) per SM as the occupancy calculator reports them
  * for this device, dynamic shared memory per CTA in bytes, and the grid of the last wbc_cycle (before any: SMs x resident
  * CTAs; small batches are launched with fewer CTAs per SM), and which solver kernel the last wbc_cycle ran (0: one warp per
- * solve, 1: stage tasks with SM roles -- chosen by batch size, see DESIGN.md).  Any pointer may be NULL.
+ * solve, 1: stage tasks with SM roles -- chosen by batch size, see DESIGN.md; 2: the exact-mode kernel of WBC_QP_EXACT, whose
+ * resident CTAs per SM and shared memory are then reported).  Any pointer may be NULL.
  * Measurement only (bench.py reports it beside the roofline); the reference has no counterpart. */
 int wbc_solver_shape(wbc_ctx* ctx, int* ctas_per_sm, int* smem_bytes, int* grid, int* stage_tasks);
 /* Per-warp profile of the last solver launch when the ctx was created with WBC_STAGE_PROF=1 in the environment: rows of 12

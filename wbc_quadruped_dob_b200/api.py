@@ -20,7 +20,9 @@ import numpy as np
 from . import build as _build
 
 MODE_STANCE, MODE_SWING_BR_FL, MODE_SWING_BL_FR = 0, 1, 2
-HOST_PTRS, DEVICE_PTRS, NO_SYNC, FIFO_DISPATCH, HOST_SLAB, SAMPLED_TRAJ = 0, 1, 2, 4, 8, 16
+HOST_PTRS, DEVICE_PTRS, NO_SYNC, FIFO_DISPATCH, HOST_SLAB, SAMPLED_TRAJ, QP_EXACT = 0, 1, 2, 4, 8, 16, 32
+ST_BAD_MODE, ST_NONFINITE, ST_INFEASIBLE, ST_NOT_PD = -20, -21, -22, -23
+SOLVER_KERNELS = {0: "wbc_solve_kernel", 1: "wbc_solve_staged_kernel", 2: "wbc_solve_exact_kernel"}
 
 _dp = C.POINTER(C.c_double)
 _ip = C.POINTER(C.c_int)
@@ -303,9 +305,10 @@ class WbcBatch:
         out["_slab"] = True          # cycle() passes WBC_HOST_SLAB
         return out
 
-    def cycle(self, sc, n=None, want=("x", "qp_obj", "status", "qp_info", "qp_flops"), out=None, sampled_traj=False):
+    def cycle(self, sc, n=None, want=("x", "qp_obj", "status", "qp_info", "qp_flops"), out=None, sampled_traj=False, exact=False):
         """One control cycle on HOST (numpy) SoA inputs; returns a dict of numpy arrays [k, n].  `out`: preallocated
-        result arrays to fill (e.g. page-locked ones from pinned()); its keys decide what is returned."""
+        result arrays to fill (e.g. page-locked ones from pinned()); its keys decide what is returned.  exact=True: solve each
+        QP to its exact optimum (WBC_QP_EXACT, the dual active-set solver) instead of DENSE-AUL at the reference's settings."""
         keep = []
         n = int(sc["mode"].shape[0]) if n is None else int(n)
         ins = self._inputs_struct(sc, n, keep, skip=TRAJ_FIELDS if sampled_traj else ())
@@ -321,13 +324,13 @@ class WbcBatch:
         for k in ("tau", "w", "x", "qp_obj", "status", "qp_info", "qp_flops", "w3"):
             setattr(o, k, _ptr(out.get(k)))
         o.ld = max(n, 1)
-        _check(self.lib.wbc_cycle(self.h, n, C.byref(ins), C.byref(o), None, HOST_PTRS | (FIFO_DISPATCH if self.fifo_dispatch else 0) | (HOST_SLAB if sc.get("_slab") else 0) | (SAMPLED_TRAJ if sampled_traj else 0)), "wbc_cycle")
+        _check(self.lib.wbc_cycle(self.h, n, C.byref(ins), C.byref(o), None, HOST_PTRS | (FIFO_DISPATCH if self.fifo_dispatch else 0) | (HOST_SLAB if sc.get("_slab") else 0) | (SAMPLED_TRAJ if sampled_traj else 0) | (QP_EXACT if exact else 0)), "wbc_cycle")
         return out
 
-    def cycle_device(self, dev_in, dev_out, n, ld, stream=None, sync=True, out_ld=None):
+    def cycle_device(self, dev_in, dev_out, n, ld, stream=None, sync=True, out_ld=None, exact=False):
         """One control cycle on DEVICE-resident SoA buffers (dicts of torch CUDA tensors or raw pointers).
         `ld` is the leading dimension of the input arrays, `out_ld` that of the output arrays (default: the outputs' own
-        second dimension when they are tensors, else `ld`)."""
+        second dimension when they are tensors, else `ld`).  exact: as in cycle()."""
         if out_ld is None:
             t = dev_out.get("tau")
             out_ld = int(t.stride(0)) if hasattr(t, "stride") and t.dim() == 2 else ld
@@ -351,7 +354,7 @@ class WbcBatch:
         for k in ("tau", "w", "x", "qp_obj", "status", "qp_info", "qp_flops", "w3"):
             setattr(o, k, _ptr(dev_out.get(k)))
         o.ld = out_ld
-        flags = DEVICE_PTRS | (0 if sync else NO_SYNC) | (FIFO_DISPATCH if self.fifo_dispatch else 0)
+        flags = DEVICE_PTRS | (0 if sync else NO_SYNC) | (FIFO_DISPATCH if self.fifo_dispatch else 0) | (QP_EXACT if exact else 0)
         _check(self.lib.wbc_cycle(self.h, n, C.byref(ins), C.byref(o), stream, flags), "wbc_cycle")
 
     def qp_records(self, n):
@@ -376,8 +379,9 @@ class WbcBatch:
         _check(self.lib.wbc_debug_update(self.h, n, C.byref(ins), C.byref(d), HOST_PTRS), "wbc_debug_update")
         return out
 
-    def qp_solve(self, Q, c, L, neq):
-        """n dense QPs, instance-major numpy arrays Q [n,30,30], c [n,30], L [n,nrows,31] (the OPT operator)."""
+    def qp_solve(self, Q, c, L, neq, exact=False):
+        """n dense QPs, instance-major numpy arrays Q [n,30,30], c [n,30], L [n,nrows,31] (the OPT operator).  exact=True: the
+        exact-mode solver (WBC_QP_EXACT); info then holds its counters (include/wbc_b200.h)."""
         Q = np.ascontiguousarray(Q, dtype=np.float64)
         c = np.ascontiguousarray(c, dtype=np.float64)
         L = np.ascontiguousarray(L, dtype=np.float64)
@@ -387,7 +391,7 @@ class WbcBatch:
         info = np.zeros((n, 8), dtype=np.int32)
         flops = np.zeros(n)
         _check(self.lib.wbc_qp_solve(self.h, n, Q.ctypes.data, c.ctypes.data, L.ctypes.data, nrows, int(neq), x.ctypes.data,
-                                     status.ctypes.data, info.ctypes.data, flops.ctypes.data, None, HOST_PTRS), "wbc_qp_solve")
+                                     status.ctypes.data, info.ctypes.data, flops.ctypes.data, None, HOST_PTRS | (QP_EXACT if exact else 0)), "wbc_qp_solve")
         return x, status, info, flops
 
     def plant_step(self, base_pos, base_vel, push, foot_force=None, x=None, n=None, ld=None, stream=None, sync=True):
@@ -436,10 +440,11 @@ class WbcBatch:
         return int(self.lib.wbc_last_launches(self.h))
 
     def solver_shape(self):
-        """(resident solver CTAs per SM, shared-memory bytes per CTA, grid of the last cycle) of the persistent solver kernel."""
+        """(resident solver CTAs per SM, shared-memory bytes per CTA, grid of the last cycle) of the persistent solver kernel the
+        last cycle ran; its name is left in last_solver_kernel."""
         a, b, g, st = C.c_int(0), C.c_int(0), C.c_int(0), C.c_int(0)
         _check(self.lib.wbc_solver_shape(self.h, C.byref(a), C.byref(b), C.byref(g), C.byref(st)), "wbc_solver_shape")
-        self.last_solver_kernel = "wbc_solve_staged_kernel" if st.value else "wbc_solve_kernel"
+        self.last_solver_kernel = SOLVER_KERNELS[st.value]
         return a.value, b.value, g.value
 
     def stage_profile(self):
@@ -465,12 +470,14 @@ class OPT:
     raises WbcError instead).
     """
 
-    def __init__(self, control_variables=30, stance_constraint=86, swing_constraint=82, batch=None):
+    def __init__(self, control_variables=30, stance_constraint=86, swing_constraint=82, batch=None, exact=False):
+        """exact=True: solve to the exact optimum (WBC_QP_EXACT) instead of DENSE-AUL at the reference's settings."""
         if control_variables != 30 or stance_constraint != 86 or swing_constraint != 82:
             raise WbcError("OPT is specialised to the controller's shapes OPT(30, 86, 82) (main.cpp:266)")
         self._own = batch is None
         self._b = batch or WbcBatch(1)
         self._Q = self._c = self._Ls = self._Lw = None
+        self.exact = bool(exact)
 
     def setQ(self, Q_):
         self._Q = np.array(Q_, dtype=np.float64).reshape(1, 30, 30)
@@ -487,7 +494,7 @@ class OPT:
     def _solve(self, L, neq):
         if self._Q is None or self._c is None or L is None:
             raise WbcError("OPT: setQ, setc and setL_* must be called before opt_*")
-        x, status, _, _ = self._b.qp_solve(self._Q, self._c, L, neq)
+        x, status, _, _ = self._b.qp_solve(self._Q, self._c, L, neq, exact=self.exact)
         if status[0] != 0:
             raise WbcError("OPT: QP solver failed with status %d" % status[0])
         return x[0]

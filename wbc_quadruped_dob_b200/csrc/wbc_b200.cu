@@ -6,6 +6,8 @@
 //                      registers each), persistent warps pulling instances from an atomic queue (iteration counts vary
 //                      4..50 Cholesky per solve): assemble (Q,c,L) from the record, DENSE-AUL/QQP solve with the
 //                      hot state in shared memory (qp_warp.cuh), torque map.
+//   wbc_solve_exact_kernel  (WBC_QP_EXACT) in place of wbc_solve_kernel: the same warp-per-instance persistent shape around the
+//                      Goldfarb-Idnani dual active-set solver of qp_dual.cuh (the exact optimum of each QP).
 // There is no CPU fallback anywhere in this file.
 #include <cuda_runtime.h>
 #include <stdio.h>
@@ -17,6 +19,7 @@
 
 #include "../../include/wbc_b200.h"
 #include "qp_warp.cuh"
+#include "qp_dual.cuh"
 #include "wbc_assemble.cuh"
 #include "wbc_front.cuh"
 #include "wbc_front_leg.cuh"
@@ -321,6 +324,155 @@ __global__ void __launch_bounds__(SOLVE_T) wbc_solve_kernel(Params P, int n, con
         unsigned long long* p = xl.prof + (long)blockIdx.x * 12;
         p[0] = pr_busy; p[1] = pr_jobs; p[2] = pr_t0; p[3] = pr_first; p[4] = pr_last; p[5] = now; p[6] = pr_longest; p[7] = express ? 1 : 0; p[8] = smid;
         p[9] = 0; p[10] = 0; p[11] = 0;
+    }
+}
+
+// ---- exact QP mode (WBC_QP_EXACT): the Goldfarb-Idnani dual active-set solver of qp_dual.cuh, one warp per solve.
+// Its shared block is 17.2 KB (R, the factor / product scratch and a few vectors) and J lives in registers; the constraint matrix
+// stays in the warp's global scratch.  Residency: with the 1 KB the SM reserves per CTA, shared memory admits 12 CTAs per SM
+// (13 x 18.6 KB > 228 KB), and __launch_bounds__(32, 12) lets the compiler use all 168 registers that 12 CTAs leave per thread
+// (ptxas: 165, no spills).  Fewer warps with more registers lost: -DWBC_EXACT_MIN_CTAS=8 (no spills then either) measured 0.93x at
+// 65 536 and 0.73x at 4 096 instances (profiles/r03_exact_ctas_ab.txt).
+constexpr int EXACT_T = 32;
+#ifndef WBC_EXACT_MIN_CTAS
+#define WBC_EXACT_MIN_CTAS 12
+#endif
+constexpr int EXACT_MIN_CTAS = WBC_EXACT_MIN_CTAS;
+static_assert(wbc::QR_MODE + 1 <= wbcdual::N * wbcdual::LD, "the QP record is staged in R's place");
+
+__device__ __forceinline__ void write_info_exact(const wbcdual::DualStats& st, long i, long ld, int* status, int* info, double* flops)
+{
+    if (status) status[i] = st.status;
+    if (info) {
+        info[0 * ld + i] = st.nfact; info[1 * ld + i] = st.adds; info[2 * ld + i] = st.drops; info[3 * ld + i] = st.nact_ineq;
+        info[4 * ld + i] = st.nact; info[5 * ld + i] = st.flags; info[6 * ld + i] = 0; info[7 * ld + i] = 0;
+    }
+    if (flops) flops[i] = st.flops;
+}
+
+// PROF = true (a ctx created with WBC_STAGE_PROF=1): per-warp cycle counters by phase, rows of 12 in `prof` (wbc_stage_profile):
+// [0..8] the wbcdual::PH_* phases summed over the warp's solves, [9] solves, [10] rows added + dropped, [11] cycles in the kernel.
+template <bool PROF>
+__global__ void __launch_bounds__(EXACT_T, EXACT_MIN_CTAS) wbc_solve_exact_kernel(Params P, int n, const double* __restrict__ recs, SolveOut out,
+                                                                                 double* __restrict__ scratch_base, int* __restrict__ queue,
+                                                                                 const int* __restrict__ order, unsigned* __restrict__ cost,
+                                                                                 int* __restrict__ hist_next, unsigned long long* __restrict__ prof,
+                                                                                 int prof_rows)
+{
+    const WarpEx ex;
+    unsigned long long pc[12];
+#pragma unroll
+    for (int k = 0; k < 12; k++) pc[k] = 0ull;
+    const long long k0 = PROF ? clock64() : 0;
+    double* sm = wbc_smem;
+    double* C = scratch_base + (long)blockIdx.x * wbcdual::SCRATCH_DOUBLES;
+    for (int k = ex.lane(); k < wbcdual::ds::TOTAL; k += EXACT_T) sm[k] = 0.0;
+    ex.sync();
+    for (;;) {
+        const int ticket = next_instance(queue);
+        if (ticket >= n) break;
+        const int i = order ? order[ticket] : ticket;
+        const long long t0 = clock64();
+        double* rec = sm + wbcdual::ds::OFF_R;
+        ex.copy_in(rec, recs + (long)i * QPREC_DOUBLES, QR_MODE + 1);
+        wbcdual::DualStats st;
+        {
+            // the record validation of wbc_solve_kernel
+            double chk = 0.0;
+#pragma unroll 1
+            for (int k = ex.lane(); k <= QR_MODE; k += EXACT_T) chk += rec[k] * 0.0;
+            const bool nonfinite = __any_sync(0xffffffffu, chk != 0.0);
+            const double md = rec[QR_MODE];
+            if (nonfinite || !(md == 0.0 || md == 1.0 || md == 2.0)) {
+                for (int k = ex.lane(); k < 12; k += EXACT_T)
+                    out.tau[(long)k * out.ld + i] = P.hold_tau_on_failure ? out.tau_prev[(long)k * out.ld_prev + i] : 0.0;
+                if (out.x)
+                    for (int k = ex.lane(); k < 30; k += EXACT_T) out.x[(long)k * out.ld + i] = 0.0;
+                if (ex.lane() == 0) {
+                    st.status = nonfinite ? WBC_ST_NONFINITE : WBC_ST_BAD_MODE;
+                    st.nfact = 0; st.adds = 0; st.drops = 0; st.nact_ineq = 0; st.nact = 0; st.flags = wbcdual::FL_EXACT; st.flops = 0.0;
+                    write_info_exact(st, i, out.ld, out.status, out.qp_info, out.qp_flops);
+                    if (out.qp_obj) out.qp_obj[i] = 0.0;
+                    cost[i] = 0u;
+                    atomicAdd(hist_next, 1);
+                }
+                ex.sync();
+                continue;
+            }
+        }
+        const QpShape sh = qp_shape((int)rec[QR_MODE]);
+        assemble_qp<wbcdual::LD>(ex, P, rec, sh, sm + wbcdual::ds::OFF_H, sm + wbcdual::ds::OFF_CV, C);
+        if (PROF) pc[wbcdual::PH_ASSEMBLE] += (unsigned long long)(clock64() - t0);
+        wbcdual::solve_dual<WarpEx, PROF>(ex, sm, C, sh.nrows, sh.neq, st, pc);
+        const long long t1 = PROF ? clock64() : 0;
+        const double* xs = sm + wbcdual::ds::OFF_Y;          // x, or 0 when the solve failed
+        ex.copy_in(rec, recs + (long)i * QPREC_DOUBLES, QR_MODE + 1);     // R's place was the solver's; stage again
+        torque_and_objective(ex, P, rec, sh, xs, out.tau + i, out.ld, out.qp_obj ? out.qp_obj + i : nullptr);
+        if (st.status == 0) {
+            for (int k = ex.lane(); k < 12; k += EXACT_T) out.tau_prev[(long)k * out.ld_prev + i] = out.tau[(long)k * out.ld + i];
+        } else if (P.hold_tau_on_failure) {
+            for (int k = ex.lane(); k < 12; k += EXACT_T) out.tau[(long)k * out.ld + i] = out.tau_prev[(long)k * out.ld_prev + i];
+        }
+        if (out.x)
+            for (int k = ex.lane(); k < 30; k += EXACT_T) out.x[(long)k * out.ld + i] = xs[k];
+        if (ex.lane() == 0) {
+            write_info_exact(st, i, out.ld, out.status, out.qp_info, out.qp_flops);
+            // the duration orders the next cycle's dispatch (longest first), as in wbc_solve_kernel: one bucket entry per instance
+            const unsigned long long dt = (unsigned long long)(clock64() - t0) >> 10;
+            const unsigned cu = dt > 0xffffffffull ? 0xffffffffu : (unsigned)dt;
+            cost[i] = cu;
+            atomicAdd(hist_next + cost_bucket(cu), 1);
+        }
+        ex.sync();
+        if (PROF) {
+            pc[wbcdual::PH_OUTPUT] += (unsigned long long)(clock64() - t1);
+            pc[9]++;
+            pc[10] += (unsigned long long)(st.adds + st.drops);
+        }
+    }
+    if (PROF && ex.lane() == 0 && (int)blockIdx.x < prof_rows) {
+        pc[11] = (unsigned long long)(clock64() - k0);
+        for (int k = 0; k < 12; k++) prof[(long)blockIdx.x * 12 + k] = pc[k];
+    }
+}
+
+// Dense-input form of the exact solver (wbc_qp_solve with WBC_QP_EXACT): Q [n][900], c [n][30], L [n][nrows*31], x [n][30].
+__global__ void __launch_bounds__(EXACT_T, EXACT_MIN_CTAS) wbc_dense_qp_exact_kernel(int n, const double* __restrict__ Q, const double* __restrict__ c,
+                                                                                    const double* __restrict__ L, int nrows, int neq, double* __restrict__ x,
+                                                                                    int* status, int* info, double* flops, double* __restrict__ scratch_base,
+                                                                                    int* __restrict__ queue)
+{
+    const WarpEx ex;
+    double* sm = wbc_smem;
+    double* C = scratch_base + (long)blockIdx.x * wbcdual::SCRATCH_DOUBLES;
+    for (int k = ex.lane(); k < wbcdual::ds::TOTAL; k += EXACT_T) sm[k] = 0.0;
+    ex.sync();
+    for (;;) {
+        const int i = next_instance(queue);
+        if (i >= n) break;
+        double* H = sm + wbcdual::ds::OFF_H;
+        double chk = 0.0;                      // x * 0 is NaN exactly for NaN and the infinities
+        for (int k = ex.lane(); k < 900; k += EXACT_T) { const double v = Q[(long)i * 900 + k]; H[(k / 30) * wbcdual::LD + (k % 30)] = v; chk += v * 0.0; }
+        for (int k = ex.lane(); k < 30; k += EXACT_T) { const double v = c[(long)i * 30 + k]; sm[wbcdual::ds::OFF_CV + k] = v; chk += v * 0.0; }
+        for (int k = ex.lane(); k < nrows * 31; k += EXACT_T) { const double v = L[(long)i * nrows * 31 + k]; C[k] = v; chk += v * 0.0; }
+        ex.sync();
+        wbcdual::DualStats st;
+        if (__any_sync(0xffffffffu, chk != 0.0)) {
+            st.status = WBC_ST_NONFINITE; st.nfact = 0; st.adds = 0; st.drops = 0; st.nact_ineq = 0; st.nact = 0; st.flags = wbcdual::FL_EXACT; st.flops = 0.0;
+            for (int k = ex.lane(); k < 30; k += EXACT_T) sm[wbcdual::ds::OFF_Y + k] = 0.0;
+            ex.sync();
+        } else
+            wbcdual::solve_dual(ex, sm, C, nrows, neq, st);
+        for (int k = ex.lane(); k < 30; k += EXACT_T) x[(long)i * 30 + k] = sm[wbcdual::ds::OFF_Y + k];
+        if (ex.lane() == 0) {   // instance-major info [n][8] on this path
+            if (status) status[i] = st.status;
+            if (flops) flops[i] = st.flops;
+            if (info) {
+                int* q = info + (long)i * 8;
+                q[0] = st.nfact; q[1] = st.adds; q[2] = st.drops; q[3] = st.nact_ineq; q[4] = st.nact; q[5] = st.flags; q[6] = 0; q[7] = 0;
+            }
+        }
+        ex.sync();
     }
 }
 
@@ -751,7 +903,8 @@ struct wbc_ctx {
     int front_leg;       // 1 (default): wbc_front_leg_kernel, four lanes per instance; 0: wbc_front_kernel, a thread per instance (WBC_FRONT=thread)
     int last_staged;     // which kernel the last wbc_cycle launched
     int m_period, m_group;   // SM roles of the staged solver
-    unsigned long long* prof;   // [nblocks][12] per-warp profile of the last staged launch (WBC_STAGE_PROF=1)
+    unsigned long long* prof;   // [prof_rows][12] per-warp profile of the last staged or exact-mode launch (WBC_STAGE_PROF=1)
+    int prof_rows;
     int* queue;          // [cost histogram A | work-queue counter | dispatch cursors | cost histogram B]: counter and cursors sit between
                          // the two histograms so that "counter + cursors + the histogram being filled" is one contiguous memset either way
     unsigned* cost;      // [max_batch] duration of each instance's last solve (1024-cycle units)
@@ -763,6 +916,8 @@ struct wbc_ctx {
     int occ_forced;         // WBC_SOLVE_CTAS_PER_SM was given: no per-launch adaptation
     int last_grid;          // solver grid of the last wbc_cycle
     int solve_smem;         // dynamic shared memory per solver CTA (sl::BYTES, or padded by WBC_SOLVE_CTAS_PER_SM)
+    int exact_per_sm;       // exact-mode kernel (WBC_QP_EXACT): resident CTAs per SM (occupancy calculator) ...
+    int exact_blocks;       // ... its persistent grid: every resident CTA that has a scratch block (wbcdual::SCRATCH_DOUBLES each)
     // staging for WBC_HOST_PTRS
     double* d_in;        // [93+40][max_batch]
     double* d_out;       // [62][max_batch]
@@ -912,7 +1067,7 @@ int wbc_create(wbc_ctx** out, int device, int max_batch, const wbc_params* param
     TRY(cudaMalloc(&c->kkt, (size_t)nteams * gl::KKT_DOUBLES * sizeof(double)));
     TRY(cudaMalloc(&c->sq_ctl, sizeof(StageCtl)));
     TRY(cudaMalloc(&c->sq_ring, (size_t)3 * c->sq_rsize * sizeof(int)));
-    if (getenv("WBC_STAGE_PROF")) { TRY(cudaMalloc(&c->prof, (size_t)nteams * 12 * sizeof(unsigned long long))); TRY(cudaMemset(c->prof, 0, (size_t)nteams * 12 * sizeof(unsigned long long))); }
+    if (getenv("WBC_STAGE_PROF")) { TRY(cudaMalloc(&c->prof, (size_t)nteams * 12 * sizeof(unsigned long long))); TRY(cudaMemset(c->prof, 0, (size_t)nteams * 12 * sizeof(unsigned long long))); c->prof_rows = (int)nteams; }
     TRY(cudaMalloc(&c->queue, (1 + 3 * ORD_NB) * sizeof(int)));
     TRY(cudaMalloc(&c->lanes, LANES_INTS * sizeof(int)));
     TRY(cudaMemset(c->lanes, 0, LANES_INTS * sizeof(int)));
@@ -937,6 +1092,9 @@ int wbc_create(wbc_ctx** out, int device, int max_batch, const wbc_params* param
     TRY(cudaFuncSetAttribute(wbc_dense_qp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, c->solve_smem));
     TRY(cudaFuncSetAttribute(wbc_solve_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     TRY(cudaFuncSetAttribute(wbc_dense_qp_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    TRY(cudaFuncSetAttribute(wbc_solve_exact_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    TRY(cudaFuncSetAttribute(wbc_solve_exact_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    TRY(cudaFuncSetAttribute(wbc_dense_qp_exact_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     if (l1_ctas > 0) {
         const int pct = (int)((100L * l1_ctas * (sl::BYTES + 1024) + 228 * 1024 - 1) / (228 * 1024));
         TRY(cudaFuncSetAttribute(wbc_solve_staged_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct > 100 ? 100 : pct));
@@ -954,6 +1112,15 @@ int wbc_create(wbc_ctx** out, int device, int max_batch, const wbc_params* param
             if (c->nblocks > c->sm_count * occ) c->nblocks = c->sm_count * occ;
             if (l1_ctas > 0 && l1_ctas < occ) c->occ_per_sm = l1_ctas;
         }
+    }
+    if (e == cudaSuccess) {
+        // exact mode: the scratch blocks of the DENSE-AUL kernels, carved into the exact solver's smaller ones
+        int occ = 0;
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, wbc_solve_exact_kernel<false>, EXACT_T, (size_t)wbcdual::ds::BYTES);
+        const long cap = (long)c->nslots * gl::TOTAL / wbcdual::SCRATCH_DOUBLES;
+        c->exact_per_sm = occ > 0 ? occ : 1;
+        const long want = (long)c->sm_count * c->exact_per_sm;
+        c->exact_blocks = (int)(want < cap ? want : cap);
     }
 #undef TRY
     if (e != cudaSuccess) {
@@ -1112,6 +1279,7 @@ int wbc_cycle(wbc_ctx* c, int n, const wbc_inputs* in, const wbc_outputs* out, v
     if (rc) return rc;
     if (!out->tau || out->ld < n) return fail(WBC_EINVAL, "wbc_cycle: outputs.tau is required and outputs.ld >= n");
     const bool dev_ptrs = (flags & WBC_DEVICE_PTRS) != 0;
+    const bool exact = (flags & WBC_QP_EXACT) != 0;
     if (sampled && c->traj_sampled_n < n) return fail(WBC_EINVAL, "wbc_cycle: WBC_SAMPLED_TRAJ without a wbc_sample_trajectory(out = NULL) covering n instances");
     if (sampled && dev_ptrs && in->ld != c->max_batch)
         return fail(WBC_EINVAL, "wbc_cycle: WBC_SAMPLED_TRAJ with device pointers needs inputs.ld == max_batch (or sample into your own arrays)");
@@ -1161,8 +1329,8 @@ int wbc_cycle(wbc_ctx* c, int n, const wbc_inputs* in, const wbc_outputs* out, v
     DispatchOrder ord;
     ord.cost = ordered ? c->cost : nullptr; ord.hist = hist_prev; ord.cursor = counter + 1; ord.order = c->order;
     // express lanes for the one-warp-per-solve kernel on a batch of a few solves per warp (see ExpressLanes)
-    const bool staged_sel = c->staged == 1 || (c->staged == 2 && n >= c->staged_min_n);
-    const bool express = !staged_sel && c->xl_period > 0 && !c->occ_forced && c->occ_per_sm >= 12 && n >= c->xl_min_n;
+    const bool staged_sel = !exact && (c->staged == 1 || (c->staged == 2 && n >= c->staged_min_n));
+    const bool express = !exact && !staged_sel && c->xl_period > 0 && !c->occ_forced && c->occ_per_sm >= 12 && n >= c->xl_min_n;
     ord.lanes = express ? c->lanes : nullptr;
     // one memset: counter, cursors and the histogram this cycle fills (A lies just before the counter, B just after the cursors)
     CU(cudaMemsetAsync((c->hist_sel ^ 1) == 0 ? c->queue : counter, 0, (1 + 2 * ORD_NB) * sizeof(int), s));
@@ -1170,7 +1338,7 @@ int wbc_cycle(wbc_ctx* c, int n, const wbc_inputs* in, const wbc_outputs* out, v
     const int fthreads = front_threads(c, n);
     StageReset sr;
     memset(&sr, 0, sizeof(sr));
-    const bool staged_next = c->staged == 1 || (c->staged == 2 && n >= c->staged_min_n);
+    const bool staged_next = !exact && (c->staged == 1 || (c->staged == 2 && n >= c->staged_min_n));
     if (staged_next) {
         sr.ctl = reinterpret_cast<int*>(c->sq_ctl); sr.nctl = (int)(sizeof(StageCtl) / sizeof(int));
         sr.free_tail_index = (int)(offsetof(StageCtl, tail) / sizeof(int)) + SQ_FREE * 32;
@@ -1192,8 +1360,8 @@ int wbc_cycle(wbc_ctx* c, int n, const wbc_inputs* in, const wbc_outputs* out, v
     // beat a plain 12 by 3 % at 4 096 instances (profiles/README.md).
     int nblocks = c->nblocks;
     int smem = c->solve_smem;
-    const bool staged = c->staged == 1 || (c->staged == 2 && n >= c->staged_min_n);
-    c->last_staged = staged ? 1 : 0;
+    const bool staged = !exact && (c->staged == 1 || (c->staged == 2 && n >= c->staged_min_n));
+    c->last_staged = exact ? 2 : (staged ? 1 : 0);
     ExpressLanes xl;
     xl.lanes = c->lanes; xl.head = 0; xl.period = 0; xl.keep = c->xl_keep; xl.cycles = c->cycles; xl.prof = c->prof; xl.time_scale = c->xl_time_scale;
     c->cycles_valid = 0;
@@ -1209,6 +1377,10 @@ int wbc_cycle(wbc_ctx* c, int n, const wbc_inputs* in, const wbc_outputs* out, v
             nblocks = c->xl_warps * c->sm_count;
             smem = (((228 * 1024) / c->xl_warps - 1024) / 16) * 16;
         }
+    } else if (exact) {
+        // the exact solver's own launch shape: every resident CTA, whatever the batch size
+        nblocks = c->exact_blocks;
+        smem = wbcdual::ds::BYTES;
     } else if (!staged && c->occ_per_sm > 8 && !c->occ_forced) {
         int per_sm = (int)((double)n / (3.4 * c->sm_count));
         per_sm = per_sm < 8 ? 8 : (per_sm > c->occ_per_sm ? c->occ_per_sm : per_sm);
@@ -1221,7 +1393,14 @@ int wbc_cycle(wbc_ctx* c, int n, const wbc_inputs* in, const wbc_outputs* out, v
     }
     if (n < nblocks) nblocks = n;
     c->last_grid = nblocks;
-    if (staged) {
+    if (exact) {
+        if (c->prof)
+            wbc_solve_exact_kernel<true><<<nblocks, EXACT_T, smem, s>>>(c->params, n, c->recs, so, c->scratch, counter, ordered ? c->order : nullptr,
+                                                                        c->cost, hist_next, c->prof, c->prof_rows);
+        else
+            wbc_solve_exact_kernel<false><<<nblocks, EXACT_T, smem, s>>>(c->params, n, c->recs, so, c->scratch, counter, ordered ? c->order : nullptr,
+                                                                         c->cost, hist_next, nullptr, 0);
+    } else if (staged) {
         StageQueues sq;
         sq.ctl = c->sq_ctl; sq.ring = c->sq_ring; sq.rmask = c->sq_rsize - 1; sq.nslots = c->nslots;
         wbc_solve_staged_kernel<<<nblocks, c->threads, c->solve_smem, s>>>(c->params, n, c->recs, so, c->scratch, c->kkt, sq, ordered ? c->order : nullptr,
@@ -1472,8 +1651,8 @@ int wbc_stage_profile(wbc_ctx* c, unsigned long long* out, int max_rows)
 int wbc_solver_shape(wbc_ctx* c, int* ctas_per_sm, int* smem_bytes, int* grid, int* stage_tasks)
 {
     if (!c) return fail(WBC_EINVAL, "null ctx");
-    if (ctas_per_sm) *ctas_per_sm = c->occ_per_sm;
-    if (smem_bytes) *smem_bytes = c->solve_smem;
+    if (ctas_per_sm) *ctas_per_sm = c->last_staged == 2 ? c->exact_per_sm : c->occ_per_sm;
+    if (smem_bytes) *smem_bytes = c->last_staged == 2 ? wbcdual::ds::BYTES : c->solve_smem;
     if (grid) *grid = c->last_grid > 0 ? c->last_grid : c->nblocks;
     if (stage_tasks) *stage_tasks = c->last_staged;
     return WBC_OK;
@@ -1601,10 +1780,15 @@ int wbc_qp_solve(wbc_ctx* c, int n, const double* Q, const double* cvec, const d
         dinfo = info ? ip + n : nullptr;
     }
     CU(cudaMemsetAsync(c->queue + ORD_NB, 0, sizeof(int), s));
-    const int nblocks = n < c->nblocks ? n : c->nblocks;
+    const bool exact = (flags & WBC_QP_EXACT) != 0;
+    const int nblocks = exact ? (n < c->exact_blocks ? n : c->exact_blocks) : (n < c->nblocks ? n : c->nblocks);
     CU(cudaEventRecord(c->ev0, s));
     CU(cudaEventRecord(c->ev1, s));
-    wbc_dense_qp_kernel<<<nblocks, c->threads, c->solve_smem, s>>>(c->params, n, dQ, dc, dL, nrows, neq, dx, dstatus, dinfo, dflops, c->scratch, c->kkt, c->queue + ORD_NB);
+    if (exact)
+        wbc_dense_qp_exact_kernel<<<nblocks, EXACT_T, wbcdual::ds::BYTES, s>>>(n, dQ, dc, dL, nrows, neq, dx, dstatus, dinfo, dflops, c->scratch,
+                                                                                c->queue + ORD_NB);
+    else
+        wbc_dense_qp_kernel<<<nblocks, c->threads, c->solve_smem, s>>>(c->params, n, dQ, dc, dL, nrows, neq, dx, dstatus, dinfo, dflops, c->scratch, c->kkt, c->queue + ORD_NB);
     CU(cudaEventRecord(c->ev2, s));
     CU(cudaGetLastError());
     c->launches = 1;
