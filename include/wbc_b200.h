@@ -69,6 +69,14 @@ extern "C" {
                                   * included), [2] rows dropped, [3] active inequality rows, [4] active-set size, [5] flags: 256 always
                                   * (exact mode), | 512 a dependent consistent equality was skipped, | 1024 a violated row depended on
                                   * the active set and dual steps were taken; [6], [7] 0.  qp_flops: the exact solver's own count. */
+#define WBC_QP_WARM 64u          /* wbc_cycle, only together with WBC_QP_EXACT (else WBC_EINVAL, nothing done): warm-start each instance
+                                  * from the active set the ctx stored for its index (wbc_get_active_set) when that set was solved in
+                                  * the instance's current contact mode; any other instance starts cold.  Every exact-mode cycle, warm
+                                  * or cold, stores each instance's final active inequality rows (none when it failed or was refused).
+                                  * x is the same unique optimum as in cold exact mode, to the solver's precision but not bit for bit:
+                                  * it depends on the ctx's history.  qp_info in this mode: [1], [2] include the warm-start phase's
+                                  * additions and drops, [6] warm rows added before the GI loop, [7] warm rows dropped before it (a
+                                  * negative multiplier), [5] | 2048 when the instance was warm-started. */
 #define WBC_HOST_SLAB 8u         /* (host pointers) the input arrays are carved, in wbc_inputs field order, from ONE page-locked
                                   * allocation with ld == n: adjacent fields are moved with a single copy */
 
@@ -204,6 +212,18 @@ int wbc_debug_qp_records(wbc_ctx* ctx, int n, double* recs, int* doubles_per_rec
  *   and flops [n] may be NULL.  A failed instance (status < 0) returns x = 0. */
 int wbc_qp_solve(wbc_ctx* ctx, int n, const double* Q, const double* c, const double* L, int nrows, int neq, double* x,
                  int* status, int* info, double* flops, void* cuda_stream, unsigned flags);
+/* wbc_qp_solve with the exact solver (WBC_QP_EXACT implied), warm-started: active [n][3] (host or device per flags, like x) is read
+ * as each instance's warm set -- bit r of word r / 32 is inequality row r; bits at equality rows or beyond nrows are ignored, an
+ * all-zero set is a cold start -- and overwritten with the instance's final active inequality rows (all zero when it failed).
+ * Feeding the output back on the next call warm-starts a QP that changes little from call to call.  info[6], info[7] as for
+ * WBC_QP_WARM. */
+int wbc_qp_solve_warm(wbc_ctx* ctx, int n, const double* Q, const double* c, const double* L, int nrows, int neq, double* x,
+                      int* status, int* info, double* flops, unsigned* active, void* cuda_stream, unsigned flags);
+/* The exact-mode active sets the ctx stores per instance index (see WBC_QP_WARM): sets [4][ld], host pointer; rows 0..2 the active
+ * inequality rows as bit masks, row 3 the contact mode they were solved in + 1 (0: no set).  The ctx zero-initialises them.
+ * Restore them with the observer state after a checkpoint, or after moving instances to other indices or ctxs (re-sharding). */
+int wbc_set_active_set(wbc_ctx* ctx, int n, const unsigned* sets, long ld);
+int wbc_get_active_set(wbc_ctx* ctx, int n, unsigned* sets, long ld);
 
 /* Synthetic plant of BASELINE config 5 (disturbance-rejection sweep).  Stands in for Gazebo + the ModelPush plugin
  * (force_plugin/src/force_plugin.cpp:124-491), which cannot run here: a CoM momentum integrator with locked joints,

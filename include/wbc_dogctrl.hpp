@@ -93,24 +93,32 @@ public:
             for (int j = 0; j < 31; j++) Lw_[i * 31 + j] = L(i, j);
     }
     // first 18 rows "=" (lopt.cpp:40-47); x_ must hold 30 entries (main.cpp:1122-1123)
-    template <class Vec> void opt_stance(Vec& x_) { solve(Ls_.data(), 86, 18, x_); }
+    template <class Vec> void opt_stance(Vec& x_) { solve(Ls_.data(), 86, 18, x_, active_stance_); }
     // first 12 rows "=" (lopt.cpp:57-64)
-    template <class Vec> void opt_swing(Vec& x_) { solve(Lw_.data(), 82, 12, x_); }
+    template <class Vec> void opt_swing(Vec& x_) { solve(Lw_.data(), 82, 12, x_, active_swing_); }
 
     bool swallow_failures;   // true: behave like lopt.cpp:114-116 (x_ untouched, nothing reported)
     bool exact_qp = false;   // true: solve to the exact optimum (WBC_QP_EXACT, dual active-set) instead of DENSE-AUL at the
                              // reference's settings; last_info then holds the exact-mode counters (wbc_b200.h)
+    bool warm_start = false; // with exact_qp: opt_stance and opt_swing each start from the active set of their own previous solve
+                             // (wbc_qp_solve_warm) -- for a control loop that solves almost the same QP every cycle
     int last_status;         // 0 ok, <0 solver failure of the last opt_* call
     int last_info[8];        // ncholesky, outer its, QQP calls, working set, max KKT dim, flags, 0, 0
 
 private:
-    template <class Vec> void solve(const double* L, int nrows, int neq, Vec& x_)
+    template <class Vec> void solve(const double* L, int nrows, int neq, Vec& x_, unsigned* active)
     {
         double x[30];
         for (int i = 0; i < 30; i++) x[i] = x_(i);
-        check(wbc_qp_solve(ctx_.get(), 1, Q_.data(), c_.data(), L, nrows, neq, x, &last_status, last_info, nullptr, nullptr,
-                           WBC_HOST_PTRS | (exact_qp ? WBC_QP_EXACT : 0u)),
-              "wbc_qp_solve");
+        if (warm_start && !exact_qp) throw Error(WBC_EINVAL, "OPT: warm_start needs exact_qp");
+        if (warm_start)
+            check(wbc_qp_solve_warm(ctx_.get(), 1, Q_.data(), c_.data(), L, nrows, neq, x, &last_status, last_info, nullptr, active, nullptr,
+                                    WBC_HOST_PTRS),
+                  "wbc_qp_solve_warm");
+        else
+            check(wbc_qp_solve(ctx_.get(), 1, Q_.data(), c_.data(), L, nrows, neq, x, &last_status, last_info, nullptr, nullptr,
+                               WBC_HOST_PTRS | (exact_qp ? WBC_QP_EXACT : 0u)),
+                  "wbc_qp_solve");
         if (last_status != 0) {
             if (swallow_failures) return;
             throw Error(last_status, exact_qp ? "OPT: the exact QP solver reported failure" : "OPT: the DENSE-AUL solver reported failure");
@@ -119,6 +127,7 @@ private:
     }
     Context ctx_;
     std::vector<double> Q_, c_, Ls_, Lw_;
+    unsigned active_stance_[3] = {0u, 0u, 0u}, active_swing_[3] = {0u, 0u, 0u};   // warm_start: the last final active sets
 };
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -143,6 +152,7 @@ public:
     void get_observer_state2(double* yg) { check(wbc_get_observer_state2(ctx_.get(), n_, yg, n_), "wbc_get_observer_state2"); }
     bool want_w3 = false;   // also compute ESTIMATOR_SEM::getw3 (estimator_sem.cpp:64-70) into w3
     bool exact_qp = false;  // solve each QP to its exact optimum (WBC_QP_EXACT) instead of DENSE-AUL at the reference's settings
+    bool warm_qp = false;   // with exact_qp: start each instance from its previous exact-mode active set (WBC_QP_WARM)
     // Planner hand-over (once per plan): the node tables of the four towr splines of every instance, see wbc_trajectory.
     // durations [4*nseg][n], nodes [4*(nseg+1)*6][n].  Replaces keeping `SplineHolder solution` on the host (main.cpp:900-960).
     void set_trajectory(int nseg, const double* durations, const double* nodes)
@@ -167,7 +177,8 @@ public:
         wbc_outputs out;
         out.tau = tau.data(); out.w = w.data(); out.x = x.data(); out.qp_obj = qp_obj.data(); out.status = status.data();
         out.qp_info = nullptr; out.qp_flops = nullptr; out.ld = n_; out.w3 = want_w3 ? w3.data() : nullptr;
-        check(wbc_cycle(ctx_.get(), n_, &in, &out, nullptr, WBC_HOST_PTRS | (sampled_trajectory ? WBC_SAMPLED_TRAJ : 0u) | (exact_qp ? WBC_QP_EXACT : 0u)),
+        check(wbc_cycle(ctx_.get(), n_, &in, &out, nullptr, WBC_HOST_PTRS | (sampled_trajectory ? WBC_SAMPLED_TRAJ : 0u) | (exact_qp ? WBC_QP_EXACT : 0u) |
+                                                     (warm_qp ? WBC_QP_WARM : 0u)),
               "wbc_cycle");
     }
 
@@ -242,11 +253,18 @@ public:
     // set_swing_desired: solution.*->GetPoint(t) is evaluated on the GPU (main.cpp:1004-1010, 1333-1368).
     void set_trajectory(int nseg, const double* durations, const double* nodes) { b_.set_trajectory(nseg, durations, nodes); }
     void sample_trajectory(double t) { b_.sample_trajectory(t); }
-    void cycle_stance(bool sampled_trajectory = false) { b_.mode[0] = WBC_MODE_STANCE; b_.exact_qp = exact_qp; b_.cycle(sampled_trajectory); }
+    void cycle_stance(bool sampled_trajectory = false)
+    {
+        b_.mode[0] = WBC_MODE_STANCE;
+        b_.exact_qp = exact_qp;
+        b_.warm_qp = warm_qp;
+        b_.cycle(sampled_trajectory);
+    }
     void cycle_swing(bool first_half, bool sampled_trajectory = false)
     {
         b_.mode[0] = first_half ? WBC_MODE_SWING_BR_FL : WBC_MODE_SWING_BL_FR;
         b_.exact_qp = exact_qp;
+        b_.warm_qp = warm_qp;
         b_.cycle(sampled_trajectory);
     }
 
@@ -259,6 +277,7 @@ public:
     int status() const { return b_.status[0]; }
     Batch& batch() { return b_; }
     bool exact_qp = false;  // cycles solve each QP to its exact optimum (WBC_QP_EXACT) instead of DENSE-AUL
+    bool warm_qp = false;   // with exact_qp: warm-start each cycle's QP from the previous exact-mode cycle's active set (WBC_QP_WARM)
 
 private:
     Batch b_;

@@ -20,7 +20,8 @@ import numpy as np
 from . import build as _build
 
 MODE_STANCE, MODE_SWING_BR_FL, MODE_SWING_BL_FR = 0, 1, 2
-HOST_PTRS, DEVICE_PTRS, NO_SYNC, FIFO_DISPATCH, HOST_SLAB, SAMPLED_TRAJ, QP_EXACT = 0, 1, 2, 4, 8, 16, 32
+HOST_PTRS, DEVICE_PTRS, NO_SYNC, FIFO_DISPATCH, HOST_SLAB, SAMPLED_TRAJ, QP_EXACT, QP_WARM = 0, 1, 2, 4, 8, 16, 32, 64
+FL_WARM_STARTED = 2048       # qp_info[5] of an instance that a WBC_QP_WARM cycle started from its stored active set
 ST_BAD_MODE, ST_NONFINITE, ST_INFEASIBLE, ST_NOT_PD = -20, -21, -22, -23
 SOLVER_KERNELS = {0: "wbc_solve_kernel", 1: "wbc_solve_staged_kernel", 2: "wbc_solve_exact_kernel"}
 
@@ -82,6 +83,7 @@ _lib = None
 
 EXPORTS = ["wbc_default_params", "wbc_last_error", "wbc_version", "wbc_create", "wbc_destroy", "wbc_set_params",
            "wbc_set_observer_state", "wbc_get_observer_state", "wbc_set_observer_state2", "wbc_get_observer_state2", "wbc_cycle", "wbc_debug_update", "wbc_debug_qp_records", "wbc_qp_solve",
+           "wbc_qp_solve_warm", "wbc_set_active_set", "wbc_get_active_set",
            "wbc_plant_step", "wbc_plant_dynamics_step", "wbc_last_timing", "wbc_last_solve_cycles", "wbc_last_launches", "wbc_solver_shape", "wbc_stage_profile", "wbc_host_alloc",
            "wbc_host_free",
            "wbc_set_trajectory", "wbc_sample_trajectory",
@@ -119,6 +121,10 @@ def load():
     lib.wbc_debug_update.argtypes = [C.c_void_p, C.c_int, C.POINTER(_Inputs), C.POINTER(_Debug), C.c_uint]
     lib.wbc_qp_solve.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p,
                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint]
+    lib.wbc_qp_solve_warm.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p,
+                                      C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint]
+    lib.wbc_set_active_set.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_long]
+    lib.wbc_get_active_set.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_long]
     lib.wbc_plant_step.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_long, C.c_void_p,
                                    C.c_uint]
     lib.wbc_plant_dynamics_step.argtypes = [C.c_void_p, C.c_int, C.POINTER(_PlantState), C.c_void_p, C.c_void_p, C.c_long, C.c_int, C.c_double,
@@ -141,6 +147,11 @@ def default_params():
     p = Params()
     load().wbc_default_params(C.byref(p))
     return p
+
+
+def _warm_needs_exact(warm, exact):
+    if warm and not exact:
+        raise WbcError("warm start (WBC_QP_WARM) is only available with the exact solver: pass exact=True as well")
 
 
 def _check(rc, what):
@@ -210,6 +221,18 @@ class WbcBatch:
         yg = np.zeros((6, n))
         _check(self.lib.wbc_get_observer_state2(self.h, n, yg.ctypes.data_as(_dp), n), "wbc_get_observer_state2")
         return yg
+
+    def set_active_set(self, sets):
+        """The exact-mode active sets stored per instance index, uint32 [4, n] (rows 0..2 bit masks of the active inequality rows,
+        row 3 the contact mode + 1, 0 = none): restore them with the observer state after a checkpoint or a re-sharding."""
+        sets = np.ascontiguousarray(sets, dtype=np.uint32)
+        n = sets.shape[1]
+        _check(self.lib.wbc_set_active_set(self.h, n, sets.ctypes.data, n), "wbc_set_active_set")
+
+    def get_active_set(self, n):
+        sets = np.zeros((4, n), dtype=np.uint32)
+        _check(self.lib.wbc_get_active_set(self.h, n, sets.ctypes.data, n), "wbc_get_active_set")
+        return sets
 
     @staticmethod
     def _inputs_struct(sc, n, keep, skip=()):
@@ -305,10 +328,13 @@ class WbcBatch:
         out["_slab"] = True          # cycle() passes WBC_HOST_SLAB
         return out
 
-    def cycle(self, sc, n=None, want=("x", "qp_obj", "status", "qp_info", "qp_flops"), out=None, sampled_traj=False, exact=False):
+    def cycle(self, sc, n=None, want=("x", "qp_obj", "status", "qp_info", "qp_flops"), out=None, sampled_traj=False, exact=False,
+              warm=False):
         """One control cycle on HOST (numpy) SoA inputs; returns a dict of numpy arrays [k, n].  `out`: preallocated
         result arrays to fill (e.g. page-locked ones from pinned()); its keys decide what is returned.  exact=True: solve each
-        QP to its exact optimum (WBC_QP_EXACT, the dual active-set solver) instead of DENSE-AUL at the reference's settings."""
+        QP to its exact optimum (WBC_QP_EXACT, the dual active-set solver) instead of DENSE-AUL at the reference's settings.
+        warm=True (needs exact=True): start each instance from the active set of its previous exact-mode cycle (WBC_QP_WARM)."""
+        _warm_needs_exact(warm, exact)
         keep = []
         n = int(sc["mode"].shape[0]) if n is None else int(n)
         ins = self._inputs_struct(sc, n, keep, skip=TRAJ_FIELDS if sampled_traj else ())
@@ -324,13 +350,14 @@ class WbcBatch:
         for k in ("tau", "w", "x", "qp_obj", "status", "qp_info", "qp_flops", "w3"):
             setattr(o, k, _ptr(out.get(k)))
         o.ld = max(n, 1)
-        _check(self.lib.wbc_cycle(self.h, n, C.byref(ins), C.byref(o), None, HOST_PTRS | (FIFO_DISPATCH if self.fifo_dispatch else 0) | (HOST_SLAB if sc.get("_slab") else 0) | (SAMPLED_TRAJ if sampled_traj else 0) | (QP_EXACT if exact else 0)), "wbc_cycle")
+        _check(self.lib.wbc_cycle(self.h, n, C.byref(ins), C.byref(o), None, HOST_PTRS | (FIFO_DISPATCH if self.fifo_dispatch else 0) | (HOST_SLAB if sc.get("_slab") else 0) | (SAMPLED_TRAJ if sampled_traj else 0) | (QP_EXACT if exact else 0) | (QP_WARM if warm else 0)), "wbc_cycle")
         return out
 
-    def cycle_device(self, dev_in, dev_out, n, ld, stream=None, sync=True, out_ld=None, exact=False):
+    def cycle_device(self, dev_in, dev_out, n, ld, stream=None, sync=True, out_ld=None, exact=False, warm=False):
         """One control cycle on DEVICE-resident SoA buffers (dicts of torch CUDA tensors or raw pointers).
         `ld` is the leading dimension of the input arrays, `out_ld` that of the output arrays (default: the outputs' own
-        second dimension when they are tensors, else `ld`).  exact: as in cycle()."""
+        second dimension when they are tensors, else `ld`).  exact, warm: as in cycle()."""
+        _warm_needs_exact(warm, exact)
         if out_ld is None:
             t = dev_out.get("tau")
             out_ld = int(t.stride(0)) if hasattr(t, "stride") and t.dim() == 2 else ld
@@ -354,7 +381,7 @@ class WbcBatch:
         for k in ("tau", "w", "x", "qp_obj", "status", "qp_info", "qp_flops", "w3"):
             setattr(o, k, _ptr(dev_out.get(k)))
         o.ld = out_ld
-        flags = DEVICE_PTRS | (0 if sync else NO_SYNC) | (FIFO_DISPATCH if self.fifo_dispatch else 0) | (QP_EXACT if exact else 0)
+        flags = DEVICE_PTRS | (0 if sync else NO_SYNC) | (FIFO_DISPATCH if self.fifo_dispatch else 0) | (QP_EXACT if exact else 0) | (QP_WARM if warm else 0)
         _check(self.lib.wbc_cycle(self.h, n, C.byref(ins), C.byref(o), stream, flags), "wbc_cycle")
 
     def qp_records(self, n):
@@ -379,9 +406,12 @@ class WbcBatch:
         _check(self.lib.wbc_debug_update(self.h, n, C.byref(ins), C.byref(d), HOST_PTRS), "wbc_debug_update")
         return out
 
-    def qp_solve(self, Q, c, L, neq, exact=False):
+    def qp_solve(self, Q, c, L, neq, exact=False, warm=False, active=None):
         """n dense QPs, instance-major numpy arrays Q [n,30,30], c [n,30], L [n,nrows,31] (the OPT operator).  exact=True: the
-        exact-mode solver (WBC_QP_EXACT); info then holds its counters (include/wbc_b200.h)."""
+        exact-mode solver (WBC_QP_EXACT); info then holds its counters (include/wbc_b200.h).
+        warm=True (needs exact=True; wbc_qp_solve_warm): `active` uint32 [n,3] is each instance's warm set (bit r of word r // 32:
+        inequality row r; None or zeros: a cold start); returns (x, status, info, flops, active) with the final active sets."""
+        _warm_needs_exact(warm, exact)
         Q = np.ascontiguousarray(Q, dtype=np.float64)
         c = np.ascontiguousarray(c, dtype=np.float64)
         L = np.ascontiguousarray(L, dtype=np.float64)
@@ -390,6 +420,12 @@ class WbcBatch:
         status = np.zeros(n, dtype=np.int32)
         info = np.zeros((n, 8), dtype=np.int32)
         flops = np.zeros(n)
+        if warm:
+            act = np.zeros((n, 3), np.uint32) if active is None else np.array(active, dtype=np.uint32).reshape(n, 3)
+            _check(self.lib.wbc_qp_solve_warm(self.h, n, Q.ctypes.data, c.ctypes.data, L.ctypes.data, nrows, int(neq), x.ctypes.data,
+                                              status.ctypes.data, info.ctypes.data, flops.ctypes.data, act.ctypes.data, None, HOST_PTRS),
+                   "wbc_qp_solve_warm")
+            return x, status, info, flops, act
         _check(self.lib.wbc_qp_solve(self.h, n, Q.ctypes.data, c.ctypes.data, L.ctypes.data, nrows, int(neq), x.ctypes.data,
                                      status.ctypes.data, info.ctypes.data, flops.ctypes.data, None, HOST_PTRS | (QP_EXACT if exact else 0)), "wbc_qp_solve")
         return x, status, info, flops
@@ -470,14 +506,19 @@ class OPT:
     raises WbcError instead).
     """
 
-    def __init__(self, control_variables=30, stance_constraint=86, swing_constraint=82, batch=None, exact=False):
-        """exact=True: solve to the exact optimum (WBC_QP_EXACT) instead of DENSE-AUL at the reference's settings."""
+    def __init__(self, control_variables=30, stance_constraint=86, swing_constraint=82, batch=None, exact=False, warm_start=False):
+        """exact=True: solve to the exact optimum (WBC_QP_EXACT) instead of DENSE-AUL at the reference's settings.
+        warm_start=True (needs exact=True): opt_stance and opt_swing each start from the active set of their own previous solve
+        (wbc_qp_solve_warm), which a control loop that solves almost the same QP every cycle gains from."""
+        _warm_needs_exact(warm_start, exact)
         if control_variables != 30 or stance_constraint != 86 or swing_constraint != 82:
             raise WbcError("OPT is specialised to the controller's shapes OPT(30, 86, 82) (main.cpp:266)")
         self._own = batch is None
         self._b = batch or WbcBatch(1)
         self._Q = self._c = self._Ls = self._Lw = None
         self.exact = bool(exact)
+        self.warm_start = bool(warm_start)
+        self._active = {18: np.zeros((1, 3), np.uint32), 12: np.zeros((1, 3), np.uint32)}   # opt_stance's and opt_swing's sets
 
     def setQ(self, Q_):
         self._Q = np.array(Q_, dtype=np.float64).reshape(1, 30, 30)
@@ -494,7 +535,10 @@ class OPT:
     def _solve(self, L, neq):
         if self._Q is None or self._c is None or L is None:
             raise WbcError("OPT: setQ, setc and setL_* must be called before opt_*")
-        x, status, _, _ = self._b.qp_solve(self._Q, self._c, L, neq, exact=self.exact)
+        if self.warm_start:
+            x, status, _, _, self._active[neq] = self._b.qp_solve(self._Q, self._c, L, neq, exact=True, warm=True, active=self._active[neq])
+        else:
+            x, status, _, _ = self._b.qp_solve(self._Q, self._c, L, neq, exact=self.exact)
         if status[0] != 0:
             raise WbcError("OPT: QP solver failed with status %d" % status[0])
         return x[0]

@@ -78,6 +78,12 @@ struct DualStats {
     int flags;       // FL_*
     double flops;    // instrumented algorithmic flop count
 };
+// What a caller that keeps active sets needs besides DualStats (solve_dual's `ws`, may be NULL)
+struct WarmStats {
+    int adds;        // warm start (WARM = true): rows of the warm set added before the GI loop ...
+    int drops;       // ... and dropped again for a negative multiplier before it
+    unsigned act[3]; // active inequality rows at the end (bit r: row r); 0 on failure
+};
 
 // Per-phase cycle counters of a solve (the kernel's profiled instantiation, PROF = true; see solve_dual).  Slots 0 and 8 are the
 // kernel's (record staging, validation and assembly; torque map and outputs).
@@ -88,6 +94,16 @@ WBC_HD long long dual_clock()
     return clock64();
 #else
     return 0;
+#endif
+}
+
+// index of the lowest set bit (b != 0)
+WBC_HD int low_bit(unsigned b)
+{
+#if defined(__CUDA_ARCH__)
+    return __ffs((int)b) - 1;
+#else
+    return __builtin_ctz(b);
 #endif
 }
 
@@ -159,11 +175,21 @@ WBC_HD double row_value(const Ex& ex, const double* np, const double* y, double 
 // On exit: sm + OFF_Y holds x (0 on failure); C and the rest of the shared block are overwritten.
 // PROF = true adds the SM cycles spent in each phase to pc[PH_*] (measurement only; the shipped path is PROF = false).
 //
+// ws (may be NULL) receives the final active inequality rows, and the warm phase's counters.
+// WARM = true: warm start from the inequality rows of `wset` (bit r: row r; a guess -- bits at equality rows, at rows >= nrows and
+// at rows that depend on those already active are skipped).  After the equalities, the rows of wset are added in ascending order
+// without steps (d = J'n, the dependence test, add_row); then the point and the multipliers of that active set are recomputed from
+// the factorisation, and the most negative inequality multiplier is dropped until none is negative.  That leaves the GI loop a
+// valid start: linearly independent active rows, y optimal with them held as equalities, every inequality multiplier >= 0.
+// The warm phase is bounded by the size of wset and does not count against the iteration cap; its time goes to PH_D, PH_ADD,
+// PH_ZR (the recomputation) and PH_DROP.  WARM = false compiles to the cold solver.
+//
 // The factorisation is not qp_warp.cuh's chol_cols / tri_solve: those work on DENSE-AUL's packed, transposed factor (with its
 // column-dependency and ambiguity tests for rank-deficient working sets), whereas here H is positive definite or the solve stops,
 // and the factor is only read once more -- row by row, with ld 31, by every lane forming its own row of J = L^-T in registers.
-template <class Ex, bool PROF = false>
-WBC_HDN void solve_dual(const Ex& ex, double* sm, double* C, int nrows, int neq, DualStats& st, unsigned long long* pc = nullptr)
+template <class Ex, bool PROF = false, bool WARM = false>
+WBC_HDN void solve_dual(const Ex& ex, double* sm, double* C, int nrows, int neq, DualStats& st, unsigned long long* pc = nullptr,
+                        const unsigned* wset = nullptr, WarmStats* ws = nullptr)
 {
     long long tmark = PROF ? dual_clock() : 0;
     auto mark = [&](int k) {
@@ -189,6 +215,7 @@ WBC_HDN void solve_dual(const Ex& ex, double* sm, double* C, int nrows, int neq,
     double* SN = sm + ds::OFF_SN;
     int* A = reinterpret_cast<int*>(sm + ds::OFF_A);
     st.status = ST_OK; st.nfact = 0; st.adds = 0; st.drops = 0; st.nact_ineq = 0; st.nact = 0; st.flags = FL_EXACT; st.flops = 0.0;
+    if (ws) { ws->adds = 0; ws->drops = 0; ws->act[0] = 0u; ws->act[1] = 0u; ws->act[2] = 0u; }
     double flops = 0.0;
 
     // ---- scaling: s_i = 1 / sqrt(H_ii); H <- S H S, c <- S c, rows a <- a S / |a S|, b <- b / |a S|
@@ -283,6 +310,7 @@ WBC_HDN void solve_dual(const Ex& ex, double* sm, double* C, int nrows, int neq,
     int peq = 0;                       // of which equalities (positions [0, peq))
     unsigned act[3] = {0u, 0u, 0u};    // active inequality rows (bit mask, uniform)
     double z[RPL];
+    int warm_adds = 0, warm_drops = 0;
 
     // d = J' n, |d2|^2 = sum_{j >= iq} d_j^2 and |d|^2 (uniform)
     auto compute_d = [&](double& nd2, double& nd) {
@@ -446,6 +474,96 @@ WBC_HDN void solve_dual(const Ex& ex, double* sm, double* C, int nrows, int neq,
         mark(PH_ADD);
         peq = iq;
     }
+    if constexpr (WARM) {
+        // ---- warm start: force the rows of wset into the active set (no steps), then recompute y and u for that set.  With
+        // b'_k = -b of active row k (N'y = b' on the active rows), J = [J1 J2], J1'N = R and J2'N = 0:
+        //     y = J1 R^-T b' - J2 J2' c,      u = R^-1 (R^-T b' + J1' c).
+        // NP holds b', then w = R^-T b'; D holds J' c, then w + J1' c.
+        auto fwd = [&]() {                               // NP <- R^-T NP, forward by columns of R
+            for (int k = 0; k < iq; k++) {
+                const double wk = NP[k] * RDI[k];
+                ex.sync();
+                for (int i = k + 1 + lane; i < iq; i += Ex::NL) NP[i] -= R[k * LD + i] * wk;
+                if (lane == 0) NP[k] = wk;
+                ex.sync();
+            }
+        };
+        auto recompute = [&]() {
+            for (int k = lane; k < iq; k += Ex::NL) NP[k] = -C[A[k] * LD + N];
+            ex.sync();
+            fwd();
+            jt_times(ex, J, CV, H, D);
+#pragma unroll
+            for (int q = 0; q < RPL; q++) {
+                const int i = lane + q * Ex::NL;
+                if (i < N) {
+                    double s = 0.0;
+#pragma unroll
+                    for (int j = 0; j < N; j++) s += (j < iq) ? J[q][j] * NP[j] : -(J[q][j] * D[j]);
+                    Y[i] = s;
+                }
+            }
+            for (int k = lane; k < iq; k += Ex::NL) D[k] += NP[k];
+            ex.sync();
+            // one refinement of y on the active rows' residuals b' - N'y = a.y - b (y += J1 R^-T r): the forced rows meet at
+            // degenerate vertices, where a residual left by the cancellation in J1 w - J2 J2' c would show a row through the
+            // vertex as violated and cost the GI loop a dual step
+            for (int k = lane; k < iq; k += Ex::NL) {
+                const double* a = C + A[k] * LD;
+                double s = -a[N];
+                for (int j = 0; j < N; j++) s += a[j] * Y[j];
+                NP[k] = s;
+            }
+            ex.sync();
+            fwd();
+#pragma unroll
+            for (int q = 0; q < RPL; q++) {
+                const int i = lane + q * Ex::NL;
+                if (i < N) {
+                    double s = 0.0;
+#pragma unroll
+                    for (int j = 0; j < N; j++) s += (j < iq) ? J[q][j] * NP[j] : 0.0;
+                    Y[i] += s;
+                }
+            }
+            ex.sync();
+            compute_r();
+            for (int k = lane; k < 32; k += Ex::NL) U[k] = (k < iq) ? RV[k] : 0.0;
+            ex.sync();
+            flops += 3.0 * iq * iq + 1800.0 + 2.0 * N * N + 4.0 * N * iq;
+        };
+        if (st.status == ST_OK && wset) {
+#pragma unroll 1
+            for (int w = 0; w < 3; w++) {
+                unsigned bits = wset[w];
+                while (bits) {
+                    const int row = 32 * w + low_bit(bits);
+                    bits &= bits - 1u;
+                    if (row < neq || row >= nrows) continue;
+                    load_row(row);
+                    double nd2, nd;
+                    compute_d(nd2, nd);
+                    mark(PH_D);
+                    if (nd2 <= TOL_DEP * TOL_DEP * nd) continue;     // depends on the active rows (or 30 are active)
+                    add_row(row, nd2);
+                    mark(PH_ADD);
+                    warm_adds++;
+                }
+            }
+            while (warm_adds > 0) {
+                recompute();
+                mark(PH_ZR);
+                double umin = 0.0;
+                int kp = -1;
+                for (int k = peq; k < iq; k++)
+                    if (U[k] < umin) { umin = U[k]; kp = k; }
+                if (kp < 0) break;
+                drop_at(kp);
+                warm_drops++;
+                mark(PH_DROP);
+            }
+        }
+    }
     // ---- inequalities
     while (st.status == ST_OK) {
         const int ip = most_violated(ex, C, Y, nrows, neq, act);
@@ -504,6 +622,10 @@ WBC_HDN void solve_dual(const Ex& ex, double* sm, double* C, int nrows, int neq,
     st.nact = iq;
     st.nact_ineq = iq - peq;
     st.flops = flops;
+    if (ws) {
+        ws->adds = warm_adds; ws->drops = warm_drops;
+        for (int w = 0; w < 3; w++) ws->act[w] = (st.status == ST_OK) ? act[w] : 0u;
+    }
     mark(PH_STEP);
 }
 

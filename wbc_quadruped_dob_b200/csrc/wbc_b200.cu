@@ -7,7 +7,8 @@
 //                      4..50 Cholesky per solve): assemble (Q,c,L) from the record, DENSE-AUL/QQP solve with the
 //                      hot state in shared memory (qp_warp.cuh), torque map.
 //   wbc_solve_exact_kernel  (WBC_QP_EXACT) in place of wbc_solve_kernel: the same warp-per-instance persistent shape around the
-//                      Goldfarb-Idnani dual active-set solver of qp_dual.cuh (the exact optimum of each QP).
+//                      Goldfarb-Idnani dual active-set solver of qp_dual.cuh (the exact optimum of each QP); its WARM
+//                      instantiation (WBC_QP_WARM) starts each instance from the active set of its previous exact-mode cycle.
 // There is no CPU fallback anywhere in this file.
 #include <cuda_runtime.h>
 #include <stdio.h>
@@ -340,24 +341,32 @@ constexpr int EXACT_T = 32;
 constexpr int EXACT_MIN_CTAS = WBC_EXACT_MIN_CTAS;
 static_assert(wbc::QR_MODE + 1 <= wbcdual::N * wbcdual::LD, "the QP record is staged in R's place");
 
-__device__ __forceinline__ void write_info_exact(const wbcdual::DualStats& st, long i, long ld, int* status, int* info, double* flops)
+// ws (warm mode): [6], [7] are the warm rows added and dropped before the GI loop (0 in cold exact mode)
+__device__ __forceinline__ void write_info_exact(const wbcdual::DualStats& st, long i, long ld, int* status, int* info, double* flops,
+                                                 const wbcdual::WarmStats* ws = nullptr)
 {
     if (status) status[i] = st.status;
     if (info) {
         info[0 * ld + i] = st.nfact; info[1 * ld + i] = st.adds; info[2 * ld + i] = st.drops; info[3 * ld + i] = st.nact_ineq;
-        info[4 * ld + i] = st.nact; info[5 * ld + i] = st.flags; info[6 * ld + i] = 0; info[7 * ld + i] = 0;
+        info[4 * ld + i] = st.nact; info[5 * ld + i] = st.flags; info[6 * ld + i] = ws ? ws->adds : 0; info[7 * ld + i] = ws ? ws->drops : 0;
     }
     if (flops) flops[i] = st.flops;
 }
 
+// qp_info[5] flag of an instance that wbc_cycle with WBC_QP_WARM started from its stored active set
+constexpr int FL_WARM_STARTED = 2048;
+
 // PROF = true (a ctx created with WBC_STAGE_PROF=1): per-warp cycle counters by phase, rows of 12 in `prof` (wbc_stage_profile):
 // [0..8] the wbcdual::PH_* phases summed over the warp's solves, [9] solves, [10] rows added + dropped, [11] cycles in the kernel.
-template <bool PROF>
+// aset [4][aset_ld]: the ctx's stored active set per instance index -- words 0..2 the active inequality rows, word 3 the contact
+// mode they were solved in + 1 (0: none).  Every instance writes its own (its final set, or none when it failed or was refused);
+// WARM = true (WBC_QP_WARM) first reads it and starts from it when the stored mode is the instance's mode.
+template <bool PROF, bool WARM = false>
 __global__ void __launch_bounds__(EXACT_T, EXACT_MIN_CTAS) wbc_solve_exact_kernel(Params P, int n, const double* __restrict__ recs, SolveOut out,
                                                                                  double* __restrict__ scratch_base, int* __restrict__ queue,
                                                                                  const int* __restrict__ order, unsigned* __restrict__ cost,
                                                                                  int* __restrict__ hist_next, unsigned long long* __restrict__ prof,
-                                                                                 int prof_rows)
+                                                                                 int prof_rows, unsigned* __restrict__ aset, long aset_ld)
 {
     const WarpEx ex;
     unsigned long long pc[12];
@@ -395,6 +404,7 @@ __global__ void __launch_bounds__(EXACT_T, EXACT_MIN_CTAS) wbc_solve_exact_kerne
                     if (out.qp_obj) out.qp_obj[i] = 0.0;
                     cost[i] = 0u;
                     atomicAdd(hist_next, 1);
+                    for (int k = 0; k < 4; k++) aset[k * aset_ld + i] = 0u;
                 }
                 ex.sync();
                 continue;
@@ -403,7 +413,13 @@ __global__ void __launch_bounds__(EXACT_T, EXACT_MIN_CTAS) wbc_solve_exact_kerne
         const QpShape sh = qp_shape((int)rec[QR_MODE]);
         assemble_qp<wbcdual::LD>(ex, P, rec, sh, sm + wbcdual::ds::OFF_H, sm + wbcdual::ds::OFF_CV, C);
         if (PROF) pc[wbcdual::PH_ASSEMBLE] += (unsigned long long)(clock64() - t0);
-        wbcdual::solve_dual<WarpEx, PROF>(ex, sm, C, sh.nrows, sh.neq, st, pc);
+        unsigned wset[3] = {0u, 0u, 0u};
+        if constexpr (WARM) {
+            if (aset[3 * aset_ld + i] == (unsigned)rec[QR_MODE] + 1u)
+                for (int k = 0; k < 3; k++) wset[k] = aset[k * aset_ld + i];
+        }
+        wbcdual::WarmStats ws;
+        wbcdual::solve_dual<WarpEx, PROF, WARM>(ex, sm, C, sh.nrows, sh.neq, st, pc, wset, &ws);
         const long long t1 = PROF ? clock64() : 0;
         const double* xs = sm + wbcdual::ds::OFF_Y;          // x, or 0 when the solve failed
         ex.copy_in(rec, recs + (long)i * QPREC_DOUBLES, QR_MODE + 1);     // R's place was the solver's; stage again
@@ -416,7 +432,11 @@ __global__ void __launch_bounds__(EXACT_T, EXACT_MIN_CTAS) wbc_solve_exact_kerne
         if (out.x)
             for (int k = ex.lane(); k < 30; k += EXACT_T) out.x[(long)k * out.ld + i] = xs[k];
         if (ex.lane() == 0) {
-            write_info_exact(st, i, out.ld, out.status, out.qp_info, out.qp_flops);
+            const unsigned mode1 = (unsigned)rec[QR_MODE] + 1u;      // rec is staged again: the mode is read after the solve
+            if (WARM && aset[3 * aset_ld + i] == mode1) st.flags |= FL_WARM_STARTED;
+            write_info_exact(st, i, out.ld, out.status, out.qp_info, out.qp_flops, WARM ? &ws : nullptr);
+            for (int k = 0; k < 3; k++) aset[k * aset_ld + i] = ws.act[k];
+            aset[3 * aset_ld + i] = st.status == 0 ? mode1 : 0u;
             // the duration orders the next cycle's dispatch (longest first), as in wbc_solve_kernel: one bucket entry per instance
             const unsigned long long dt = (unsigned long long)(clock64() - t0) >> 10;
             const unsigned cu = dt > 0xffffffffull ? 0xffffffffu : (unsigned)dt;
@@ -437,10 +457,13 @@ __global__ void __launch_bounds__(EXACT_T, EXACT_MIN_CTAS) wbc_solve_exact_kerne
 }
 
 // Dense-input form of the exact solver (wbc_qp_solve with WBC_QP_EXACT): Q [n][900], c [n][30], L [n][nrows*31], x [n][30].
+// WARM = true (wbc_qp_solve_warm): active [n][3] is read as each instance's warm set and overwritten with its final active
+// inequality rows (0 on failure).
+template <bool WARM = false>
 __global__ void __launch_bounds__(EXACT_T, EXACT_MIN_CTAS) wbc_dense_qp_exact_kernel(int n, const double* __restrict__ Q, const double* __restrict__ c,
                                                                                     const double* __restrict__ L, int nrows, int neq, double* __restrict__ x,
                                                                                     int* status, int* info, double* flops, double* __restrict__ scratch_base,
-                                                                                    int* __restrict__ queue)
+                                                                                    int* __restrict__ queue, unsigned* __restrict__ active = nullptr)
 {
     const WarpEx ex;
     double* sm = wbc_smem;
@@ -457,10 +480,14 @@ __global__ void __launch_bounds__(EXACT_T, EXACT_MIN_CTAS) wbc_dense_qp_exact_ke
         for (int k = ex.lane(); k < nrows * 31; k += EXACT_T) { const double v = L[(long)i * nrows * 31 + k]; C[k] = v; chk += v * 0.0; }
         ex.sync();
         wbcdual::DualStats st;
+        wbcdual::WarmStats ws;
         if (__any_sync(0xffffffffu, chk != 0.0)) {
             st.status = WBC_ST_NONFINITE; st.nfact = 0; st.adds = 0; st.drops = 0; st.nact_ineq = 0; st.nact = 0; st.flags = wbcdual::FL_EXACT; st.flops = 0.0;
+            if constexpr (WARM) { ws.adds = 0; ws.drops = 0; ws.act[0] = 0u; ws.act[1] = 0u; ws.act[2] = 0u; }
             for (int k = ex.lane(); k < 30; k += EXACT_T) sm[wbcdual::ds::OFF_Y + k] = 0.0;
             ex.sync();
+        } else if constexpr (WARM) {
+            wbcdual::solve_dual<WarpEx, false, true>(ex, sm, C, nrows, neq, st, nullptr, active + (long)i * 3, &ws);
         } else
             wbcdual::solve_dual(ex, sm, C, nrows, neq, st);
         for (int k = ex.lane(); k < 30; k += EXACT_T) x[(long)i * 30 + k] = sm[wbcdual::ds::OFF_Y + k];
@@ -469,8 +496,11 @@ __global__ void __launch_bounds__(EXACT_T, EXACT_MIN_CTAS) wbc_dense_qp_exact_ke
             if (flops) flops[i] = st.flops;
             if (info) {
                 int* q = info + (long)i * 8;
-                q[0] = st.nfact; q[1] = st.adds; q[2] = st.drops; q[3] = st.nact_ineq; q[4] = st.nact; q[5] = st.flags; q[6] = 0; q[7] = 0;
+                q[0] = st.nfact; q[1] = st.adds; q[2] = st.drops; q[3] = st.nact_ineq; q[4] = st.nact; q[5] = st.flags;
+                q[6] = WARM ? ws.adds : 0; q[7] = WARM ? ws.drops : 0;
             }
+            if constexpr (WARM)
+                for (int k = 0; k < 3; k++) active[(long)i * 3 + k] = ws.act[k];
         }
         ex.sync();
     }
@@ -918,6 +948,8 @@ struct wbc_ctx {
     int solve_smem;         // dynamic shared memory per solver CTA (sl::BYTES, or padded by WBC_SOLVE_CTAS_PER_SM)
     int exact_per_sm;       // exact-mode kernel (WBC_QP_EXACT): resident CTAs per SM (occupancy calculator) ...
     int exact_blocks;       // ... its persistent grid: every resident CTA that has a scratch block (wbcdual::SCRATCH_DOUBLES each)
+    unsigned* aset;         // [4][max_batch] exact mode: each instance's active inequality rows (words 0..2) and contact mode + 1 (word 3,
+                            // 0 = none) of its last exact-mode solve; the warm set of WBC_QP_WARM
     // staging for WBC_HOST_PTRS
     double* d_in;        // [93+40][max_batch]
     double* d_out;       // [62][max_batch]
@@ -960,7 +992,7 @@ int wbc_destroy(wbc_ctx* c)
 {
     if (!c) return WBC_OK;
     cudaSetDevice(c->device);
-    cudaFree(c->recs); cudaFree(c->yd); cudaFree(c->yw); cudaFree(c->yg); cudaFree(c->w_dev); cudaFree(c->tau_prev); cudaFree(c->scratch); cudaFree(c->kkt); cudaFree(c->sq_ctl); cudaFree(c->sq_ring); cudaFree(c->prof); cudaFree(c->queue); cudaFree(c->lanes); cudaFree(c->cost); cudaFree(c->cycles); cudaFree(c->order);
+    cudaFree(c->recs); cudaFree(c->yd); cudaFree(c->yw); cudaFree(c->yg); cudaFree(c->w_dev); cudaFree(c->tau_prev); cudaFree(c->scratch); cudaFree(c->kkt); cudaFree(c->sq_ctl); cudaFree(c->sq_ring); cudaFree(c->prof); cudaFree(c->queue); cudaFree(c->lanes); cudaFree(c->cost); cudaFree(c->cycles); cudaFree(c->order); cudaFree(c->aset);
     cudaFree(c->traj_dur); cudaFree(c->traj_nodes); cudaFree(c->traj_s); cudaFree(c->traj_t);
     cudaFree(c->d_in); cudaFree(c->d_out); cudaFree(c->d_mode); cudaFree(c->d_iout); cudaFree(c->d_dense);
     if (c->h_pin) cudaFreeHost(c->h_pin);
@@ -1073,6 +1105,8 @@ int wbc_create(wbc_ctx** out, int device, int max_batch, const wbc_params* param
     TRY(cudaMemset(c->lanes, 0, LANES_INTS * sizeof(int)));
     TRY(cudaMemset(c->queue, 0, (1 + 3 * ORD_NB) * sizeof(int)));
     TRY(cudaMalloc(&c->cost, nb * sizeof(unsigned)));
+    TRY(cudaMalloc(&c->aset, nb * 4 * sizeof(unsigned)));
+    TRY(cudaMemset(c->aset, 0, nb * 4 * sizeof(unsigned)));
     TRY(cudaMalloc(&c->cycles, nb * sizeof(unsigned)));
     TRY(cudaMalloc(&c->order, nb * sizeof(int)));
     TRY(cudaMalloc(&c->d_in, nb * (kInDoublesNoTerrain + 41) * sizeof(double)));
@@ -1094,7 +1128,10 @@ int wbc_create(wbc_ctx** out, int device, int max_batch, const wbc_params* param
     TRY(cudaFuncSetAttribute(wbc_dense_qp_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     TRY(cudaFuncSetAttribute(wbc_solve_exact_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     TRY(cudaFuncSetAttribute(wbc_solve_exact_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    TRY(cudaFuncSetAttribute(wbc_dense_qp_exact_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    TRY(cudaFuncSetAttribute(wbc_solve_exact_kernel<false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    TRY(cudaFuncSetAttribute(wbc_solve_exact_kernel<true, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    TRY(cudaFuncSetAttribute(wbc_dense_qp_exact_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    TRY(cudaFuncSetAttribute(wbc_dense_qp_exact_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     if (l1_ctas > 0) {
         const int pct = (int)((100L * l1_ctas * (sl::BYTES + 1024) + 228 * 1024 - 1) / (228 * 1024));
         TRY(cudaFuncSetAttribute(wbc_solve_staged_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct > 100 ? 100 : pct));
@@ -1280,6 +1317,8 @@ int wbc_cycle(wbc_ctx* c, int n, const wbc_inputs* in, const wbc_outputs* out, v
     if (!out->tau || out->ld < n) return fail(WBC_EINVAL, "wbc_cycle: outputs.tau is required and outputs.ld >= n");
     const bool dev_ptrs = (flags & WBC_DEVICE_PTRS) != 0;
     const bool exact = (flags & WBC_QP_EXACT) != 0;
+    const bool warm = (flags & WBC_QP_WARM) != 0;
+    if (warm && !exact) return fail(WBC_EINVAL, "wbc_cycle: WBC_QP_WARM is only valid together with WBC_QP_EXACT");
     if (sampled && c->traj_sampled_n < n) return fail(WBC_EINVAL, "wbc_cycle: WBC_SAMPLED_TRAJ without a wbc_sample_trajectory(out = NULL) covering n instances");
     if (sampled && dev_ptrs && in->ld != c->max_batch)
         return fail(WBC_EINVAL, "wbc_cycle: WBC_SAMPLED_TRAJ with device pointers needs inputs.ld == max_batch (or sample into your own arrays)");
@@ -1394,12 +1433,20 @@ int wbc_cycle(wbc_ctx* c, int n, const wbc_inputs* in, const wbc_outputs* out, v
     if (n < nblocks) nblocks = n;
     c->last_grid = nblocks;
     if (exact) {
-        if (c->prof)
-            wbc_solve_exact_kernel<true><<<nblocks, EXACT_T, smem, s>>>(c->params, n, c->recs, so, c->scratch, counter, ordered ? c->order : nullptr,
-                                                                        c->cost, hist_next, c->prof, c->prof_rows);
+        const int* ordp = ordered ? c->order : nullptr;
+        const long mb = c->max_batch;
+        if (c->prof && warm)
+            wbc_solve_exact_kernel<true, true><<<nblocks, EXACT_T, smem, s>>>(c->params, n, c->recs, so, c->scratch, counter, ordp, c->cost, hist_next,
+                                                                              c->prof, c->prof_rows, c->aset, mb);
+        else if (c->prof)
+            wbc_solve_exact_kernel<true><<<nblocks, EXACT_T, smem, s>>>(c->params, n, c->recs, so, c->scratch, counter, ordp, c->cost, hist_next,
+                                                                        c->prof, c->prof_rows, c->aset, mb);
+        else if (warm)
+            wbc_solve_exact_kernel<false, true><<<nblocks, EXACT_T, smem, s>>>(c->params, n, c->recs, so, c->scratch, counter, ordp, c->cost, hist_next,
+                                                                               nullptr, 0, c->aset, mb);
         else
-            wbc_solve_exact_kernel<false><<<nblocks, EXACT_T, smem, s>>>(c->params, n, c->recs, so, c->scratch, counter, ordered ? c->order : nullptr,
-                                                                         c->cost, hist_next, nullptr, 0);
+            wbc_solve_exact_kernel<false><<<nblocks, EXACT_T, smem, s>>>(c->params, n, c->recs, so, c->scratch, counter, ordp, c->cost, hist_next,
+                                                                         nullptr, 0, c->aset, mb);
     } else if (staged) {
         StageQueues sq;
         sq.ctl = c->sq_ctl; sq.ring = c->sq_ring; sq.rmask = c->sq_rsize - 1; sq.nslots = c->nslots;
@@ -1743,8 +1790,9 @@ int wbc_debug_qp_records(wbc_ctx* c, int n, double* recs, int* doubles_per_recor
     return WBC_OK;
 }
 
-int wbc_qp_solve(wbc_ctx* c, int n, const double* Q, const double* cvec, const double* L, int nrows, int neq, double* x, int* status,
-                 int* info, double* flops, void* cuda_stream, unsigned flags)
+// wbc_qp_solve, and wbc_qp_solve_warm (active != NULL: the exact solver's warm instantiation, active [n][3] in/out)
+static int qp_solve_impl(wbc_ctx* c, int n, const double* Q, const double* cvec, const double* L, int nrows, int neq, double* x, int* status,
+                         int* info, double* flops, unsigned* active, void* cuda_stream, unsigned flags)
 {
     if (!c || !Q || !cvec || !L || !x) return fail(WBC_EINVAL, "wbc_qp_solve: null argument");
     if (n < 0 || n > c->max_batch) return fail(WBC_EINVAL, "wbc_qp_solve: n outside [0, max_batch]");
@@ -1759,8 +1807,9 @@ int wbc_qp_solve(wbc_ctx* c, int n, const double* Q, const double* cvec, const d
     double* dx = x;
     int *dstatus = status, *dinfo = info;
     double* dflops = flops;
+    unsigned* dactive = active;
     if (!dev_ptrs) {
-        const size_t need = (nq + nc + nl + nx + n) * sizeof(double) + (size_t)n * 9 * sizeof(int);
+        const size_t need = (nq + nc + nl + nx + n) * sizeof(double) + (size_t)n * (active ? 12 : 9) * sizeof(int);
         if (need > c->dense_cap) {
             CU(cudaStreamSynchronize(s));
             cudaFree(c->d_dense);
@@ -1778,13 +1827,20 @@ int wbc_qp_solve(wbc_ctx* c, int n, const double* Q, const double* cvec, const d
         int* ip = reinterpret_cast<int*>(p);
         dstatus = status ? ip : nullptr;
         dinfo = info ? ip + n : nullptr;
+        if (active) {
+            dactive = reinterpret_cast<unsigned*>(ip + 9L * n);
+            CU(cudaMemcpyAsync(dactive, active, (size_t)n * 3 * sizeof(unsigned), cudaMemcpyHostToDevice, s));
+        }
     }
     CU(cudaMemsetAsync(c->queue + ORD_NB, 0, sizeof(int), s));
-    const bool exact = (flags & WBC_QP_EXACT) != 0;
+    const bool exact = active || (flags & WBC_QP_EXACT) != 0;
     const int nblocks = exact ? (n < c->exact_blocks ? n : c->exact_blocks) : (n < c->nblocks ? n : c->nblocks);
     CU(cudaEventRecord(c->ev0, s));
     CU(cudaEventRecord(c->ev1, s));
-    if (exact)
+    if (active)
+        wbc_dense_qp_exact_kernel<true><<<nblocks, EXACT_T, wbcdual::ds::BYTES, s>>>(n, dQ, dc, dL, nrows, neq, dx, dstatus, dinfo, dflops, c->scratch,
+                                                                                      c->queue + ORD_NB, dactive);
+    else if (exact)
         wbc_dense_qp_exact_kernel<<<nblocks, EXACT_T, wbcdual::ds::BYTES, s>>>(n, dQ, dc, dL, nrows, neq, dx, dstatus, dinfo, dflops, c->scratch,
                                                                                 c->queue + ORD_NB);
     else
@@ -1797,10 +1853,44 @@ int wbc_qp_solve(wbc_ctx* c, int n, const double* Q, const double* cvec, const d
         if (flops) CU(cudaMemcpyAsync(flops, dflops, (size_t)n * 8, cudaMemcpyDeviceToHost, s));
         if (status) CU(cudaMemcpyAsync(status, dstatus, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
         if (info) CU(cudaMemcpyAsync(info, dinfo, (size_t)n * 8 * 4, cudaMemcpyDeviceToHost, s));
+        if (active) CU(cudaMemcpyAsync(active, dactive, (size_t)n * 3 * sizeof(unsigned), cudaMemcpyDeviceToHost, s));
         CU(cudaStreamSynchronize(s));
     } else if (!(flags & WBC_NO_SYNC)) {
         CU(cudaStreamSynchronize(s));
     }
+    return WBC_OK;
+}
+
+int wbc_qp_solve(wbc_ctx* c, int n, const double* Q, const double* cvec, const double* L, int nrows, int neq, double* x, int* status,
+                 int* info, double* flops, void* cuda_stream, unsigned flags)
+{
+    return qp_solve_impl(c, n, Q, cvec, L, nrows, neq, x, status, info, flops, nullptr, cuda_stream, flags);
+}
+
+int wbc_qp_solve_warm(wbc_ctx* c, int n, const double* Q, const double* cvec, const double* L, int nrows, int neq, double* x, int* status,
+                      int* info, double* flops, unsigned* active, void* cuda_stream, unsigned flags)
+{
+    if (!active) return fail(WBC_EINVAL, "wbc_qp_solve_warm: null argument");
+    return qp_solve_impl(c, n, Q, cvec, L, nrows, neq, x, status, info, flops, active, cuda_stream, flags);
+}
+
+int wbc_set_active_set(wbc_ctx* c, int n, const unsigned* sets, long ld)
+{
+    if (!c || !sets || n < 0 || n > c->max_batch || ld < n) return fail(WBC_EINVAL, "wbc_set_active_set: bad arguments");
+    if (n == 0) return WBC_OK;
+    CU(cudaSetDevice(c->device));
+    CU(cudaStreamSynchronize(c->stream));
+    CU(cudaMemcpy2D(c->aset, (size_t)c->max_batch * 4, sets, (size_t)ld * 4, (size_t)n * 4, 4, cudaMemcpyHostToDevice));
+    return WBC_OK;
+}
+
+int wbc_get_active_set(wbc_ctx* c, int n, unsigned* sets, long ld)
+{
+    if (!c || !sets || n < 0 || n > c->max_batch || ld < n) return fail(WBC_EINVAL, "wbc_get_active_set: bad arguments");
+    if (n == 0) return WBC_OK;
+    CU(cudaSetDevice(c->device));
+    CU(cudaStreamSynchronize(c->stream));
+    CU(cudaMemcpy2D(sets, (size_t)ld * 4, c->aset, (size_t)c->max_batch * 4, (size_t)n * 4, 4, cudaMemcpyDeviceToHost));
     return WBC_OK;
 }
 
