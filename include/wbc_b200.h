@@ -261,6 +261,36 @@ typedef struct wbc_plant_state {
 int wbc_plant_dynamics_step(wbc_ctx* ctx, int n, const wbc_plant_state* st, const double* tau, const double* push, long ld, int substeps,
                             double gamma, double* diag, void* cuda_stream, unsigned flags);
 
+/* Contact plant: forward dynamics with unilateral, frictional point contacts at the feet (DESIGN.md 4.5).  One control period
+ * (params.obs_dt) of every robot under the joint torques `tau` [12][ld] and the world wrench `push` [6][ld] at the CoM, in `substeps`
+ * steps of dt.  Each foot point k (stacked order) has its own horizontal ground plane z = ground_z[k] ([4][ld], NULL = 0) and friction
+ * coefficient mu ([1][ld], NULL = params.mu; mu >= 0).  Per step: nu_free = nu + dt M^-1 (S'tau + push_gen - h); the candidate feet
+ * are those whose gap phi_k = p_k,z - ground_z[k] <= margin (geometry only: st->mode is not read and may be NULL); the contact
+ * impulses lambda (3 per candidate foot, world axes) are the unique minimiser of
+ *     min 1/2 lambda'(G + eps D) lambda + lambda'(J nu_free - b),   G = J M^-1 J', D = diag(G),
+ * over every candidate foot's friction pyramid (lambda_z >= 0, |lambda_x|, |lambda_y| <= mu lambda_z), with b = 0 tangentially and
+ * -phi/dt (phi >= 0) or -beta phi/dt (phi < 0) along the normal; nu+ = nu_free + M^-1 J' lambda, then semi-implicit Euler.  This is
+ * the convex (Anitescu-type) relaxation of Coulomb contact: a sticking foot is exact; a sliding foot drifts off the plane at a normal
+ * velocity of at most mu times its slip speed.  Each QP is solved to its KKT optimum (a Goldfarb-Idnani dual active-set method,
+ * warm-started from the previous step's active rows, at most max_iter dual steps).
+ * The state advances in place; foot_force receives the last step's contact forces lambda/dt in the sensor frames (R_foot' lambda / dt,
+ * 0 off contact), as from wbc_plant_dynamics_step.  contact [4][ld] (may be NULL), last step: 0 no contact force, 1 sticking,
+ * 2 sliding (a friction row active) -- a gait loop can end a swing phase on touchdown.  diag [4][ld] (may be NULL): largest
+ * penetration over the steps (gaps at each step's start), smallest normal force of a candidate foot, largest scaled KKT residual of
+ * the contact QPs, total dual active-set steps.  status [ld] (may be NULL): 0; WBC_ST_NONFINITE for a NaN or infinity among the
+ * inputs or produced from them; -100 when a contact QP reaches max_iter.  A failed instance's state (foot_force included) is left
+ * as it was at the start of the call, and its contact flags are 0.  Host or device pointers per flags, like wbc_plant_dynamics_step. */
+typedef struct wbc_contact_params {
+    double beta;     /* 0.2:  Baumgarte factor of the push-out of a penetrating foot          */
+    double eps;      /* 1e-8: regularisation of the Delassus matrix, G + eps diag(G)           */
+    double margin;   /* 2e-3: a foot is a contact candidate when its gap is <= margin (m)     */
+    int max_iter;    /* 64:   dual active-set steps per contact QP before status -100          */
+} wbc_contact_params;
+void wbc_default_contact_params(wbc_contact_params* cp);
+int wbc_plant_contact_step(wbc_ctx* ctx, int n, const wbc_plant_state* st, const double* tau, const double* push, const double* ground_z,
+                           const double* mu, long ld, int substeps, const wbc_contact_params* cp, int* contact, double* diag, int* status,
+                           void* cuda_stream, unsigned flags);
+
 /* Device-side timing of the last wbc_cycle on this ctx (CUDA events on the launching stream), ms. */
 int wbc_last_timing(wbc_ctx* ctx, float* front_ms, float* solve_ms);
 /* Per-instance solve duration of the last wbc_cycle on this ctx, in SM clock cycles (clock64 around the instance's

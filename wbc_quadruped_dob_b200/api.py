@@ -64,6 +64,14 @@ class _PlantState(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("base_pos", "base_rot", "base_rpy", "base_vel", "q", "dq", "foot_force", "mode")]
 
 
+class ContactParams(C.Structure):
+    """wbc_contact_params: Baumgarte factor, Delassus regularisation, candidate margin (m), dual steps per contact QP."""
+    _fields_ = [("beta", C.c_double), ("eps", C.c_double), ("margin", C.c_double), ("max_iter", C.c_int)]
+
+
+CONTACT_NONE, CONTACT_STICK, CONTACT_SLIDE = 0, 1, 2
+
+
 class _Trajectory(C.Structure):
     _fields_ = [("nseg", C.c_int), ("durations", C.c_void_p), ("nodes", C.c_void_p), ("ld", C.c_long)]
 
@@ -84,7 +92,7 @@ _lib = None
 EXPORTS = ["wbc_default_params", "wbc_last_error", "wbc_version", "wbc_create", "wbc_destroy", "wbc_set_params",
            "wbc_set_observer_state", "wbc_get_observer_state", "wbc_set_observer_state2", "wbc_get_observer_state2", "wbc_cycle", "wbc_debug_update", "wbc_debug_qp_records", "wbc_qp_solve",
            "wbc_qp_solve_warm", "wbc_set_active_set", "wbc_get_active_set",
-           "wbc_plant_step", "wbc_plant_dynamics_step", "wbc_last_timing", "wbc_last_solve_cycles", "wbc_last_launches", "wbc_solver_shape", "wbc_stage_profile", "wbc_host_alloc",
+           "wbc_plant_step", "wbc_plant_dynamics_step", "wbc_default_contact_params", "wbc_plant_contact_step", "wbc_last_timing", "wbc_last_solve_cycles", "wbc_last_launches", "wbc_solver_shape", "wbc_stage_profile", "wbc_host_alloc",
            "wbc_host_free",
            "wbc_set_trajectory", "wbc_sample_trajectory",
            "wbc_measure_dfma_peak"]
@@ -129,6 +137,9 @@ def load():
                                    C.c_uint]
     lib.wbc_plant_dynamics_step.argtypes = [C.c_void_p, C.c_int, C.POINTER(_PlantState), C.c_void_p, C.c_void_p, C.c_long, C.c_int, C.c_double,
                                             C.c_void_p, C.c_void_p, C.c_uint]
+    lib.wbc_default_contact_params.argtypes = [C.POINTER(ContactParams)]
+    lib.wbc_plant_contact_step.argtypes = [C.c_void_p, C.c_int, C.POINTER(_PlantState), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_long,
+                                           C.c_int, C.POINTER(ContactParams), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint]
     lib.wbc_last_timing.argtypes = [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_float)]
     lib.wbc_last_solve_cycles.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_ulonglong)]
     lib.wbc_last_launches.argtypes = [C.c_void_p]
@@ -147,6 +158,12 @@ def default_params():
     p = Params()
     load().wbc_default_params(C.byref(p))
     return p
+
+
+def default_contact_params():
+    cp = ContactParams()
+    load().wbc_default_contact_params(C.byref(cp))
+    return cp
 
 
 def _warm_needs_exact(warm, exact):
@@ -460,6 +477,34 @@ class WbcBatch:
         flags = (HOST_PTRS if host else DEVICE_PTRS) | (0 if (sync or host) else NO_SYNC)
         _check(self.lib.wbc_plant_dynamics_step(self.h, n, C.byref(ps), _ptr(tau), _ptr(push), ld, int(substeps), float(gamma), _ptr(diag), stream, flags),
                "wbc_plant_dynamics_step")
+
+    def plant_contact_step(self, state, tau, push, ground_z=None, mu=None, n=None, ld=None, substeps=5, params=None, contact=None, diag=None,
+                           status=None, stream=None, sync=True):
+        """Contact plant (wbc_plant_contact_step): unilateral, frictional foot contacts on per-foot ground planes.  `state` is a dict
+        with base_pos, base_rot, base_rpy, base_vel, q, dq, foot_force (numpy arrays: host path, advanced in place; torch CUDA tensors:
+        device path); its mode is not read.  ground_z [4, ld] (None: 0), mu [ld] (None: params.mu), params a ContactParams (None:
+        the defaults); contact int32 [4, ld], diag [4, ld] and status int32 [ld] are filled when given."""
+        host = isinstance(state["q"], np.ndarray)
+        n = int(state["q"].shape[1]) if n is None else int(n)
+        ld = n if ld is None else int(ld)
+        ps = _PlantState()
+        for k in ("base_pos", "base_rot", "base_rpy", "base_vel", "q", "dq", "foot_force"):
+            setattr(ps, k, _ptr(state[k]))
+        ps.mode = _ptr(state.get("mode"))
+        keep = []
+        if host:
+            for a in (state["base_pos"], state["base_rot"], state["base_rpy"], state["base_vel"], state["q"], state["dq"], state["foot_force"], diag):
+                assert a is None or (a.flags.c_contiguous and a.dtype == np.float64)
+            for a in (contact, status):
+                assert a is None or (a.flags.c_contiguous and a.dtype == np.int32)
+            tau, push = np.ascontiguousarray(tau, dtype=np.float64), np.ascontiguousarray(push, dtype=np.float64)
+            ground_z = None if ground_z is None else np.ascontiguousarray(ground_z, dtype=np.float64)
+            mu = None if mu is None else np.ascontiguousarray(mu, dtype=np.float64)
+            keep += [tau, push, ground_z, mu]
+        cp = params if params is not None else default_contact_params()
+        flags = (HOST_PTRS if host else DEVICE_PTRS) | (0 if (sync or host) else NO_SYNC)
+        _check(self.lib.wbc_plant_contact_step(self.h, n, C.byref(ps), _ptr(tau), _ptr(push), _ptr(ground_z), _ptr(mu), ld, int(substeps), C.byref(cp),
+                                               _ptr(contact), _ptr(diag), _ptr(status), stream, flags), "wbc_plant_contact_step")
 
     def last_timing(self):
         a, b = C.c_float(0), C.c_float(0)

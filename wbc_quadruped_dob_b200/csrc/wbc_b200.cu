@@ -22,6 +22,7 @@
 #include "qp_warp.cuh"
 #include "qp_dual.cuh"
 #include "wbc_assemble.cuh"
+#include "wbc_contact.cuh"
 #include "wbc_front.cuh"
 #include "wbc_front_leg.cuh"
 #include "wbc_traj.cuh"
@@ -867,6 +868,14 @@ __global__ void __launch_bounds__(64) wbc_fdyn_kernel(Params P, wbc::FdynIO io, 
     wbc::fdyn_step_instance(P, io, i, nsub, gamma);
 }
 
+// Contact plant (unilateral, frictional foot contacts), thread per instance (wbc_contact.cuh, contact_step_instance).
+__global__ void __launch_bounds__(64) wbc_contact_kernel(Params P, wbc::ContactParams cp, wbc::ContactIO io, int n, int nsub)
+{
+    const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    wbc::contact_step_instance(P, cp, io, i, nsub);
+}
+
 // FP64 DFMA peak: 8 independent chains per thread, fully unrolled.
 __global__ void __launch_bounds__(256) wbc_dfma_peak_kernel(double* out, int iters)
 {
@@ -983,6 +992,13 @@ void wbc_default_params(wbc_params* p)
     p->qp_epsx = 1.0e-2; p->qp_rho = 1.0e4; p->qp_outerits = 5;
     p->observer_enabled = 1; p->fix_swing_rhs = 0; p->qp_literal_kkt = 0; p->hold_tau_on_failure = 0;
     p->obs_gain2 = 1.0; p->obs_order = 1; p->obs_form = 0;
+}
+
+void wbc_default_contact_params(wbc_contact_params* cp)
+{
+    if (!cp) return;
+    memset(cp, 0, sizeof(*cp));
+    cp->beta = 0.2; cp->eps = 1.0e-8; cp->margin = 2.0e-3; cp->max_iter = 64;
 }
 
 const char* wbc_last_error(void) { return g_err; }
@@ -1648,6 +1664,71 @@ int wbc_plant_dynamics_step(wbc_ctx* c, int n, const wbc_plant_state* st, const 
         for (int f = 0; f < 7; f++)
             for (int k = 0; k < K[f]; k++, off++) memcpy(host[f] + (size_t)k * ld, c->h_pin + off * N, N * 8);
         if (diag) for (int k = 0; k < 2; k++) memcpy(diag + (size_t)k * ld, c->h_pin + (size_t)(75 + k) * N, N * 8);
+    } else if (!(flags & WBC_NO_SYNC)) {
+        CU(cudaStreamSynchronize(s));
+    }
+    return WBC_OK;
+}
+
+int wbc_plant_contact_step(wbc_ctx* c, int n, const wbc_plant_state* st, const double* tau, const double* push, const double* ground_z,
+                           const double* mu, long ld, int substeps, const wbc_contact_params* cp, int* contact, double* diag, int* status,
+                           void* cuda_stream, unsigned flags)
+{
+    if (!c || !st || !tau || !push) return fail(WBC_EINVAL, "wbc_plant_contact_step: null argument");
+    if (!st->base_pos || !st->base_rot || !st->base_rpy || !st->base_vel || !st->q || !st->dq || !st->foot_force)
+        return fail(WBC_EINVAL, "wbc_plant_contact_step: a state array is NULL");
+    if (n < 0 || n > c->max_batch || ld < n) return fail(WBC_EINVAL, "wbc_plant_contact_step: n outside [0, max_batch] or ld < n");
+    if (substeps < 1 || substeps > 1000) return fail(WBC_EINVAL, "wbc_plant_contact_step: substeps outside [1, 1000]");
+    wbc_contact_params cpv;
+    wbc_default_contact_params(&cpv);
+    if (cp) cpv = *cp;
+    if (!(cpv.beta >= 0.0 && cpv.beta <= 1.0) || !(cpv.eps >= 0.0 && cpv.eps < 1.0) || !(cpv.margin >= 0.0 && cpv.margin < 1.0e300) ||
+        cpv.max_iter < 1)
+        return fail(WBC_EINVAL, "wbc_plant_contact_step: contact params outside beta in [0, 1], eps in [0, 1), finite margin >= 0, max_iter >= 1");
+    if (n == 0) { c->launches = 0; return WBC_OK; }
+    CU(cudaSetDevice(c->device));
+    cudaStream_t s = cuda_stream ? (cudaStream_t)cuda_stream : c->stream;
+    const bool dev_ptrs = (flags & WBC_DEVICE_PTRS) != 0;
+    const wbc::ContactParams kp = {cpv.beta, cpv.eps, cpv.margin, cpv.max_iter};
+    wbc::ContactIO io;
+    static const int K[7] = {3, 9, 3, 6, 12, 12, 12};
+    double* host[7] = {st->base_pos, st->base_rot, st->base_rpy, st->base_vel, st->q, st->dq, st->foot_force};
+    const size_t N = (size_t)n;
+    if (dev_ptrs) {
+        io.base_pos = st->base_pos; io.base_rot = st->base_rot; io.base_rpy = st->base_rpy; io.base_vel = st->base_vel; io.q = st->q; io.dq = st->dq;
+        io.foot_force = st->foot_force; io.tau = tau; io.push = push; io.ground_z = ground_z; io.mu = mu;
+        io.contact = contact; io.diag = diag; io.status = status; io.ld = ld;
+    } else {
+        // packed staging in the ctx's input buffer: state 57 rows | tau 12 | push 6 | ground_z 4 | mu 1 | diag 4;
+        // contact 4 and status 1 in the integer output buffer
+        double* h = c->h_pin;
+        size_t off = 0;
+        for (int f = 0; f < 7; f++)
+            for (int k = 0; k < K[f]; k++, off++) memcpy(h + off * N, host[f] + (size_t)k * ld, N * 8);
+        for (int k = 0; k < 12; k++, off++) memcpy(h + off * N, tau + (size_t)k * ld, N * 8);
+        for (int k = 0; k < 6; k++, off++) memcpy(h + off * N, push + (size_t)k * ld, N * 8);
+        if (ground_z) for (int k = 0; k < 4; k++) memcpy(h + (off + k) * N, ground_z + (size_t)k * ld, N * 8);
+        if (mu) memcpy(h + (off + 4) * N, mu, N * 8);
+        CU(cudaMemcpyAsync(c->d_in, h, (off + 5) * N * 8, cudaMemcpyHostToDevice, s));
+        double* d = c->d_in;
+        io.base_pos = d; io.base_rot = d + 3 * N; io.base_rpy = d + 12 * N; io.base_vel = d + 15 * N; io.q = d + 21 * N; io.dq = d + 33 * N;
+        io.foot_force = d + 45 * N; io.tau = d + 57 * N; io.push = d + 69 * N;
+        io.ground_z = ground_z ? d + 75 * N : nullptr; io.mu = mu ? d + 79 * N : nullptr; io.diag = diag ? d + 80 * N : nullptr;
+        io.contact = contact ? c->d_iout : nullptr; io.status = status ? c->d_iout + 4 * N : nullptr; io.ld = n;
+    }
+    wbc_contact_kernel<<<(n + 63) / 64, 64, 0, s>>>(c->params, kp, io, n, substeps);
+    CU(cudaGetLastError());
+    c->launches = 1;
+    if (!dev_ptrs) {
+        CU(cudaMemcpyAsync(c->h_pin, c->d_in, (size_t)84 * N * 8, cudaMemcpyDeviceToHost, s));
+        if (contact || status) CU(cudaMemcpyAsync(c->h_pin_i, c->d_iout, 5 * N * sizeof(int), cudaMemcpyDeviceToHost, s));
+        CU(cudaStreamSynchronize(s));
+        size_t off = 0;
+        for (int f = 0; f < 7; f++)
+            for (int k = 0; k < K[f]; k++, off++) memcpy(host[f] + (size_t)k * ld, c->h_pin + off * N, N * 8);
+        if (diag) for (int k = 0; k < 4; k++) memcpy(diag + (size_t)k * ld, c->h_pin + (size_t)(80 + k) * N, N * 8);
+        if (contact) for (int k = 0; k < 4; k++) memcpy(contact + (size_t)k * ld, c->h_pin_i + (size_t)k * N, N * sizeof(int));
+        if (status) memcpy(status, c->h_pin_i + 4 * N, N * sizeof(int));
     } else if (!(flags & WBC_NO_SYNC)) {
         CU(cudaStreamSynchronize(s));
     }
