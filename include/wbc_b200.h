@@ -44,6 +44,7 @@ extern "C" {
 #define WBC_ST_NONFINITE (-21)   /* a NaN or infinity among the inputs, or produced from them before the QP */
 #define WBC_ST_INFEASIBLE (-22)  /* exact mode (WBC_QP_EXACT): the constraints admit no point (row-scaled residuals) */
 #define WBC_ST_NOT_PD (-23)      /* exact mode: H (the lower triangle of Q mirrored) is not positive definite */
+#define WBC_ST_BAD_TERRAIN (-24) /* wbc_plant_contact_step_terrain: a foot frame not orthonormal to 1e-9, or mu < 0 */
 
 /* contact modes: which feet swing */
 #define WBC_MODE_STANCE 0        /* main.cpp:979-1148, 1516-1675 */
@@ -290,6 +291,19 @@ void wbc_default_contact_params(wbc_contact_params* cp);
 int wbc_plant_contact_step(wbc_ctx* ctx, int n, const wbc_plant_state* st, const double* tau, const double* push, const double* ground_z,
                            const double* mu, long ld, int substeps, const wbc_contact_params* cp, int* contact, double* diag, int* status,
                            void* cuda_stream, unsigned flags);
+/* Contact plant on inclined ground: wbc_plant_contact_step with each foot's plane, contact frame and friction coefficient taken
+ * from the controller's terrain layout (wbc_inputs.terrain), so that the plant's ground is the ground the controller is told about.
+ * terrain [40][ld] (required; flat ground is wbc_plant_contact_step): for stacked foot k, rows 10k..10k+2 the unit normal n,
+ * +3..+5 the tangent t1, +6..+8 the tangent t2, +9 mu.  plane_d [4][ld] (NULL = 0): foot k's plane is {p : n . p = d_k}.  Per step
+ * the gap is measured along the normal, phi_k = n . p_k - d_k (candidates, speculative and Baumgarte targets, diag[0]); each
+ * candidate foot's impulse is expressed in its frame, lambda = (lambda_t1, lambda_t2, lambda_n) with Jacobian rows F' J, F = [t1 t2 n],
+ * over the pyramid |lambda_t1|, |lambda_t2| <= mu lambda_n, lambda_n >= 0 -- the controller's cone rows.  foot_force gets
+ * R_foot' F lambda / dt; contact flags, diag (diag[1]: smallest lambda_n / dt) and status as in wbc_plant_contact_step.  An
+ * instance whose frame is not orthonormal to 1e-9 or whose mu < 0 is refused with WBC_ST_BAD_TERRAIN, one with a non-finite terrain
+ * or plane_d entry with WBC_ST_NONFINITE; its state is untouched and its flags are 0.  A foot keeps its plane for the whole call. */
+int wbc_plant_contact_step_terrain(wbc_ctx* ctx, int n, const wbc_plant_state* st, const double* tau, const double* push,
+                                   const double* terrain, const double* plane_d, long ld, int substeps, const wbc_contact_params* cp,
+                                   int* contact, double* diag, int* status, void* cuda_stream, unsigned flags);
 
 /* Device-side timing of the last wbc_cycle on this ctx (CUDA events on the launching stream), ms. */
 int wbc_last_timing(wbc_ctx* ctx, float* front_ms, float* solve_ms);

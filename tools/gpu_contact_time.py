@@ -1,8 +1,10 @@
-"""Time per control period of the contact plant (wbc_plant_contact_step, five substeps) beside the bilateral forward-dynamics plant
-(wbc_plant_dynamics_step) on the same states, device pointers, CUDA events around 20 calls after 3 warm-up calls.  The states are a
-stance / swing mix whose feet stand on, above and up to 3 mm below per-foot ground planes, under random torques and pushes (the
-mixed states of tests/test_contact_plant.py), so that every kind of contact solve occurs.  Each timed call starts from the same
-state.  Prints the GPU's name and power limit with the numbers."""
+"""Time per control period of the contact plant (wbc_plant_contact_step, five substeps), of its terrain form
+(wbc_plant_contact_step_terrain) and of the bilateral forward-dynamics plant (wbc_plant_dynamics_step) on the same states, device
+pointers, CUDA events around 20 calls of each after 3 warm-up calls, the three plants called in turn.  The states are a stance /
+swing mix whose feet stand on, above and up to 3 mm below per-foot ground planes, under random torques and pushes (the mixed states
+of tests/test_contact_plant.py), so that every kind of contact solve occurs; the terrain form gets the same gaps, measured along
+per-foot normals up to 15 deg from vertical, and each foot's mu the instance's.  Each timed call starts from the same state.
+Prints the GPU's name and power limit with the numbers."""
 import subprocess
 import sys
 import time
@@ -27,7 +29,12 @@ for n in (4096, 65536):
     init["mode"] = T(sc["mode"].astype(np.int32))
     din = {k: v.clone() for k, v in init.items()}
     tau, push = T(rng.normal(0.0, 4.0, (12, n))), T(rng.normal(0.0, 15.0, (6, n)))
-    gz, mu = T(feet[:, :, 2].T - gap), T(rng.uniform(0.05, 1.0, n))
+    mu_h = rng.uniform(0.05, 1.0, n)
+    gz, mu = T(feet[:, :, 2].T - gap), T(mu_h)
+    ct = rng.uniform(np.cos(np.deg2rad(15.0)), 1.0, (4, n))
+    ph = rng.uniform(0.0, 2 * np.pi, (4, n))
+    tr_h, d_h = S.terrain_frames(np.stack([np.sqrt(1 - ct * ct) * np.cos(ph), np.sqrt(1 - ct * ct) * np.sin(ph), ct], axis=1), mu_h, feet)
+    tr, pd = T(tr_h), T(d_h - gap)
     diag = torch.zeros(4, n, dtype=torch.float64, device=dev)
     status = torch.zeros(n, dtype=torch.int32, device=dev)
     b = api.WbcBatch(max_batch=n)
@@ -35,12 +42,14 @@ for n in (4096, 65536):
     s = ts.cuda_stream
     plants = {
         "contact": lambda: b.plant_contact_step(din, tau, push, ground_z=gz, mu=mu, n=n, ld=n, substeps=5, diag=diag, status=status, stream=s, sync=False),
+        "terrain": lambda: b.plant_contact_step(din, tau, push, terrain=tr, plane_d=pd, n=n, ld=n, substeps=5, diag=diag, status=status, stream=s,
+                                                sync=False),
         "bilateral": lambda: b.plant_dynamics_step(din, tau, push, n=n, ld=n, substeps=5, gamma=100.0, stream=s, sync=False),
     }
     torch.cuda.synchronize()
-    for name, call in plants.items():
-        ms, wall = [], []
-        for it in range(23):
+    ms, wall, extra = {k: [] for k in plants}, {k: [] for k in plants}, {}
+    for it in range(23):
+        for name, call in plants.items():
             with torch.cuda.stream(ts):
                 for k in init:
                     din[k].copy_(init[k])
@@ -50,13 +59,14 @@ for n in (4096, 65536):
                 e0.record(ts); call(); e1.record(ts)
             torch.cuda.synchronize()
             if it >= 3:
-                ms.append(e0.elapsed_time(e1))
-                wall.append(1e3 * (time.perf_counter() - t0))
-        extra = ""
-        if name == "contact":
-            dg, st = diag.cpu().numpy(), status.cpu().numpy()
-            extra = ", failed %d, dual steps per robot-period %.2f (max %d), max KKT residual %.1e" % (
-                int((st != 0).sum()), dg[3].mean(), int(dg[3].max()), dg[2].max())
+                ms[name].append(e0.elapsed_time(e1))
+                wall[name].append(1e3 * (time.perf_counter() - t0))
+            if name != "bilateral" and it == 22:
+                dg, st = diag.cpu().numpy(), status.cpu().numpy()
+                extra[name] = ", failed %d, dual steps per robot-period %.2f (max %d), max KKT residual %.1e" % (
+                    int((st != 0).sum()), dg[3].mean(), int(dg[3].max()), dg[2].max())
+    for name in plants:
         print("n %6d %-9s plant, 5 substeps: median %.3f ms per control period (min %.3f, max %.3f; host clock to the synchronise %.3f ms)%s"
-              % (n, name, np.median(ms), min(ms), max(ms), np.median(wall), extra))
+              % (n, name, np.median(ms[name]), min(ms[name]), max(ms[name]), np.median(wall[name]), extra.get(name, "")))
+    print("n %6d terrain / flat contact plant: %.3f (median of the per-call ratios)" % (n, np.median(np.array(ms["terrain"]) / np.array(ms["contact"]))))
     b.close()

@@ -92,7 +92,7 @@ _lib = None
 EXPORTS = ["wbc_default_params", "wbc_last_error", "wbc_version", "wbc_create", "wbc_destroy", "wbc_set_params",
            "wbc_set_observer_state", "wbc_get_observer_state", "wbc_set_observer_state2", "wbc_get_observer_state2", "wbc_cycle", "wbc_debug_update", "wbc_debug_qp_records", "wbc_qp_solve",
            "wbc_qp_solve_warm", "wbc_set_active_set", "wbc_get_active_set",
-           "wbc_plant_step", "wbc_plant_dynamics_step", "wbc_default_contact_params", "wbc_plant_contact_step", "wbc_last_timing", "wbc_last_solve_cycles", "wbc_last_launches", "wbc_solver_shape", "wbc_stage_profile", "wbc_host_alloc",
+           "wbc_plant_step", "wbc_plant_dynamics_step", "wbc_default_contact_params", "wbc_plant_contact_step", "wbc_plant_contact_step_terrain", "wbc_last_timing", "wbc_last_solve_cycles", "wbc_last_launches", "wbc_solver_shape", "wbc_stage_profile", "wbc_host_alloc",
            "wbc_host_free",
            "wbc_set_trajectory", "wbc_sample_trajectory",
            "wbc_measure_dfma_peak"]
@@ -140,6 +140,7 @@ def load():
     lib.wbc_default_contact_params.argtypes = [C.POINTER(ContactParams)]
     lib.wbc_plant_contact_step.argtypes = [C.c_void_p, C.c_int, C.POINTER(_PlantState), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_long,
                                            C.c_int, C.POINTER(ContactParams), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint]
+    lib.wbc_plant_contact_step_terrain.argtypes = lib.wbc_plant_contact_step.argtypes
     lib.wbc_last_timing.argtypes = [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_float)]
     lib.wbc_last_solve_cycles.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_ulonglong)]
     lib.wbc_last_launches.argtypes = [C.c_void_p]
@@ -479,11 +480,17 @@ class WbcBatch:
                "wbc_plant_dynamics_step")
 
     def plant_contact_step(self, state, tau, push, ground_z=None, mu=None, n=None, ld=None, substeps=5, params=None, contact=None, diag=None,
-                           status=None, stream=None, sync=True):
+                           status=None, stream=None, sync=True, terrain=None, plane_d=None):
         """Contact plant (wbc_plant_contact_step): unilateral, frictional foot contacts on per-foot ground planes.  `state` is a dict
         with base_pos, base_rot, base_rpy, base_vel, q, dq, foot_force (numpy arrays: host path, advanced in place; torch CUDA tensors:
         device path); its mode is not read.  ground_z [4, ld] (None: 0), mu [ld] (None: params.mu), params a ContactParams (None:
-        the defaults); contact int32 [4, ld], diag [4, ld] and status int32 [ld] are filled when given."""
+        the defaults); contact int32 [4, ld], diag [4, ld] and status int32 [ld] are filled when given.
+        With terrain [40, ld] (the controller's per-foot frames n, t1, t2 and mu, as in `cycle`) and plane_d [4, ld] (None: 0), each
+        foot stands on the plane n . p = d_k instead (wbc_plant_contact_step_terrain); ground_z and mu must then be None."""
+        if terrain is None and plane_d is not None:
+            raise ValueError("plant_contact_step: plane_d needs terrain")
+        if terrain is not None and (ground_z is not None or mu is not None):
+            raise ValueError("plant_contact_step: terrain replaces ground_z and mu; pass plane_d for the plane offsets")
         host = isinstance(state["q"], np.ndarray)
         n = int(state["q"].shape[1]) if n is None else int(n)
         ld = n if ld is None else int(ld)
@@ -500,9 +507,16 @@ class WbcBatch:
             tau, push = np.ascontiguousarray(tau, dtype=np.float64), np.ascontiguousarray(push, dtype=np.float64)
             ground_z = None if ground_z is None else np.ascontiguousarray(ground_z, dtype=np.float64)
             mu = None if mu is None else np.ascontiguousarray(mu, dtype=np.float64)
-            keep += [tau, push, ground_z, mu]
+            terrain = None if terrain is None else np.ascontiguousarray(terrain, dtype=np.float64)
+            plane_d = None if plane_d is None else np.ascontiguousarray(plane_d, dtype=np.float64)
+            keep += [tau, push, ground_z, mu, terrain, plane_d]
         cp = params if params is not None else default_contact_params()
         flags = (HOST_PTRS if host else DEVICE_PTRS) | (0 if (sync or host) else NO_SYNC)
+        if terrain is not None:
+            _check(self.lib.wbc_plant_contact_step_terrain(self.h, n, C.byref(ps), _ptr(tau), _ptr(push), _ptr(terrain), _ptr(plane_d), ld,
+                                                           int(substeps), C.byref(cp), _ptr(contact), _ptr(diag), _ptr(status), stream, flags),
+                   "wbc_plant_contact_step_terrain")
+            return
         _check(self.lib.wbc_plant_contact_step(self.h, n, C.byref(ps), _ptr(tau), _ptr(push), _ptr(ground_z), _ptr(mu), ld, int(substeps), C.byref(cp),
                                                _ptr(contact), _ptr(diag), _ptr(status), stream, flags), "wbc_plant_contact_step")
 

@@ -876,6 +876,15 @@ __global__ void __launch_bounds__(64) wbc_contact_kernel(Params P, wbc::ContactP
     wbc::contact_step_instance(P, cp, io, i, nsub);
 }
 
+// Contact plant on per-foot planes and contact frames (the terrain form of contact_step_instance); io.ground_z holds the plane offsets.
+__global__ void __launch_bounds__(64) wbc_contact_terrain_kernel(Params P, wbc::ContactParams cp, wbc::ContactIO io, int n, int nsub,
+                                                                 const double* terrain)
+{
+    const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    wbc::contact_step_instance<true>(P, cp, io, i, nsub, terrain);
+}
+
 // FP64 DFMA peak: 8 independent chains per thread, fully unrolled.
 __global__ void __launch_bounds__(256) wbc_dfma_peak_kernel(double* out, int iters)
 {
@@ -1670,27 +1679,30 @@ int wbc_plant_dynamics_step(wbc_ctx* c, int n, const wbc_plant_state* st, const 
     return WBC_OK;
 }
 
-int wbc_plant_contact_step(wbc_ctx* c, int n, const wbc_plant_state* st, const double* tau, const double* push, const double* ground_z,
-                           const double* mu, long ld, int substeps, const wbc_contact_params* cp, int* contact, double* diag, int* status,
-                           void* cuda_stream, unsigned flags)
+// The host side of both contact-plant entry points; terrain == nullptr runs the flat kernel (ground_z, mu), otherwise the terrain
+// kernel (ground_z then holds the plane offsets, mu is NULL).
+static int contact_step(const char* fn, wbc_ctx* c, int n, const wbc_plant_state* st, const double* tau, const double* push,
+                        const double* ground_z, const double* mu, const double* terrain, long ld, int substeps, const wbc_contact_params* cp,
+                        int* contact, double* diag, int* status, void* cuda_stream, unsigned flags)
 {
-    if (!c || !st || !tau || !push) return fail(WBC_EINVAL, "wbc_plant_contact_step: null argument");
+    if (!c || !st || !tau || !push) return fail(WBC_EINVAL, "%s: null argument", fn);
     if (!st->base_pos || !st->base_rot || !st->base_rpy || !st->base_vel || !st->q || !st->dq || !st->foot_force)
-        return fail(WBC_EINVAL, "wbc_plant_contact_step: a state array is NULL");
-    if (n < 0 || n > c->max_batch || ld < n) return fail(WBC_EINVAL, "wbc_plant_contact_step: n outside [0, max_batch] or ld < n");
-    if (substeps < 1 || substeps > 1000) return fail(WBC_EINVAL, "wbc_plant_contact_step: substeps outside [1, 1000]");
+        return fail(WBC_EINVAL, "%s: a state array is NULL", fn);
+    if (n < 0 || n > c->max_batch || ld < n) return fail(WBC_EINVAL, "%s: n outside [0, max_batch] or ld < n", fn);
+    if (substeps < 1 || substeps > 1000) return fail(WBC_EINVAL, "%s: substeps outside [1, 1000]", fn);
     wbc_contact_params cpv;
     wbc_default_contact_params(&cpv);
     if (cp) cpv = *cp;
     if (!(cpv.beta >= 0.0 && cpv.beta <= 1.0) || !(cpv.eps >= 0.0 && cpv.eps < 1.0) || !(cpv.margin >= 0.0 && cpv.margin < 1.0e300) ||
         cpv.max_iter < 1)
-        return fail(WBC_EINVAL, "wbc_plant_contact_step: contact params outside beta in [0, 1], eps in [0, 1), finite margin >= 0, max_iter >= 1");
+        return fail(WBC_EINVAL, "%s: contact params outside beta in [0, 1], eps in [0, 1), finite margin >= 0, max_iter >= 1", fn);
     if (n == 0) { c->launches = 0; return WBC_OK; }
     CU(cudaSetDevice(c->device));
     cudaStream_t s = cuda_stream ? (cudaStream_t)cuda_stream : c->stream;
     const bool dev_ptrs = (flags & WBC_DEVICE_PTRS) != 0;
     const wbc::ContactParams kp = {cpv.beta, cpv.eps, cpv.margin, cpv.max_iter};
     wbc::ContactIO io;
+    const double* dterrain = terrain;
     static const int K[7] = {3, 9, 3, 6, 12, 12, 12};
     double* host[7] = {st->base_pos, st->base_rot, st->base_rpy, st->base_vel, st->q, st->dq, st->foot_force};
     const size_t N = (size_t)n;
@@ -1699,7 +1711,7 @@ int wbc_plant_contact_step(wbc_ctx* c, int n, const wbc_plant_state* st, const d
         io.foot_force = st->foot_force; io.tau = tau; io.push = push; io.ground_z = ground_z; io.mu = mu;
         io.contact = contact; io.diag = diag; io.status = status; io.ld = ld;
     } else {
-        // packed staging in the ctx's input buffer: state 57 rows | tau 12 | push 6 | ground_z 4 | mu 1 | diag 4;
+        // packed staging in the ctx's input buffer: state 57 rows | tau 12 | push 6 | ground_z 4 | mu 1 | diag 4 | terrain 40;
         // contact 4 and status 1 in the integer output buffer
         double* h = c->h_pin;
         size_t off = 0;
@@ -1711,12 +1723,20 @@ int wbc_plant_contact_step(wbc_ctx* c, int n, const wbc_plant_state* st, const d
         if (mu) memcpy(h + (off + 4) * N, mu, N * 8);
         CU(cudaMemcpyAsync(c->d_in, h, (off + 5) * N * 8, cudaMemcpyHostToDevice, s));
         double* d = c->d_in;
+        if (terrain) {
+            for (int k = 0; k < 40; k++) memcpy(h + (84 + k) * N, terrain + (size_t)k * ld, N * 8);
+            CU(cudaMemcpyAsync(d + 84 * N, h + 84 * N, 40 * N * 8, cudaMemcpyHostToDevice, s));
+            dterrain = d + 84 * N;
+        }
         io.base_pos = d; io.base_rot = d + 3 * N; io.base_rpy = d + 12 * N; io.base_vel = d + 15 * N; io.q = d + 21 * N; io.dq = d + 33 * N;
         io.foot_force = d + 45 * N; io.tau = d + 57 * N; io.push = d + 69 * N;
         io.ground_z = ground_z ? d + 75 * N : nullptr; io.mu = mu ? d + 79 * N : nullptr; io.diag = diag ? d + 80 * N : nullptr;
         io.contact = contact ? c->d_iout : nullptr; io.status = status ? c->d_iout + 4 * N : nullptr; io.ld = n;
     }
-    wbc_contact_kernel<<<(n + 63) / 64, 64, 0, s>>>(c->params, kp, io, n, substeps);
+    if (terrain)
+        wbc_contact_terrain_kernel<<<(n + 63) / 64, 64, 0, s>>>(c->params, kp, io, n, substeps, dterrain);
+    else
+        wbc_contact_kernel<<<(n + 63) / 64, 64, 0, s>>>(c->params, kp, io, n, substeps);
     CU(cudaGetLastError());
     c->launches = 1;
     if (!dev_ptrs) {
@@ -1733,6 +1753,23 @@ int wbc_plant_contact_step(wbc_ctx* c, int n, const wbc_plant_state* st, const d
         CU(cudaStreamSynchronize(s));
     }
     return WBC_OK;
+}
+
+int wbc_plant_contact_step(wbc_ctx* c, int n, const wbc_plant_state* st, const double* tau, const double* push, const double* ground_z,
+                           const double* mu, long ld, int substeps, const wbc_contact_params* cp, int* contact, double* diag, int* status,
+                           void* cuda_stream, unsigned flags)
+{
+    return contact_step("wbc_plant_contact_step", c, n, st, tau, push, ground_z, mu, nullptr, ld, substeps, cp, contact, diag, status,
+                        cuda_stream, flags);
+}
+
+int wbc_plant_contact_step_terrain(wbc_ctx* c, int n, const wbc_plant_state* st, const double* tau, const double* push, const double* terrain,
+                                   const double* plane_d, long ld, int substeps, const wbc_contact_params* cp, int* contact, double* diag,
+                                   int* status, void* cuda_stream, unsigned flags)
+{
+    if (!terrain) return fail(WBC_EINVAL, "wbc_plant_contact_step_terrain: terrain is NULL (flat ground is wbc_plant_contact_step)");
+    return contact_step("wbc_plant_contact_step_terrain", c, n, st, tau, push, plane_d, nullptr, terrain, ld, substeps, cp, contact, diag,
+                        status, cuda_stream, flags);
 }
 
 int wbc_last_timing(wbc_ctx* c, float* front_ms, float* solve_ms)

@@ -17,6 +17,12 @@
 //
 // The M^-1 block elimination is a copy of fdyn_step_instance's rather than a function shared with it, so that the bilateral
 // plant's code (and its results) stay exactly as they are.
+//
+// Terrain form (TERRAIN = true, wbc_plant_contact_step_terrain): foot k has the plane {p : n_k . p = d_k} and its own frame
+// F_k = [t1 t2 n] and mu_k, in the controller's terrain layout [40][ld] (rows 10k..10k+2 n, +3..+5 t1, +6..+8 t2, +9 mu); d_k is
+// read where the flat form reads ground_z.  The gap is measured along n_k, each candidate foot's three Jacobian rows are rotated
+// into its frame (J_local = F_k' J_world), so lambda = (lambda_t1, lambda_t2, lambda_n) and the same pyramid rows describe the
+// controller's cone rows; the forces leave as R_foot' F_k lambda / dt.  With F_k = I the arithmetic is the flat form's.
 #pragma once
 #include <math.h>
 
@@ -32,7 +38,7 @@ struct ContactParams {     // wbc_contact_params
 struct ContactIO {
     double *base_pos, *base_rot, *base_rpy, *base_vel, *q, *dq, *foot_force;   // state, SoA [k][ld], advanced in place on success
     const double *tau, *push;        // [12][ld], [6][ld]
-    const double *ground_z, *mu;     // [4][ld] or nullptr (0), [ld] or nullptr (Params::mu)
+    const double *ground_z, *mu;     // [4][ld] or nullptr (0), [ld] or nullptr (Params::mu); terrain form: plane offsets d, mu unused
     int* contact;                    // [4][ld] or nullptr: 0 no contact force, 1 sticking, 2 sliding (last step)
     double* diag;                    // [4][ld] or nullptr: max penetration, min normal force, max KKT residual, active-set iterations
     int* status;                     // [ld] or nullptr
@@ -40,6 +46,7 @@ struct ContactIO {
 };
 
 constexpr int CONTACT_ST_NONFINITE = -21;   // WBC_ST_NONFINITE
+constexpr int CONTACT_ST_BAD_TERRAIN = -24; // WBC_ST_BAD_TERRAIN
 constexpr int CONTACT_ST_MAX_ITER = -100;
 
 // Row t of a foot's friction pyramid in "n . lambda_foot >= 0" form, unit length: 0 normal, 1/2 -+x, 3/4 -+y.
@@ -264,7 +271,10 @@ WBC_HD ContactQpResult contact_qp(double* H, const double* g, int nf, const doub
     return res;
 }
 
-WBC_DEVFN inline void contact_step_instance(const Params& P, const ContactParams& cp, const ContactIO& io, long i, int nsub)
+// TERRAIN: the terrain form (see the top of this file); `terrain` [40][ld] is then required and io.ground_z holds the plane offsets.
+template <bool TERRAIN = false>
+WBC_DEVFN inline void contact_step_instance(const Params& P, const ContactParams& cp, const ContactIO& io, long i, int nsub,
+                                            const double* terrain = nullptr)
 {
     using namespace dogbot;
     const long ld = io.ld;
@@ -279,6 +289,18 @@ WBC_DEVFN inline void contact_step_instance(const Params& P, const ContactParams
     for (int k = 0; k < 12; k++) { tau[k] = io.tau[(long)k * ld + i]; finite = finite && (tau[k] - tau[k] == 0.0); }
     for (int k = 0; k < 6; k++) { push[k] = io.push[(long)k * ld + i]; finite = finite && (push[k] - push[k] == 0.0); }
     for (int k = 0; k < 4; k++) { gz[k] = io.ground_z ? io.ground_z[(long)k * ld + i] : 0.0; finite = finite && (gz[k] - gz[k] == 0.0); }
+    bool frames_ok = true;            // terrain form: every foot's frame orthonormal to 1e-9 and mu >= 0
+    if (TERRAIN)
+        for (int sf = 0; sf < 4; sf++) {
+            double fr[10];
+            for (int k = 0; k < 10; k++) { fr[k] = terrain[(long)(10 * sf + k) * ld + i]; finite = finite && (fr[k] - fr[k] == 0.0); }
+            for (int a = 0; a < 3; a++)
+                for (int c = a; c < 3; c++) {
+                    const double e = fr[3 * a] * fr[3 * c] + fr[3 * a + 1] * fr[3 * c + 1] + fr[3 * a + 2] * fr[3 * c + 2];
+                    frames_ok = frames_ok && fabs(e - (a == c ? 1.0 : 0.0)) <= 1e-9;
+                }
+            frames_ok = frames_ok && fr[9] >= 0.0;
+        }
     DevInputs in;
     in.base_pos = s; in.base_rot = s + 3; in.base_rpy = s + 12; in.base_vel = s + 15; in.q = s + 21; in.dq = s + 33;
     in.com_des_pos = in.com_des_vel = in.com_des_acc = in.sw_des_pos = in.sw_des_vel = in.sw_des_acc = nullptr;
@@ -288,6 +310,7 @@ WBC_DEVFN inline void contact_step_instance(const Params& P, const ContactParams
     double fs_out[12];
     int flag_out[4] = {0, 0, 0, 0};
     int status = finite ? 0 : CONTACT_ST_NONFINITE;
+    if (TERRAIN && status == 0 && !frames_ok) status = CONTACT_ST_BAD_TERRAIN;
     unsigned warm = 0u;               // active rows of the previous step, row id 5 * stacked foot + pyramid row
     for (int k = 0; k < 12; k++) fs_out[k] = 0.0;
     for (int it = 0; it < nsub && status == 0; it++) {
@@ -365,22 +388,46 @@ WBC_DEVFN inline void contact_step_instance(const Params& P, const ContactParams
         for (int sf = 0; sf < 4; sf++) {
             const int leg = kFootLeg[sf];
             const V3 rf = D.footp[leg];
-            phi[sf] = s[2] + rf.z - gz[sf];
+            double fr[10];            // terrain form: this foot's n, t1, t2, mu
+            if (TERRAIN) {
+                for (int k = 0; k < 10; k++) fr[k] = terrain[(long)(10 * sf + k) * ld + i];
+                phi[sf] = fr[0] * (s[0] + rf.x) + fr[1] * (s[1] + rf.y) + fr[2] * (s[2] + rf.z) - gz[sf];
+            } else {
+                phi[sf] = s[2] + rf.z - gz[sf];
+            }
             pen = fmax(pen, -phi[sf]);
             if (phi[sf] > cp.margin) continue;
             const double nSf[9] = {0, rf.z, -rf.y, -rf.z, 0, rf.x, rf.y, -rf.x, 0};
-            for (int a = 0; a < 3; a++) {
-                const int r = 3 * nf + a;
-                rleg[r] = leg;
-                for (int k = 0; k < 3; k++) { Jb[r * 6 + k] = (k == a) ? 1.0 : 0.0; Jb[r * 6 + 3 + k] = nSf[a * 3 + k]; Jl[r * 3 + k] = D.Jleg[leg][a * 3 + k]; }
-                double jn = 0.0;
-                for (int k = 0; k < 6; k++) jn += Jb[r * 6 + k] * nu[k];
-                for (int k = 0; k < 3; k++) jn += Jl[r * 3 + k] * nu[6 + dof_index(leg, k)];
-                g[r] = jn;
+            if (TERRAIN) {
+                // the world rows x, y, z, then local row c = (t1, t2, n)[c]' J_world
+                double wb[18], wl[9];
+                for (int a = 0; a < 3; a++)
+                    for (int k = 0; k < 3; k++) { wb[a * 6 + k] = (k == a) ? 1.0 : 0.0; wb[a * 6 + 3 + k] = nSf[a * 3 + k]; wl[a * 3 + k] = D.Jleg[leg][a * 3 + k]; }
+                for (int c = 0; c < 3; c++) {
+                    const double* e = fr + (c == 2 ? 0 : 3 + 3 * c);
+                    const int r = 3 * nf + c;
+                    rleg[r] = leg;
+                    for (int k = 0; k < 6; k++) Jb[r * 6 + k] = e[0] * wb[k] + e[1] * wb[6 + k] + e[2] * wb[12 + k];
+                    for (int k = 0; k < 3; k++) Jl[r * 3 + k] = e[0] * wl[k] + e[1] * wl[3 + k] + e[2] * wl[6 + k];
+                    double jn = 0.0;
+                    for (int k = 0; k < 6; k++) jn += Jb[r * 6 + k] * nu[k];
+                    for (int k = 0; k < 3; k++) jn += Jl[r * 3 + k] * nu[6 + dof_index(leg, k)];
+                    g[r] = jn;
+                }
+            } else {
+                for (int a = 0; a < 3; a++) {
+                    const int r = 3 * nf + a;
+                    rleg[r] = leg;
+                    for (int k = 0; k < 3; k++) { Jb[r * 6 + k] = (k == a) ? 1.0 : 0.0; Jb[r * 6 + 3 + k] = nSf[a * 3 + k]; Jl[r * 3 + k] = D.Jleg[leg][a * 3 + k]; }
+                    double jn = 0.0;
+                    for (int k = 0; k < 6; k++) jn += Jb[r * 6 + k] * nu[k];
+                    for (int k = 0; k < 3; k++) jn += Jl[r * 3 + k] * nu[6 + dof_index(leg, k)];
+                    g[r] = jn;
+                }
             }
             g[3 * nf + 2] += (phi[sf] >= 0.0 ? 1.0 : cp.beta) * phi[sf] / dt;
             wsub |= ((warm >> (5 * sf)) & 31u) << (5 * nf);
-            mu_f[nf] = mu;
+            mu_f[nf] = TERRAIN ? fr[9] : mu;
             cand[nf++] = sf;
         }
         const int nc = 3 * nf;
@@ -416,13 +463,21 @@ WBC_DEVFN inline void contact_step_instance(const Params& P, const ContactParams
                 warm |= rows << (5 * sf);
                 // an active normal row, or an active pair of opposite friction rows (mu > 0), means lambda_z = 0 and with it the
                 // whole pyramid: the foot carries exactly nothing (rather than a rounding residue)
-                const bool zero = (rows & 1u) || (mu > 0.0 && ((rows & 6u) == 6u || (rows & 24u) == 24u)) || lam[3 * f + 2] <= 0.0;
+                const bool zero = (rows & 1u) || ((TERRAIN ? mu_f[f] : mu) > 0.0 && ((rows & 6u) == 6u || (rows & 24u) == 24u)) || lam[3 * f + 2] <= 0.0;
                 if (zero) { lam[3 * f] = lam[3 * f + 1] = lam[3 * f + 2] = 0.0; }
                 flag_out[sf] = lam[3 * f + 2] > 0.0 ? ((rows & 30u) ? 2 : 1) : 0;
                 fzmin = fmin(fzmin, lam[3 * f + 2] / dt);
                 const M3& Rf = D.footR[kFootLeg[sf]];
-                for (int k = 0; k < 3; k++)
-                    fs_out[3 * sf + k] = (Rf.m[k] * lam[3 * f] + Rf.m[3 + k] * lam[3 * f + 1] + Rf.m[6 + k] * lam[3 * f + 2]) / dt;
+                if (TERRAIN) {
+                    double lw[3];             // world impulse F lambda = t1 lambda_t1 + t2 lambda_t2 + n lambda_n
+                    for (int a = 0; a < 3; a++)
+                        lw[a] = terrain[(long)(10 * sf + 3 + a) * ld + i] * lam[3 * f] + terrain[(long)(10 * sf + 6 + a) * ld + i] * lam[3 * f + 1] +
+                                terrain[(long)(10 * sf + a) * ld + i] * lam[3 * f + 2];
+                    for (int k = 0; k < 3; k++) fs_out[3 * sf + k] = (Rf.m[k] * lw[0] + Rf.m[3 + k] * lw[1] + Rf.m[6 + k] * lw[2]) / dt;
+                } else {
+                    for (int k = 0; k < 3; k++)
+                        fs_out[3 * sf + k] = (Rf.m[k] * lam[3 * f] + Rf.m[3 + k] * lam[3 * f + 1] + Rf.m[6 + k] * lam[3 * f + 2]) / dt;
+                }
             }
             // nu+ = nu_free + X lambda
             for (int rr = 0; rr < nc; rr++) {

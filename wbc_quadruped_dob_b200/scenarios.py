@@ -183,6 +183,45 @@ def make(n, mode_mix=(1.0, 0.0, 0.0), pushes=False, terrain=False, seed=1, start
     return {k: np.ascontiguousarray(np.concatenate([p[k] for p in parts], axis=-1)) for k in parts[0]}
 
 
+def terrain_frames(normals, mu, feet=None):
+    """Per-foot contact planes in the controller's terrain layout, so that one description feeds both the controller
+    (`terrain` of a cycle) and the contact plant (WbcBatch.plant_contact_step(terrain=..., plane_d=...)).
+
+    normals [4, 3, n] (or [3, n], the same for every foot; normalised here); mu a scalar, [n] or [4, n].  t1 is the world x axis
+    projected onto the plane (the y axis where the normal is within 26 deg of x), t2 = n x t1.  feet [n, 4, 3]
+    (forward_kinematics) puts each foot's plane through that foot point; None puts every plane through the origin.
+    Returns (terrain [40, n], plane_d [4, n])."""
+    nrm = np.asarray(normals, dtype=np.float64)
+    if nrm.ndim == 2:
+        nrm = np.broadcast_to(nrm, (4,) + nrm.shape)
+    n = nrm.shape[2]
+    mu = np.broadcast_to(np.asarray(mu, dtype=np.float64), (4, n))
+    terrain, plane_d = np.zeros((40, n)), np.zeros((4, n))
+    for f in range(4):
+        nf = nrm[f] / np.linalg.norm(nrm[f], axis=0)
+        near_x = np.abs(nf[0]) > 0.9
+        axis = np.where(near_x, np.array([0.0, 1.0, 0.0])[:, None], np.array([1.0, 0.0, 0.0])[:, None])
+        t1 = axis - nf * np.sum(axis * nf, axis=0)
+        t1 /= np.linalg.norm(t1, axis=0)
+        t2 = np.cross(nf.T, t1.T).T
+        terrain[10 * f:10 * f + 3], terrain[10 * f + 3:10 * f + 6], terrain[10 * f + 6:10 * f + 9] = nf, t1, t2
+        terrain[10 * f + 9] = mu[f]
+        if feet is not None:
+            plane_d[f] = np.sum(nf * feet[:, f, :].T, axis=0)
+    return terrain, plane_d
+
+
+def slope_terrain(feet, slope, azimuth, mu):
+    """One slope per robot: the normal tilted by `slope` (rad) toward the downhill azimuth `azimuth` (rad from the world x axis),
+    so that the ground falls by tan(slope) per metre along (cos azimuth, sin azimuth, 0), with friction mu (scalars or [n]).  Each
+    foot's plane has that normal and passes through the foot's current point (feet [n, 4, 3]); four feet that do not lie on one
+    such plane stand on parallel ones.  Returns (terrain [40, n], plane_d [4, n]), as terrain_frames."""
+    n = feet.shape[0]
+    sl, az = np.broadcast_to(np.asarray(slope, dtype=np.float64), (n,)), np.broadcast_to(np.asarray(azimuth, dtype=np.float64), (n,))
+    nrm = np.vstack([np.sin(sl) * np.cos(az), np.sin(sl) * np.sin(az), np.cos(sl)])
+    return terrain_frames(nrm, mu, feet)
+
+
 SWEEP_DIRECTIONS, SWEEP_MAGNITUDES = 16, (5.0, 10.0, 20.0, 30.0, 40.0, 50.0, 65.0, 80.0)
 SWEEP_GAINS = (1.0, 2.0, 5.0, 10.0, 20.0, 50.0, 100.0, 200.0)
 SWEEP_STATES = 256
