@@ -353,6 +353,57 @@ int wbc_set_trajectory(wbc_ctx* ctx, int n, const wbc_trajectory* tr, void* cuda
  * The sampling and the cycle that consumes it must be ordered: pass both the same stream (NULL = the ctx's own). */
 int wbc_sample_trajectory(wbc_ctx* ctx, int n, const double* t, double t_all, const wbc_traj_samples* out, void* cuda_stream, unsigned flags);
 
+/* ---- On-device trot gait generator (DESIGN.md 4.8) --------------------------------------------------------------
+ * A per-robot trot (phases 0 stance, 1 swing{BR,FL}, 2 stance, 3 swing{BL,FR}) that turns a velocity command, the robot's state
+ * and the contact plant's flags into the contact mode and the six desired-trajectory arrays of wbc_inputs, once per control cycle
+ * (dt = params.obs_dt), so that wbc_gait_step -> wbc_cycle -> wbc_plant_contact_step runs without a host round trip.  It stands in
+ * for the reference's TOWR plan: the CoM reference integrates the (ramped) command and is held within `leash` of the measured CoM;
+ * a swing foot follows a quintic from its lift-off point to a Raibert-style touchdown target with a sin^2 lift of step_height, and
+ * its swing ends early when both swing feet are in contact past half of the phase. */
+typedef struct wbc_gait_params {
+    int stance_cycles;    /* 46:   control cycles of each stance phase                                               */
+    int swing_cycles;     /* 46:   control cycles of each swing phase (>= 2)                                         */
+    double step_height;   /* 0.03: foot lift (m), the apex of the sin^2 profile at mid-swing                          */
+    double k_v;           /* 0.1:  touchdown target correction per m/s of measured minus reference velocity (s)        */
+    double max_step;      /* 0.1:  largest distance of a touchdown target from its neutral point (m)                   */
+    double acc_lin;       /* 1.0:  largest change of the reference (vx, vy) per second (m/s^2)                         */
+    double acc_yaw;       /* 2.0:  largest change of the reference yaw rate per second (rad/s^2)                       */
+    double leash;         /* 0.05: largest distance of the CoM reference from the measured CoM in xy (m, > 0)          */
+} wbc_gait_params;
+void wbc_default_gait_params(wbc_gait_params* gp);
+/* Gait state, caller-owned SoA arrays [k][ld] (a checkpoint is a copy of them). */
+typedef struct wbc_gait_state {
+    int* phase;        /* [1] 0..3                                                                                      */
+    int* tick;         /* [1] cycles into the phase, 0 .. phase length - 1                                              */
+    int* landed;       /* [1] 1 once the current swing has touched down (the robot is then in stance until the phase ends) */
+    double* com_ref;   /* [4] CoM reference x, y (world), clearance of the CoM above the ground, reference yaw            */
+    double* v_ref;     /* [3] reference velocity vx, vy (heading frame, i.e. rotated by the reference yaw) and yaw rate   */
+    double* liftoff;   /* [6] lift-off points of the current (or next) swing pair, Jsw row order: first foot xyz, second  */
+    double* target;    /* [6] their touchdown targets (equal to liftoff outside a swing phase at init)                   */
+    double* offset;    /* [8] xy of each stacked foot from its hip in the heading frame, captured at init                 */
+} wbc_gait_state;
+/* Capture the gait state of n robots from the plant state: start offset k0 [ld] (NULL = 0; taken modulo the gait period
+ * 2 (stance_cycles + swing_cycles)) gives phase and tick, landed = 0; com_ref = (measured CoM xy, CoM height above the ground,
+ * base yaw), v_ref = 0, the foot offsets; a robot that starts in a swing phase gets its lift-off points and targets from the current
+ * state.  terrain [40][ld] / plane_d [4][ld] (NULL: flat ground z = 0) as in wbc_plant_contact_step_terrain: the ground height under
+ * a point is the mean of the four feet's plane heights there.  gp NULL = the defaults.  status [ld] (may be NULL): 0;
+ * WBC_ST_NONFINITE for a non-finite input; WBC_ST_BAD_TERRAIN for a foot frame that is not orthonormal to 1e-9 or whose normal has
+ * n_z < 0.5.  A refused robot's gait state is left untouched.  Host or device pointers per flags (st->foot_force, st->dq and
+ * st->mode are not read). */
+int wbc_gait_init(wbc_ctx* ctx, int n, const wbc_gait_params* gp, const wbc_plant_state* st, const int* k0, const double* terrain,
+                  const double* plane_d, wbc_gait_state* gs, int* status, long ld, void* cuda_stream, unsigned flags);
+/* One gait step of n robots (DESIGN.md 4.8): touchdown from contact [4][ld] (the flags of the previous wbc_plant_contact_step; NULL:
+ * a swing lasts its whole phase), lift-off, the ramp of v_ref toward cmd [3][ld] (vx, vy in the heading frame, yaw rate; NULL = 0,
+ * a trot in place), the CoM reference; writes mode [ld] and the six desired arrays of `out` (com_des_* [6][out->ld]: x, y, z, roll 0,
+ * pitch 0, yaw on the measured base_rpy branch; sw_des_* in Jsw row order), then advances the state.  terrain / plane_d as in
+ * wbc_gait_init.  Bad params (non-finite, stance_cycles < 1, swing_cycles < 2, a negative step_height, k_v, max_step, acc_lin or
+ * acc_yaw, leash <= 0) return WBC_EINVAL with nothing done.  status [ld] (may be NULL): as wbc_gait_init, plus WBC_ST_BAD_MODE for a
+ * phase outside 0..3 or a tick outside its phase; a refused robot's state, mode and outputs are left untouched.  st->mode is not
+ * read.  Host or device pointers per flags, WBC_NO_SYNC with device pointers. */
+int wbc_gait_step(wbc_ctx* ctx, int n, const wbc_gait_params* gp, wbc_gait_state* gs, const wbc_plant_state* st, const double* cmd,
+                  const int* contact, const double* terrain, const double* plane_d, int* mode, const wbc_traj_samples* out, int* status,
+                  long ld, void* cuda_stream, unsigned flags);
+
 /* Page-locked host memory for the SoA arrays handed to wbc_cycle with WBC_HOST_PTRS.  Arrays that are page-locked
  * (from here, cudaMallocHost or cudaHostRegister) are copied to and from the device directly; pageable arrays go
  * through the ctx's pinned bounce buffer (one extra host-side pass over the data). */

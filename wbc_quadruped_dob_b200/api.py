@@ -83,6 +83,21 @@ class _TrajSamples(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in TRAJ_FIELDS] + [("ld", C.c_long)]
 
 
+class GaitParams(C.Structure):
+    """wbc_gait_params: phase lengths (control cycles), foot lift (m), touchdown-target velocity gain (s) and step limit (m), command
+    ramp limits (m/s^2, rad/s^2), leash of the CoM reference (m)."""
+    _fields_ = [("stance_cycles", C.c_int), ("swing_cycles", C.c_int)] + \
+               [(n, C.c_double) for n in ("step_height", "k_v", "max_step", "acc_lin", "acc_yaw", "leash")]
+
+
+GAIT_INT_FIELDS = [("phase", 1), ("tick", 1), ("landed", 1)]
+GAIT_FIELDS = [("com_ref", 4), ("v_ref", 3), ("liftoff", 6), ("target", 6), ("offset", 8)]
+
+
+class _GaitState(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n, _ in GAIT_INT_FIELDS + GAIT_FIELDS]
+
+
 class WbcError(RuntimeError):
     pass
 
@@ -95,6 +110,7 @@ EXPORTS = ["wbc_default_params", "wbc_last_error", "wbc_version", "wbc_create", 
            "wbc_plant_step", "wbc_plant_dynamics_step", "wbc_default_contact_params", "wbc_plant_contact_step", "wbc_plant_contact_step_terrain", "wbc_last_timing", "wbc_last_solve_cycles", "wbc_last_launches", "wbc_solver_shape", "wbc_stage_profile", "wbc_host_alloc",
            "wbc_host_free",
            "wbc_set_trajectory", "wbc_sample_trajectory",
+           "wbc_default_gait_params", "wbc_gait_init", "wbc_gait_step",
            "wbc_measure_dfma_peak"]
 
 
@@ -150,6 +166,12 @@ def load():
     lib.wbc_host_free.argtypes = [C.c_void_p]
     lib.wbc_set_trajectory.argtypes = [C.c_void_p, C.c_int, C.POINTER(_Trajectory), C.c_void_p, C.c_uint]
     lib.wbc_sample_trajectory.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_double, C.POINTER(_TrajSamples), C.c_void_p, C.c_uint]
+    lib.wbc_default_gait_params.argtypes = [C.POINTER(GaitParams)]
+    lib.wbc_gait_init.argtypes = [C.c_void_p, C.c_int, C.POINTER(GaitParams), C.POINTER(_PlantState), C.c_void_p, C.c_void_p, C.c_void_p,
+                                  C.POINTER(_GaitState), C.c_void_p, C.c_long, C.c_void_p, C.c_uint]
+    lib.wbc_gait_step.argtypes = [C.c_void_p, C.c_int, C.POINTER(GaitParams), C.POINTER(_GaitState), C.POINTER(_PlantState), C.c_void_p,
+                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(_TrajSamples), C.c_void_p, C.c_long, C.c_void_p,
+                                  C.c_uint]
     lib.wbc_measure_dfma_peak.argtypes = [C.c_void_p, _dp]
     _lib = lib
     return lib
@@ -165,6 +187,12 @@ def default_contact_params():
     cp = ContactParams()
     load().wbc_default_contact_params(C.byref(cp))
     return cp
+
+
+def default_gait_params():
+    gp = GaitParams()
+    load().wbc_default_gait_params(C.byref(gp))
+    return gp
 
 
 def _warm_needs_exact(warm, exact):
@@ -519,6 +547,96 @@ class WbcBatch:
             return
         _check(self.lib.wbc_plant_contact_step(self.h, n, C.byref(ps), _ptr(tau), _ptr(push), _ptr(ground_z), _ptr(mu), ld, int(substeps), C.byref(cp),
                                                _ptr(contact), _ptr(diag), _ptr(status), stream, flags), "wbc_plant_contact_step")
+
+    @staticmethod
+    def gait_state(n, device=None):
+        """A zeroed gait state for n robots (wbc_gait_state): int32 phase, tick, landed [1, n] and float64 com_ref [4, n], v_ref [3, n],
+        liftoff [6, n], target [6, n], offset [8, n]; numpy arrays, or torch tensors on `device` (e.g. "cuda:0")."""
+        if device is None:
+            st = {k: np.zeros((m, n), np.int32) for k, m in GAIT_INT_FIELDS}
+            st.update({k: np.zeros((m, n)) for k, m in GAIT_FIELDS})
+            return st
+        import torch
+        st = {k: torch.zeros(m, n, dtype=torch.int32, device=device) for k, m in GAIT_INT_FIELDS}
+        st.update({k: torch.zeros(m, n, dtype=torch.float64, device=device) for k, m in GAIT_FIELDS})
+        return st
+
+    @staticmethod
+    def _gait_structs(state, gs, others):
+        """The plant-state and gait-state structs, and whether this is the host path (numpy state).  Every array -- state, gait state
+        and the optional ones in `others` (name -> array or None) -- must live on the same side as state["q"]: numpy arrays on the host
+        path, CUDA tensors (or raw device pointers) on the device path.  A pointer of the other side would reach the kernel as if it
+        were of this one, so a mix is refused here."""
+        host = isinstance(state["q"], np.ndarray)
+        arrays = {k: state[k] for k in ("base_pos", "base_rot", "base_rpy", "base_vel", "q")}
+        arrays.update({k: gs[k] for k, _ in GAIT_INT_FIELDS + GAIT_FIELDS})
+        arrays.update({k: a for k, a in others.items() if a is not None})
+        for k, a in arrays.items():
+            on_host = isinstance(a, np.ndarray) or (hasattr(a, "is_cuda") and not a.is_cuda)
+            if host != on_host:
+                raise WbcError("gait: %r is %s memory but the state is %s memory: pass every array on the same side"
+                               % (k, "host" if on_host else "device", "host" if host else "device"))
+        ps = _PlantState()
+        for k in ("base_pos", "base_rot", "base_rpy", "base_vel", "q"):
+            setattr(ps, k, _ptr(state[k]))
+        g = _GaitState()
+        for k, _ in GAIT_INT_FIELDS + GAIT_FIELDS:
+            setattr(g, k, _ptr(gs[k]))
+        if host:
+            for k in ("base_pos", "base_rot", "base_rpy", "base_vel", "q") + tuple(k for k, _ in GAIT_FIELDS):
+                a = state[k] if k in state else gs[k]
+                assert a.flags.c_contiguous and a.dtype == np.float64, k
+            for k, _ in GAIT_INT_FIELDS:
+                assert gs[k].flags.c_contiguous and gs[k].dtype == np.int32, k
+        return ps, g, host
+
+    @staticmethod
+    def _host_in(a, dtype=np.float64):
+        return None if a is None else (np.ascontiguousarray(a, dtype=dtype) if isinstance(a, np.ndarray) else a)
+
+    def gait_init(self, state, gs, k0=None, terrain=None, plane_d=None, params=None, status=None, n=None, ld=None, stream=None, sync=True):
+        """Capture the gait state `gs` (gait_state()) of the robots in `state` (a plant-state dict: base_pos, base_rot, base_rpy, base_vel,
+        q) at start offsets k0 [n] (None: 0), on flat ground or on terrain [40, ld] / plane_d [4, ld] (wbc_gait_init).  numpy arrays: host
+        path; torch CUDA tensors: device path."""
+        ps, g, host = self._gait_structs(state, gs, {"k0": k0, "terrain": terrain, "plane_d": plane_d, "status": status})
+        n = int(state["q"].shape[1]) if n is None else int(n)
+        ld = n if ld is None else int(ld)
+        k0, terrain, plane_d = self._host_in(k0, np.int32), self._host_in(terrain), self._host_in(plane_d)
+        gp = params if params is not None else default_gait_params()
+        flags = (HOST_PTRS if host else DEVICE_PTRS) | (0 if (sync or host) else NO_SYNC)
+        _check(self.lib.wbc_gait_init(self.h, n, C.byref(gp), C.byref(ps), _ptr(k0), _ptr(terrain), _ptr(plane_d), C.byref(g), _ptr(status),
+                                      ld, stream, flags), "wbc_gait_init")
+
+    def gait_step(self, state, gs, cmd=None, contact=None, terrain=None, plane_d=None, out=None, params=None, status=None, n=None, ld=None,
+                  stream=None, sync=True):
+        """One gait step (wbc_gait_step): advances `gs` and writes the contact mode and the six desired arrays into `out`, a dict with
+        "mode" [ld] (int32) and com_des_pos, com_des_vel, com_des_acc, sw_des_pos, sw_des_vel, sw_des_acc [6, ld] -- e.g. the input
+        dict handed to cycle_device, so the controller reads them directly.  cmd [3, ld]
+        (vx, vy in the heading frame, yaw rate; None: trot in place), contact [4, ld] int32 (the contact plant's flags of the previous
+        step; None: no touchdown).  Every array must be on the same side as state["q"] (numpy: host path, CUDA tensors: device
+        path).  out=None allocates the outputs there.  Returns `out`."""
+        n = int(state["q"].shape[1]) if n is None else int(n)
+        ld = n if ld is None else int(ld)
+        if out is None:
+            if isinstance(state["q"], np.ndarray):
+                out = {"mode": np.zeros(ld, np.int32)}
+                out.update({k: np.zeros((6, ld)) for k in TRAJ_FIELDS})
+            else:
+                import torch
+                dev = state["q"].device
+                out = {"mode": torch.zeros(ld, dtype=torch.int32, device=dev)}
+                out.update({k: torch.zeros(6, ld, dtype=torch.float64, device=dev) for k in TRAJ_FIELDS})
+        ps, g, host = self._gait_structs(state, gs, {"cmd": cmd, "contact": contact, "terrain": terrain, "plane_d": plane_d, "status": status,
+                                                     "mode": out["mode"], **{k: out[k] for k in TRAJ_FIELDS}})
+        cmd, terrain, plane_d, contact = self._host_in(cmd), self._host_in(terrain), self._host_in(plane_d), self._host_in(contact, np.int32)
+        t = out[TRAJ_FIELDS[0]]
+        out_ld = int(t.strides[0] // 8) if isinstance(t, np.ndarray) else (int(t.stride(0)) if hasattr(t, "stride") else ld)
+        o = _TrajSamples(*[_ptr(out[k]) for k in TRAJ_FIELDS], out_ld)
+        gp = params if params is not None else default_gait_params()
+        flags = (HOST_PTRS if host else DEVICE_PTRS) | (0 if (sync or host) else NO_SYNC)
+        _check(self.lib.wbc_gait_step(self.h, n, C.byref(gp), C.byref(g), C.byref(ps), _ptr(cmd), _ptr(contact), _ptr(terrain), _ptr(plane_d),
+                                      _ptr(out["mode"]), C.byref(o), _ptr(status), ld, stream, flags), "wbc_gait_step")
+        return out
 
     def last_timing(self):
         a, b = C.c_float(0), C.c_float(0)

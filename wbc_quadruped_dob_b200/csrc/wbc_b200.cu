@@ -25,6 +25,7 @@
 #include "wbc_contact.cuh"
 #include "wbc_front.cuh"
 #include "wbc_front_leg.cuh"
+#include "wbc_gait.cuh"
 #include "wbc_traj.cuh"
 #include "wbc_types.h"
 
@@ -885,6 +886,21 @@ __global__ void __launch_bounds__(64) wbc_contact_terrain_kernel(Params P, wbc::
     wbc::contact_step_instance<true>(P, cp, io, i, nsub, terrain);
 }
 
+// Trot gait generator, thread per robot (wbc_gait.cuh): capture the gait state, and one gait step.
+__global__ void __launch_bounds__(128) wbc_gait_init_kernel(wbc::GaitParams G, double dt, wbc::GaitIO io, int n)
+{
+    const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    wbc::gait_init_instance(G, dt, io, i);
+}
+
+__global__ void __launch_bounds__(128) wbc_gait_kernel(wbc::GaitParams G, double dt, wbc::GaitIO io, int n)
+{
+    const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    wbc::gait_step_instance(G, dt, io, i);
+}
+
 // FP64 DFMA peak: 8 independent chains per thread, fully unrolled.
 __global__ void __launch_bounds__(256) wbc_dfma_peak_kernel(double* out, int iters)
 {
@@ -1008,6 +1024,14 @@ void wbc_default_contact_params(wbc_contact_params* cp)
     if (!cp) return;
     memset(cp, 0, sizeof(*cp));
     cp->beta = 0.2; cp->eps = 1.0e-8; cp->margin = 2.0e-3; cp->max_iter = 64;
+}
+
+void wbc_default_gait_params(wbc_gait_params* gp)
+{
+    if (!gp) return;
+    memset(gp, 0, sizeof(*gp));
+    gp->stance_cycles = 46; gp->swing_cycles = 46; gp->step_height = 0.03;
+    gp->k_v = 0.1; gp->max_step = 0.1; gp->acc_lin = 1.0; gp->acc_yaw = 2.0; gp->leash = 0.05;
 }
 
 const char* wbc_last_error(void) { return g_err; }
@@ -1770,6 +1794,128 @@ int wbc_plant_contact_step_terrain(wbc_ctx* c, int n, const wbc_plant_state* st,
     if (!terrain) return fail(WBC_EINVAL, "wbc_plant_contact_step_terrain: terrain is NULL (flat ground is wbc_plant_contact_step)");
     return contact_step("wbc_plant_contact_step_terrain", c, n, st, tau, push, plane_d, nullptr, terrain, ld, substeps, cp, contact, diag,
                         status, cuda_stream, flags);
+}
+
+// The host side of wbc_gait_init (init = true: k0, no command, outputs or contact flags) and wbc_gait_step.
+static int gait_call(const char* fn, bool init, wbc_ctx* c, int n, const wbc_gait_params* gp, wbc_gait_state* gs, const wbc_plant_state* st,
+                     const int* k0, const double* cmd, const int* contact, const double* terrain, const double* plane_d, int* mode,
+                     const wbc_traj_samples* out, int* status, long ld, void* cuda_stream, unsigned flags)
+{
+    if (!c || !gs || !st) return fail(WBC_EINVAL, "%s: null argument", fn);
+    if (!st->base_pos || !st->base_rot || !st->base_rpy || !st->base_vel || !st->q)
+        return fail(WBC_EINVAL, "%s: a state array (base_pos, base_rot, base_rpy, base_vel, q) is NULL", fn);
+    if (!gs->phase || !gs->tick || !gs->landed || !gs->com_ref || !gs->v_ref || !gs->liftoff || !gs->target || !gs->offset)
+        return fail(WBC_EINVAL, "%s: a gait state array is NULL", fn);
+    if (!init && (!mode || !out || !out->com_des_pos || !out->com_des_vel || !out->com_des_acc || !out->sw_des_pos || !out->sw_des_vel ||
+                  !out->sw_des_acc))
+        return fail(WBC_EINVAL, "%s: mode or an output array is NULL", fn);
+    if (plane_d && !terrain) return fail(WBC_EINVAL, "%s: plane_d needs terrain", fn);
+    if (n < 0 || n > c->max_batch || ld < n) return fail(WBC_EINVAL, "%s: n outside [0, max_batch] or ld < n", fn);
+    if (!init && out->ld < n) return fail(WBC_EINVAL, "%s: out->ld < n", fn);
+    wbc_gait_params g;
+    wbc_default_gait_params(&g);
+    if (gp) g = *gp;
+    const double fin[6] = {g.step_height, g.k_v, g.max_step, g.acc_lin, g.acc_yaw, g.leash};
+    bool ok = g.stance_cycles >= 1 && g.swing_cycles >= 2 && g.stance_cycles <= (1 << 20) && g.swing_cycles <= (1 << 20) && g.leash > 0.0;
+    for (int k = 0; k < 6; k++) ok = ok && fin[k] >= 0.0 && fin[k] < 1.0e300;
+    if (!ok)
+        return fail(WBC_EINVAL, "%s: gait params outside stance_cycles in [1, 2^20], swing_cycles in [2, 2^20], finite step_height, k_v, "
+                                "max_step, acc_lin, acc_yaw >= 0 and leash > 0", fn);
+    if (n == 0) { c->launches = 0; return WBC_OK; }
+    CU(cudaSetDevice(c->device));
+    cudaStream_t s = cuda_stream ? (cudaStream_t)cuda_stream : c->stream;
+    const bool dev_ptrs = (flags & WBC_DEVICE_PTRS) != 0;
+    const wbc::GaitParams G = {g.stance_cycles, g.swing_cycles, g.step_height, g.k_v, g.max_step, g.acc_lin, g.acc_yaw, g.leash};
+    wbc::GaitIO io;
+    io.k0 = k0; io.cmd = cmd; io.contact = contact; io.terrain = terrain; io.plane_d = plane_d; io.status = status; io.mode = mode;
+    io.base_pos = st->base_pos; io.base_rot = st->base_rot; io.base_rpy = st->base_rpy; io.base_vel = st->base_vel; io.q = st->q;
+    io.phase = gs->phase; io.tick = gs->tick; io.landed = gs->landed;
+    io.com_ref = gs->com_ref; io.v_ref = gs->v_ref; io.liftoff = gs->liftoff; io.target = gs->target; io.offset = gs->offset;
+    double* const hout[6] = {init ? nullptr : out->com_des_pos, init ? nullptr : out->com_des_vel, init ? nullptr : out->com_des_acc,
+                             init ? nullptr : out->sw_des_pos, init ? nullptr : out->sw_des_vel, init ? nullptr : out->sw_des_acc};
+    for (int b = 0; b < 6; b++) io.des[b] = hout[b];
+    io.out_ld = init ? ld : out->ld; io.ld = ld;
+    // host path: packed staging.  Doubles in d_in: state 30 rows (base_pos 3, base_rot 9, base_rpy 3, base_vel[0:3], q 12) | gait
+    // state 27 (com_ref 4, v_ref 3, liftoff 6, target 6, offset 8) | cmd 3 | plane_d 4 | terrain 40; the six outputs in d_out; ints in
+    // d_iout: phase, tick, landed | contact 4 (k0 in its first row) | mode | status.  The gait state and the outputs are uploaded too,
+    // since a refused robot keeps them as they were.
+    static const int KS[5] = {3, 9, 3, 3, 12};
+    static const int KG[5] = {4, 3, 6, 6, 8};
+    const double* hst[5] = {st->base_pos, st->base_rot, st->base_rpy, st->base_vel, st->q};
+    double* hgs[5] = {gs->com_ref, gs->v_ref, gs->liftoff, gs->target, gs->offset};
+    int* hint[3] = {gs->phase, gs->tick, gs->landed};
+    const size_t N = (size_t)n;
+    if (!dev_ptrs) {
+        double* h = c->h_pin;
+        int* hi = c->h_pin_i;
+        double* d = c->d_in;
+        size_t off = 0;
+        for (int f = 0; f < 5; f++)
+            for (int k = 0; k < KS[f]; k++, off++) memcpy(h + off * N, hst[f] + (size_t)k * ld, N * 8);
+        for (int f = 0; f < 5; f++)
+            for (int k = 0; k < KG[f]; k++, off++) memcpy(h + off * N, hgs[f] + (size_t)k * ld, N * 8);
+        if (cmd) for (int k = 0; k < 3; k++) memcpy(h + (57 + k) * N, cmd + (size_t)k * ld, N * 8);
+        if (plane_d) for (int k = 0; k < 4; k++) memcpy(h + (60 + k) * N, plane_d + (size_t)k * ld, N * 8);
+        if (terrain) for (int k = 0; k < 40; k++) memcpy(h + (64 + k) * N, terrain + (size_t)k * ld, N * 8);
+        CU(cudaMemcpyAsync(d, h, (terrain ? 104 : 64) * N * 8, cudaMemcpyHostToDevice, s));
+        for (int k = 0; k < 3; k++) memcpy(hi + k * N, hint[k], N * sizeof(int));
+        if (k0) memcpy(hi + 3 * N, k0, N * sizeof(int));
+        if (contact) for (int k = 0; k < 4; k++) memcpy(hi + (3 + k) * N, contact + (size_t)k * ld, N * sizeof(int));
+        if (mode) memcpy(hi + 7 * N, mode, N * sizeof(int));
+        CU(cudaMemcpyAsync(c->d_iout, hi, 8 * N * sizeof(int), cudaMemcpyHostToDevice, s));
+        if (!init) {
+            for (int b = 0; b < 6; b++)
+                CU(cudaMemcpy2DAsync(c->d_out + (size_t)b * 6 * N, N * 8, hout[b], (size_t)out->ld * 8, N * 8, 6, cudaMemcpyHostToDevice, s));
+            for (int b = 0; b < 6; b++) io.des[b] = c->d_out + (size_t)b * 6 * N;
+        }
+        io.base_pos = d; io.base_rot = d + 3 * N; io.base_rpy = d + 12 * N; io.base_vel = d + 15 * N; io.q = d + 18 * N;
+        io.com_ref = d + 30 * N; io.v_ref = d + 34 * N; io.liftoff = d + 37 * N; io.target = d + 43 * N; io.offset = d + 49 * N;
+        io.cmd = cmd ? d + 57 * N : nullptr; io.plane_d = plane_d ? d + 60 * N : nullptr; io.terrain = terrain ? d + 64 * N : nullptr;
+        io.phase = c->d_iout; io.tick = c->d_iout + N; io.landed = c->d_iout + 2 * N;
+        io.k0 = k0 ? c->d_iout + 3 * N : nullptr; io.contact = contact ? c->d_iout + 3 * N : nullptr;
+        io.mode = mode ? c->d_iout + 7 * N : nullptr; io.status = status ? c->d_iout + 8 * N : nullptr;
+        io.out_ld = n; io.ld = n;
+    }
+    const double dt = c->params.obs_dt;
+    if (init)
+        wbc_gait_init_kernel<<<(n + 127) / 128, 128, 0, s>>>(G, dt, io, n);
+    else
+        wbc_gait_kernel<<<(n + 127) / 128, 128, 0, s>>>(G, dt, io, n);
+    CU(cudaGetLastError());
+    c->launches = 1;
+    if (!dev_ptrs) {
+        CU(cudaMemcpyAsync(c->h_pin + 30 * N, c->d_in + 30 * N, 27 * N * 8, cudaMemcpyDeviceToHost, s));
+        if (!init) CU(cudaMemcpyAsync(c->h_pin + 57 * N, c->d_out, 36 * N * 8, cudaMemcpyDeviceToHost, s));
+        CU(cudaMemcpyAsync(c->h_pin_i, c->d_iout, 9 * N * sizeof(int), cudaMemcpyDeviceToHost, s));
+        CU(cudaStreamSynchronize(s));
+        size_t off = 30;
+        for (int f = 0; f < 5; f++)
+            for (int k = 0; k < KG[f]; k++, off++) memcpy(hgs[f] + (size_t)k * ld, c->h_pin + off * N, N * 8);
+        if (!init)
+            for (int b = 0; b < 6; b++)
+                for (int k = 0; k < 6; k++) memcpy(hout[b] + (size_t)k * out->ld, c->h_pin + (57 + 6 * b + k) * N, N * 8);
+        for (int k = 0; k < 3; k++) memcpy(hint[k], c->h_pin_i + k * N, N * sizeof(int));
+        if (mode) memcpy(mode, c->h_pin_i + 7 * N, N * sizeof(int));
+        if (status) memcpy(status, c->h_pin_i + 8 * N, N * sizeof(int));
+    } else if (!(flags & WBC_NO_SYNC)) {
+        CU(cudaStreamSynchronize(s));
+    }
+    return WBC_OK;
+}
+
+int wbc_gait_init(wbc_ctx* c, int n, const wbc_gait_params* gp, const wbc_plant_state* st, const int* k0, const double* terrain,
+                  const double* plane_d, wbc_gait_state* gs, int* status, long ld, void* cuda_stream, unsigned flags)
+{
+    return gait_call("wbc_gait_init", true, c, n, gp, gs, st, k0, nullptr, nullptr, terrain, plane_d, nullptr, nullptr, status, ld,
+                     cuda_stream, flags);
+}
+
+int wbc_gait_step(wbc_ctx* c, int n, const wbc_gait_params* gp, wbc_gait_state* gs, const wbc_plant_state* st, const double* cmd,
+                  const int* contact, const double* terrain, const double* plane_d, int* mode, const wbc_traj_samples* out, int* status,
+                  long ld, void* cuda_stream, unsigned flags)
+{
+    return gait_call("wbc_gait_step", false, c, n, gp, gs, st, nullptr, cmd, contact, terrain, plane_d, mode, out, status, ld, cuda_stream,
+                     flags);
 }
 
 int wbc_last_timing(wbc_ctx* c, float* front_ms, float* solve_ms)
