@@ -69,7 +69,9 @@ extern "C" {
                                   * qp_info in this mode: [0] factorisations (1), [1] rows added to the active set (equalities
                                   * included), [2] rows dropped, [3] active inequality rows, [4] active-set size, [5] flags: 256 always
                                   * (exact mode), | 512 a dependent consistent equality was skipped, | 1024 a violated row depended on
-                                  * the active set and dual steps were taken; [6], [7] 0.  qp_flops: the exact solver's own count. */
+                                  * the active set and dual steps were taken, | 4096 a violated row depended on the active set, was
+                                  * implied by it and violated only by rounding, and was held out; [6], [7] 0.  qp_flops: the exact
+                                  * solver's own count. */
 #define WBC_QP_WARM 64u          /* wbc_cycle, only together with WBC_QP_EXACT (else WBC_EINVAL, nothing done): warm-start each instance
                                   * from the active set the ctx stored for its index (wbc_get_active_set) when that set was solved in
                                   * the instance's current contact mode; any other instance starts cold.  Every exact-mode cycle, warm

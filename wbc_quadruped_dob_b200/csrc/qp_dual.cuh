@@ -20,7 +20,10 @@
 //     residual is within the feasibility tolerance and reports WBC_ST_INFEASIBLE otherwise;
 //   * a violated row whose normal depends on the active set (a degenerate vertex: e.g. the 5 friction rows of an unloaded foot
 //     through one point of its 3 force components) is never added: the method takes dual steps, dropping active rows,
-//     until it is independent -- or reports WBC_ST_INFEASIBLE when no row can be dropped;
+//     until it is independent -- or reports WBC_ST_INFEASIBLE when no row can be dropped.  Before any such step, a dependent
+//     row that the active rows imply is met (n = sum r_k n_k and b - sum r_k b_k within the feasibility tolerance), and that
+//     is violated only by rounding (TOL_HOLD), is held out of the search until the next drop: with mu = 0 each tangential
+//     friction row comes with its negation, and the second of a pair must not end the solve;
 //   * iterations (one per d = J'n evaluation) are capped at 2 nrows + 30; an overrun returns -100.
 // A failed solve returns x = 0.
 #pragma once
@@ -35,6 +38,7 @@ constexpr int MAXROWS = 88;
 constexpr double TOL_DEP = 1.0e-10;     // |d2| <= TOL_DEP |d|: the row is a combination of the active rows
 constexpr double TOL_FEAS = 1.0e-12;    // row-scaled residual counted as feasible (relative to max(1, |b|, sum |a_j y_j|))
 constexpr double TOL_PIV = 1.0e-14;     // Cholesky pivot of the unit-diagonal scaled H below which H is not positive definite
+constexpr double TOL_HOLD = 1.0e-9;     // row-scaled violation up to which a dependent, consistent row counts as rounding
 
 // status (include/wbc_b200.h)
 constexpr int ST_OK = 0;
@@ -45,6 +49,7 @@ constexpr int ST_ITERATIONS = -100;
 constexpr int FL_EXACT = 256;           // set on every exact-mode result (no DENSE-AUL path uses this bit)
 constexpr int FL_DEP_EQ = 512;          // a dependent, consistent equality row was skipped
 constexpr int FL_DUAL_STEP = 1024;      // a violated row depended on the active set: pure dual steps were taken
+constexpr int FL_DEP_HELD = 4096;       // a violated, dependent, consistent inequality row was held out (rounding)
 
 // shared-memory layout of one warp (doubles)
 namespace ds {
@@ -309,6 +314,7 @@ WBC_HDN void solve_dual(const Ex& ex, double* sm, double* C, int nrows, int neq,
     int iq = 0;                        // active rows
     int peq = 0;                       // of which equalities (positions [0, peq))
     unsigned act[3] = {0u, 0u, 0u};    // active inequality rows (bit mask, uniform)
+    unsigned held[3] = {0u, 0u, 0u};   // dependent, consistent rows held out of the search until the next drop (uniform)
     double z[RPL];
     int warm_adds = 0, warm_drops = 0;
 
@@ -404,6 +410,7 @@ WBC_HDN void solve_dual(const Ex& ex, double* sm, double* C, int nrows, int neq,
             A[iq] = -1; U[iq] = 0.0;
         }
         act[row >> 5] &= ~(1u << (row & 31));
+        held[0] = 0u; held[1] = 0u; held[2] = 0u;
         iq--;
         st.drops++;
         ex.sync();
@@ -566,7 +573,8 @@ WBC_HDN void solve_dual(const Ex& ex, double* sm, double* C, int nrows, int neq,
     }
     // ---- inequalities
     while (st.status == ST_OK) {
-        const int ip = most_violated(ex, C, Y, nrows, neq, act);
+        const unsigned skip[3] = {act[0] | held[0], act[1] | held[1], act[2] | held[2]};
+        const int ip = most_violated(ex, C, Y, nrows, neq, skip);
         flops += 2.0 * N * (nrows - neq);
         mark(PH_SWEEP);
         if (ip < 0) break;                                   // every row feasible: optimal
@@ -576,7 +584,7 @@ WBC_HDN void solve_dual(const Ex& ex, double* sm, double* C, int nrows, int neq,
         if (lane == 0) U[iq] = 0.0;
         ex.sync();
         mark(PH_D);
-        for (;;) {
+        for (bool first = true;; first = false) {
             if (++iters > maxit) { st.status = ST_ITERATIONS; break; }
             double nd2, nd;
             compute_d(nd2, nd);
@@ -585,6 +593,17 @@ WBC_HDN void solve_dual(const Ex& ex, double* sm, double* C, int nrows, int neq,
             if (!dep) compute_z();
             compute_r();
             mark(PH_ZR);
+            if (dep && first) {
+                // where the active rows hold (n_k.y = -b_k), n.y + b = b - sum r_k b_k: the row is implied, not violated
+                double p[2] = {0.0, 0.0};
+                for (int k = lane; k < iq; k += Ex::NL) { const double t = RV[k] * C[A[k] * LD + N]; p[0] += t; p[1] += fabs(t); }
+                wbcqp::red_sum<2>(ex, p);
+                if (b - p[0] >= -TOL_FEAS * fmax(1.0, fabs(b) + p[1]) && s >= -(TOL_HOLD / TOL_FEAS) * tol) {
+                    held[ip >> 5] |= 1u << (ip & 31);
+                    st.flags |= FL_DEP_HELD;
+                    break;
+                }
+            }
             // dual step length t1: the first active inequality multiplier to reach zero
             double t1 = 1.0e300;
             int kp = -1;
